@@ -2,6 +2,7 @@
 """bench.py — MCTS simulations/sec of the batched Stochastic-MuZero search (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--net auto|bf16|tc32|fp32]
+                    [--dump-outputs DIR]
 
 A "step" is one whole batched search: root step (representation + prediction, root expansion,
 Dirichlet mixing) + 50 simulations for 4096 concurrent trees (BASELINE.json configs[1]: CartPole MLP
@@ -127,6 +128,31 @@ class ClockSampler(threading.Thread):
                 "power_w_max": max((r[2] for r in rows), default=None), "window": label}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, roots):
+    """Writes the root statistics of the last timed step (SearchEngine.read_roots: visit counts, root values, root
+    priors and rewards of the children, error flag) as <path>/<name>.npy in float32 / float64, so that two builds
+    can be compared output for output.  Above DUMP_LIMIT_BYTES a fixed, seeded sample of trees is kept;
+    tree_index.npy says which."""
+    import numpy as np
+    arrays = {"visits": roots["visits"].float(), "root_values": roots["root_values"], "priors": roots["priors"],
+              "rewards": roots["rewards"]}
+    arrays = {k: v.cpu().numpy() for k, v in arrays.items()}
+    n = len(arrays["visits"])
+    per_tree = sum(a.nbytes for a in arrays.values()) // n + 8
+    idx = np.arange(n)
+    if n * per_tree > DUMP_LIMIT_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(n, DUMP_LIMIT_BYTES // per_tree, replace=False))
+    arrays = {k: v[idx] for k, v in arrays.items()}
+    arrays["tree_index"] = idx.astype(np.float64)
+    arrays["error"] = roots["error"].cpu().numpy().astype(np.float32)
+    os.makedirs(path, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), v)
+
+
 def run_reference(args):
     """Reference arm: the reference's CPU search path on all host cores (the unmodified reference where a
     checkout is reachable, else the oracle port — see oracle/cpu_baseline.py); each step is a bounded sample of
@@ -205,8 +231,10 @@ class Bench:
             dist.barrier()
         st = self.eng.stats()
         dev_ms = sum(a.elapsed_time(b) for a, b in evs)
+        # what a caller of the timed path receives from its last step (--dump-outputs)
+        self.last_roots = self.eng.read_roots()
         # every rank must have finished every tree: sum of root visits over all ranks == world * B * N
-        visits = self.eng.read_roots()["visits"].sum().to(torch.float64).reshape(1)
+        visits = self.last_roots["visits"].sum().to(torch.float64).reshape(1)
         t = torch.tensor([dev_ms], dtype=torch.float64, device=self.dev)
         if world > 1:
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -373,7 +401,11 @@ def main():
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--soak-seconds", type=float, default=2.5)
     ap.add_argument("--profile-only", action="store_true", help="timed steps only (for runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the root statistics of the last timed step to DIR/<name>.npy (rank 0's trees)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
     args.warmup = max(args.warmup, 3)
@@ -444,6 +476,8 @@ def main():
     main_b = Bench(torch, dist, args, wl, net, B, N, world, rank, local, blob, obs)
     res = main_b.timed(args.steps, args.warmup, flush, sampler,
                        soak_s=0.0 if (args.profile_only or args.no_extras) else args.soak_seconds)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, main_b.last_roots)
     if args.profile_only:
         if rank == 0:
             print(json.dumps({"metric": METRIC, "value": res["value"], "unit": UNIT, "ms_per_step": res["ms_per_step"],

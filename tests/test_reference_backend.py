@@ -1,61 +1,45 @@
-"""Container-only checks (skipped where the reference checkout does not exist, e.g. on the GPU box):
-the torch re-statement of the inference facade in batched_model.ReferenceModuleBackend against the
-reference's own batch-1 `*_function_inference` methods, for the MLP and the vision model families."""
-import warnings
-
+"""The torch re-statement of the inference facade in batched_model.ReferenceModuleBackend against the
+reference's own batch-1 `*_function_inference` outputs stored in tests/golden (net_*.npz for the MLP family,
+vision_*.npz for the vision family), evaluated on reference-shaped modules filled with the stored weights."""
 import numpy as np
 import pytest
 import torch
 
-from oracle import ref_shim
+import golden_io
+from fake_muzero import FakeMuzero, FakeVisionMuzero
 
-pytestmark = pytest.mark.skipif(not ref_shim.available(), reason="reference checkout not present")
 
-
-def _vision_muzero(A=4, S=61, H=32, L=2, seed=0):
-    _, ref_model = ref_shim.load()
-    torch.manual_seed(seed)
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        return ref_model.Muzero(model_structure="vision_model",
-                                observation_space_dimensions=ref_shim.Box(0, 1, (98, 98, 3)),
-                                action_space_dimensions=ref_shim.Discrete(A), state_space_dimensions=S,
-                                hidden_layer_dimensions=H, number_of_hidden_layer=L, device="cpu", use_amp=False)
+def _cases(family):
+    if family == "mlp":
+        for name in golden_io.net_cases():
+            z = golden_io.load_net_case(name)
+            yield name, FakeMuzero(z["weights"], *[int(v) for v in z["dims"]]), z
+    else:
+        for name in golden_io.vision_cases():
+            z = golden_io.load_vision_case(name)
+            yield name, FakeVisionMuzero(z["weights"], *[int(v) for v in z["dims"]]), z
 
 
 @pytest.mark.parametrize("family", ["mlp", "vision"])
 def test_reference_module_backend_matches_reference_inference(family):
     from stochastic_muzero_b200.batched_model import ReferenceModuleBackend
     torch.set_num_threads(1)
-    if family == "mlp":
-        mz = ref_shim.make_muzero(obs_dim=5, action_dim=3, state_dim=11, hidden_dim=14, n_hidden=2, seed=1)
-        obs = torch.randn(6, 5)
-    else:
-        mz = _vision_muzero()
-        obs = torch.rand(3, 3, 98, 98)
     # vision: scale_to_bound_action normalises over the 3 CHANNELS of each pixel (vision:495-503); when the
     # three values nearly coincide the division amplifies fp32 noise (batched vs batch-1 conv algorithms)
     hid_tol = 1e-5 if family == "mlp" else 2e-4
-    be = ReferenceModuleBackend(mz, device="cpu")
-    A = mz.action_dimension
-    acts = torch.arange(obs.shape[0]) % A
-    h = be.representation(obs)
-    p, v = be.prediction(h)
-    ah = be.afterstate_dynamics(h, acts)
-    ap, av = be.afterstate_prediction(ah)
-    r, dh = be.dynamics(ah, acts)
-    with torch.no_grad():
-        for i in range(obs.shape[0]):
-            rh = mz.representation_function_inference(obs[i:i + 1])
-            np.testing.assert_allclose(h[i:i + 1].numpy(), rh.numpy(), atol=hid_tol)
-            rp, rv = mz.prediction_function_inference(rh)
-            np.testing.assert_allclose(p[i].numpy(), rp[0], atol=1e-5)
-            np.testing.assert_allclose(v[i].item(), rv, atol=1e-5, rtol=5e-5)
-            rah = mz.afterstate_dynamics_function_inference(rh, int(acts[i]))
-            np.testing.assert_allclose(ah[i:i + 1].numpy(), rah.numpy(), atol=hid_tol)
-            rap, rav = mz.afterstate_prediction_function_inference(rah)
-            np.testing.assert_allclose(ap[i].numpy(), rap[0], atol=1e-5)
-            np.testing.assert_allclose(av[i].item(), rav, atol=1e-5, rtol=5e-5)
-            rr, rdh = mz.dynamics_function_inference(rah, int(acts[i]))
-            np.testing.assert_allclose(dh[i:i + 1].numpy(), rdh.numpy(), atol=hid_tol)
-            np.testing.assert_allclose(r[i].item(), rr, atol=1e-5, rtol=5e-5)
+    for name, mz, z in _cases(family):
+        be = ReferenceModuleBackend(mz, device="cpu")
+        t = {k: torch.from_numpy(z[k]) for k in ("obs", "repr_h", "adyn_h", "dyn_h")}
+        acts = torch.from_numpy(z["actions"]).long()
+        np.testing.assert_allclose(be.representation(t["obs"]).numpy(), z["repr_h"], atol=hid_tol, err_msg=name)
+        for h, pol, val, fn in (("repr_h", "pred_policy", "pred_value", be.prediction),
+                                ("adyn_h", "apred_policy", "apred_value", be.afterstate_prediction),
+                                ("dyn_h", "dpred_policy", "dpred_value", be.prediction)):
+            p, v = fn(t[h])
+            np.testing.assert_allclose(p.numpy(), z[pol], atol=1e-5, err_msg=f"{name} {pol}")
+            np.testing.assert_allclose(v.numpy(), z[val], atol=1e-5, rtol=5e-5, err_msg=f"{name} {val}")
+        ah = be.afterstate_dynamics(t["repr_h"], acts)
+        np.testing.assert_allclose(ah.numpy(), z["adyn_h"], atol=hid_tol, err_msg=name)
+        r, dh = be.dynamics(t["adyn_h"], acts)
+        np.testing.assert_allclose(dh.numpy(), z["dyn_h"], atol=hid_tol, err_msg=name)
+        np.testing.assert_allclose(r.numpy(), z["dyn_reward"], atol=1e-5, rtol=5e-5, err_msg=name)
