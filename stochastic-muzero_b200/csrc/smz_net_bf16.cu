@@ -1059,10 +1059,17 @@ k_bf16_chain_pipeN(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
 // read with tcgen05.ld.16x256b so that all 32 lanes carry data (thread t: row t/4 and row t/4 + 8, two consecutive
 // columns per 8-column group — the m16n8 accumulator fragment).  Same issuer warp / rounds / named-barrier
 // structure as k_bf16_chain_pipe.
+// Only layer 0 (gathered rows + one-hot columns) reads A from shared memory.  The MMAs of every later layer read it from
+// tensor memory (umma_ts): A row m sits in the lane of accumulator row m, so each epilogue thread writes its packed bf16
+// results with tcgen05.st.16x128b into the very lanes it loaded them from, and the hand-off to the issuer is
+// tcgen05.wait::st + tcgen05 fence + named barrier — no st.shared, no generic -> async proxy fence.
+// TMEM: one 128-column accumulator (every epilogue thread has loaded all of it before its first arrive, so the next
+// layer may overwrite it) + the 64-column A operand (K = 128 bf16) = the same 256-column allocation as two accumulators.
 // ---------------------------------------------------------------------------------------------
 constexpr int TM64 = 64;
-constexpr int A64_BYTES = TM64 * KMAX * 2;       // 16 KB
+constexpr int A64_BYTES = TM64 * KMAX * 2;       // 16 KB (layer 0 only)
 constexpr int CHUNK_A64 = TM64 * 16;             // LBO of the 64-row A operand
+constexpr unsigned A64_TCOL = TN;                // TMEM column of the A operand of layers 1 .. nl-1
 constexpr unsigned IDESC64 = (1u << 4) | (1u << 7) | (1u << 10) | ((unsigned)(TN >> 3) << 17) | ((unsigned)(TM64 >> 4) << 24);
 
 struct Smem64 {
@@ -1085,8 +1092,24 @@ __device__ __forceinline__ void umma64(unsigned tmem_d, unsigned long long adesc
       "l"(adesc), "l"(bdesc), "r"(IDESC64), "r"(accum)
       : "memory");
 }
-__device__ __forceinline__ void a64_store2(unsigned char* a, int row, int col, unsigned v) {   // two bf16 at (row, col), col even
-  asm volatile("st.shared.b32 [%0], %1;" ::"r"(s32(a + (col >> 3) * CHUNK_A64 + row * 16 + (col & 7) * 2)), "r"(v) : "memory");
+// N consecutive 8-column accumulator groups of this thread (pa: row t/4, pb: row t/4 + 8, packed bf16 pairs) -> the 4N
+// TMEM columns of the A operand that hold the same K range, starting at taddr (lane quarter base + A64_TCOL + group * 4)
+template <int N>
+__device__ __forceinline__ void a64_tstore(unsigned taddr, const unsigned* pa, const unsigned* pb) {
+  unsigned r[2 * N];
+#pragma unroll
+  for (int i = 0; i < N; ++i) { r[2 * i] = pa[i]; r[2 * i + 1] = pb[i]; }
+  if constexpr (N == 1) {
+    tmem_st16x128_x1(taddr, r[0], r[1]);
+  } else if constexpr (N == 2) {
+    tmem_st16x128_x2(taddr, r);
+  } else if constexpr (N == 3) {
+    tmem_st16x128_x2(taddr, r);
+    tmem_st16x128_x1(taddr + 8, r[4], r[5]);
+  } else {
+    static_assert(N == 4, "a64_tstore: 1 .. 4 groups");
+    tmem_st16x128_x4(taddr, r);
+  }
 }
 
 // R0 = columns of the first hidden-layer round (64: two even rounds; 96: 96 + 32, two K-steps left for the tail).
@@ -1209,7 +1232,6 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
         if (slot) ++nseen1; else ++nseen0;
       }
       const unsigned long long bd = umma_desc(s32(sm.w[slot]), CHUNK_W, 128);
-      const unsigned d = tmem + (unsigned)((l & 1) * TN);
       for (int c = 0; c < 2; ++c) {
         nb_sync(2 + c);
         if (tl && c == 1) tl[1 + l * 4 + 0] = clock64();       // last round of the layer is in the A operand
@@ -1218,9 +1240,13 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
         if (elect_one()) {
 #pragma unroll
           for (int k = 0; k < 8; ++k)
-            if (k >= (c ? R0 / 16 : 0) && k < (c ? 8 : R0 / 16) && k < nk)
-              umma64(d, ad + (unsigned long long)(k * ((2 * CHUNK_A64) >> 4)), bd + (unsigned long long)(k * ((2 * CHUNK_W) >> 4)),
-                     k > 0 ? 1u : 0u);
+            if (k >= (c ? R0 / 16 : 0) && k < (c ? 8 : R0 / 16) && k < nk) {
+              const unsigned long long bk = bd + (unsigned long long)(k * ((2 * CHUNK_W) >> 4));
+              if (l == 0)
+                umma64(tmem, ad + (unsigned long long)(k * ((2 * CHUNK_A64) >> 4)), bk, k > 0 ? 1u : 0u);
+              else
+                umma_ts(tmem, tmem + A64_TCOL + 8 * k, bk, IDESC64, k > 0 ? 1u : 0u);
+            }
         }
         __syncwarp();
         if (tl && c == 0 && l == 3) tl[1 + 4 * MAXL + 11] = clock64();
@@ -1269,14 +1295,13 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
     for (int c = 0; c < 2; ++c) nb_arrive(2 + c);
     mbar_wait(&sm.bbar, 0);
     epi_sync();                              // rowidx is read by other threads from here on
-    const unsigned lane_t = tmem + ((unsigned)(q * 32) << 16);
+    const unsigned lane_t = tmem + ((unsigned)(q * 32) << 16), a_t = lane_t + A64_TCOL;
     const int S = job.S;
     const int idxA = sm.rowidx[rA], idxB = HALF ? -1 : sm.rowidx[rB];
     const float (*bias)[TN] = sm.bias[branch];
 
     for (int l = 0; l < nl; ++l) {
       const int kind = ch.layer[l].kind;
-      const unsigned dcol = (unsigned)((l & 1) * TN);
       // hidden layers: this warp's bias pairs are fetched before the accumulator wait (the asm volatile stores below
       // are compiler barriers: a load placed after one of them waits for it)
       constexpr int G0 = R0 / 32, G1 = (TN - R0) / 32;          // 8-column groups per warp in round 0 / 1
@@ -1292,26 +1317,28 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
       tc_fence_after();
       if (kind == LK_HIDDEN) {
         // two rounds: columns [0, R0) and [R0, 128); this warp owns a quarter of each round for its 16 rows.  All the
-        // arithmetic of both rounds first (independent chains: the MUFU latencies overlap), then stores + fence per round.
+        // arithmetic of both rounds first (independent chains: the MUFU latencies overlap), then stores + hand-off per round.
         unsigned raw[4 * (G0 + G1)];
         if constexpr (R0 == 64) {
-          tmem_ld16x256_x2(lane_t + dcol + cb * 16, raw);
-          tmem_ld16x256_x2(lane_t + dcol + 64 + cb * 16, raw + 8);
+          tmem_ld16x256_x2(lane_t + cb * 16, raw);
+          tmem_ld16x256_x2(lane_t + 64 + cb * 16, raw + 8);
         } else {
-          tmem_ld16x256_x2(lane_t + dcol + cb * 24, raw);
-          tmem_ld16x256_x1(lane_t + dcol + cb * 24 + 16, raw + 8);
-          tmem_ld16x256_x1(lane_t + dcol + 96 + cb * 8, raw + 12);
+          tmem_ld16x256_x2(lane_t + cb * 24, raw);
+          tmem_ld16x256_x1(lane_t + cb * 24 + 16, raw + 8);
+          tmem_ld16x256_x1(lane_t + 96 + cb * 8, raw + 12);
         }
         tmem_wait_ld();
         const bool fine = tl && warp == 0 && l == 2;
         if (fine) tl[1 + 4 * MAXL + 2] = clock64();
-        // 32-leaf tiles: the arithmetic of both rounds first (8 values per thread), then stores + fence per round;
-        // 64-leaf tiles (16 values per thread): round by round, or the packed results spill
+        // 32-leaf tiles: the arithmetic of both rounds first (8 values per thread), then stores + hand-off per round;
+        // 64-leaf tiles (16 values per thread): round by round, or the packed results spill.
+        // HALF: the rows without a leaf (rB) get zeros, so that the A operand holds finite values in every lane
         unsigned pa[G0 + G1], pb[G0 + G1];
         auto math = [&](int g) {
           const unsigned* rr = raw + 4 * g;
           pa[g] = pack_bf16(elu_fast(__uint_as_float(rr[0]) + bi[g].x), elu_fast(__uint_as_float(rr[1]) + bi[g].y));
           if constexpr (!HALF) pb[g] = pack_bf16(elu_fast(__uint_as_float(rr[2]) + bi[g].x), elu_fast(__uint_as_float(rr[3]) + bi[g].y));
+          else pb[g] = 0u;
         };
         if constexpr (HALF) {
 #pragma unroll
@@ -1323,15 +1350,13 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
 #pragma unroll
             for (int g = 0; g < (c ? G1 : G0); ++g) math((c ? G0 : 0) + g);
           }
-#pragma unroll
-          for (int g = 0; g < (c ? G1 : G0); ++g) {
-            const int col = (c ? R0 + cb * 8 * G1 : cb * 8 * G0) + g * 8 + cq;
-            a64_store2(sm.a, rA, col, pa[(c ? G0 : 0) + g]);
-            if constexpr (!HALF) a64_store2(sm.a, rB, col, pb[(c ? G0 : 0) + g]);
-          }
+          if (c == 0)
+            a64_tstore<G0>(a_t + cb * 4 * G0, pa, pb);
+          else
+            a64_tstore<G1>(a_t + R0 / 2 + cb * 4 * G1, pa + G0, pb + G0);
           if (fine) tl[1 + 4 * MAXL + 3 + 3 * c] = clock64();
-          fence_async_smem();
-          if (c == 1) tc_fence_before();
+          tmem_wait_st();
+          tc_fence_before();
           if (fine) tl[1 + 4 * MAXL + 4 + 3 * c] = clock64();
           nb_arrive(2 + c);
           if (fine) tl[1 + 4 * MAXL + 5 + 3 * c] = clock64();
@@ -1340,7 +1365,7 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
         // head layer: this warp owns the 32-column block cb of its 16 rows (fragment: 4 groups x {rowA, rowB} x 2 columns)
         const int c0 = cb * 32;
         unsigned raw[16];
-        tmem_ld16x256_x4(lane_t + dcol + c0, raw);
+        tmem_ld16x256_x4(lane_t + c0, raw);
         tmem_wait_ld();
         float xa[8], xb[8];
 #pragma unroll
@@ -1418,14 +1443,10 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
 #pragma unroll
           for (int g = 0; g < 4; ++g) {
             pend_a[g] = pack_bf16((xa[2 * g] - loa) * ia, (xa[2 * g + 1] - loa) * ia);
-            a64_store2(sm.a, rA, c0 + g * 8 + cq, pend_a[g]);
-            if constexpr (!HALF) {
-              pend_b[g] = pack_bf16((xb[2 * g] - lob) * ib, (xb[2 * g + 1] - lob) * ib);
-              a64_store2(sm.a, rB, c0 + g * 8 + cq, pend_b[g]);
-            } else {
-              pend_b[g] = 0u;
-            }
+            if constexpr (!HALF) pend_b[g] = pack_bf16((xb[2 * g] - lob) * ib, (xb[2 * g + 1] - lob) * ib);
+            else pend_b[g] = 0u;
           }
+          a64_tstore<4>(a_t + c0 / 2, pend_a, pend_b);
           have_pend = job.hidden16_dst != nullptr;
         } else if (soft_seg && (cb & 1) == 0) {
           if ((lane & 3) == 0) {
@@ -1477,7 +1498,7 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
           }
         }
         if (l + 1 < nl) {
-          fence_async_smem();
+          tmem_wait_st();
           tc_fence_before();
           for (int c = 0; c < 2; ++c) nb_arrive(2 + c);
         }

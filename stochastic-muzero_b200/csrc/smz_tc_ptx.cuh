@@ -1,6 +1,6 @@
 // smz_tc_ptx.cuh — PTX wrappers shared by the tensor-core network-step kernels (smz_net_bf16.cu, smz_net_tc32.cu):
-// mbarriers, bulk (TMA) copies, proxy / tcgen05 fences, UMMA shared-memory descriptors, tcgen05.commit, the
-// tcgen05.ld shapes the epilogues use, and the head-layer reductions (softmax expectation over the categorical
+// mbarriers, bulk (TMA) copies, proxy / tcgen05 fences, UMMA shared-memory descriptors, the tensor-memory-A form of
+// tcgen05.mma, tcgen05.commit, the tcgen05.ld / tcgen05.st shapes the epilogues use, and the head-layer reductions (softmax expectation over the categorical
 // support, muzero_model.py:575-591).
 #pragma once
 #include <cuda_bf16.h>
@@ -64,6 +64,17 @@ __device__ __forceinline__ bool elect_one() {
       "selp.u32 %0, 1, 0, p;\n\t}"
       : "=r"(pred));
   return pred != 0;
+}
+// tcgen05.mma kind::f16 with A read from tensor memory ("TS"): tmem_a = column (and lane 0) of the operand, which holds
+// row m of A in the lane of accumulator row m and two bf16 per 32-bit column (K index 2j in the low half of column j),
+// so a K = 16 step advances tmem_a by 8 columns.  B stays a shared-memory descriptor.
+__device__ __forceinline__ void umma_ts(unsigned tmem_d, unsigned tmem_a, unsigned long long bdesc, unsigned idesc, unsigned accum) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(tmem_d),
+      "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accum)
+      : "memory");
 }
 __device__ __forceinline__ void umma_commit(unsigned long long* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s32(bar)) : "memory");
@@ -166,6 +177,25 @@ __device__ __forceinline__ void tmem_ld16x256_x4(unsigned taddr, unsigned* r) {
       : "r"(taddr)
       : "memory");
 }
+
+// 16 lanes x (4 * X) columns, the store-side twin of the 16x256b fragment above for packed bf16 pairs: repetition i
+// writes r[2i] to lane t/4 and r[2i+1] to lane t/4 + 8, column 4i + t%4 (probe in tools/microbench/a_operand_handoff.cu,
+// result in profiles/r3_a_operand_handoff.txt).
+// No wait: pair with tmem_wait_st before the hand-off to the MMA issuer.
+__device__ __forceinline__ void tmem_st16x128_x1(unsigned taddr, unsigned r0, unsigned r1) {
+  asm volatile("tcgen05.st.sync.aligned.16x128b.x1.b32 [%0], {%1, %2};" ::"r"(taddr), "r"(r0), "r"(r1) : "memory");
+}
+__device__ __forceinline__ void tmem_st16x128_x2(unsigned taddr, const unsigned* r) {
+  asm volatile("tcgen05.st.sync.aligned.16x128b.x2.b32 [%0], {%1, %2, %3, %4};" ::"r"(taddr), "r"(r[0]), "r"(r[1]), "r"(r[2]),
+               "r"(r[3])
+               : "memory");
+}
+__device__ __forceinline__ void tmem_st16x128_x4(unsigned taddr, const unsigned* r) {
+  asm volatile("tcgen05.st.sync.aligned.16x128b.x4.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(r[0]), "r"(r[1]),
+               "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7])
+               : "memory");
+}
+__device__ __forceinline__ void tmem_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
 __device__ __forceinline__ SoftPart soft_merge(SoftPart a, SoftPart b) {
   const float m = fmaxf(a.m, b.m);
