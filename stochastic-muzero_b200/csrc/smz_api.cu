@@ -73,7 +73,7 @@ struct smz_engine {
   cudaGraphExec_t graph_exec;
   int graph_trees, graph_sims, graph_first, graph_launches;
   cudaStream_t capture_stream;
-  int use_pdl, use_fused_tree, use_mega;
+  int use_pdl;
 };
 
 const char* smz_last_error(void) { return g_err; }
@@ -150,10 +150,6 @@ int smz_create(const smz_config* cfg, smz_engine** out) {
   e->img32_buf = nullptr; e->blob_buf = nullptr; e->bf16 = nullptr; e->tc32 = nullptr; e->vision = nullptr;
   e->n_trees = 0; e->sims_done = 0; e->have_weights = 0; e->launches = 0; e->launches_total = 0;
   e->use_pdl = getenv("SMZ_NO_PDL") ? 0 : 1;
-  e->use_mega = getenv("SMZ_MEGA") ? 1 : 0;
-  // measured on B200 (4096 trees): the single-launch variant is ~4 % SLOWER than network kernel + tree kernel —
-  // 128 trees per SM on 33 SMs lose more to per-SM latency than the saved launch gains — so it is opt-in
-  e->use_fused_tree = getenv("SMZ_FUSED_TREE") ? 1 : 0;
   e->graph_exec = nullptr; e->graph_trees = e->graph_sims = e->graph_first = -1; e->capture_stream = nullptr;
 
   SmzArena& a = e->a;
@@ -432,9 +428,9 @@ int smz_select(smz_engine* e, int32_t sim, int32_t* slot, int32_t* action, int32
 }
 
 // returns the number of kernels launched
-static int enqueue_net(smz_engine* e, int sim, cudaStream_t s, bool pdl = false, int tree_mode = 0) {
+static int enqueue_net(smz_engine* e, int sim, cudaStream_t s, bool pdl = false) {
   if (e->vision) return smz_vision_sim(e->vision, e->a, e->n_trees, sim, pdl, s);
-  if (e->bf16) smz_bf16_sim(e->bf16, e->a, e->shape, e->n_trees, sim, pdl, tree_mode, s);
+  if (e->bf16) smz_bf16_sim(e->bf16, e->a, e->shape, e->n_trees, sim, pdl, s);
   else if (e->tc32) smz_tc32_sim(e->tc32, e->a, e->shape, e->n_trees, sim, pdl, s);
   else smz_net_f32_sim(e->a, e->shape, e->img32, e->n_trees, sim, s);
   return 1;
@@ -489,12 +485,8 @@ static int enqueue_sims(smz_engine* e, int first, int n_sims, cudaStream_t s) {
   const bool pdl = (e->bf16 != nullptr || e->tc32 != nullptr || smz_vision_has_tc(e->vision)) && e->use_pdl;
   smz_launch_select(a, G, e->n_trees, first, nullptr, nullptr, nullptr, s);
   int launched = 1;
-  // tensor-core network + 4 lanes per tree: the tree phases run in the tail of the network kernel (one launch
-  // per simulation); otherwise a second, fused tree kernel follows each network step
-  const bool fuse = e->bf16 != nullptr && G == 4 && e->use_fused_tree;
   for (int sim = first; sim < first + n_sims; ++sim) {
     const bool last = sim + 1 >= first + n_sims;
-    if (fuse) { launched += enqueue_net(e, sim, s, pdl, last ? 1 : 2); continue; }
     launched += enqueue_net(e, sim, s, pdl) + 1;
     if (!last) smz_launch_backup_select(a, G, e->n_trees, sim, pdl, s);
     else smz_launch_expand_backup(a, G, e->n_trees, sim, a.out_policy, a.W, a.out_value, a.out_reward, s);
@@ -513,14 +505,6 @@ int smz_simulate(smz_engine* e, int32_t n_sims, void* stream) {
   cudaStream_t s = (cudaStream_t)stream;
   ON_DEVICE(e);
   const int first = e->sims_done;
-  if (e->use_mega && smz_bf16_mega_supported(e->bf16, e->a, e->cfg.lanes_per_tree)) {
-    // tensor-core network + narrow policies: one persistent launch runs the whole loop, tile by tile
-    smz_bf16_mega(e->bf16, e->a, e->shape, e->n_trees, first, n_sims, s);
-    CU(cudaGetLastError());
-    count_launches(e, 1);
-    e->sims_done += n_sims;
-    return SMZ_OK;
-  }
   // The N-step loop is launch-bound: capture it once per (trees, first, count) into a CUDA graph and
   // replay it on the caller's stream.
   if (!e->graph_exec || e->graph_trees != e->n_trees || e->graph_sims != n_sims || e->graph_first != first) {

@@ -23,8 +23,8 @@
 
 #include "../../include/smz.h"
 #include "smz_net_bf16.h"
+#include "smz_common.cuh"
 #include "smz_tc_ptx.cuh"
-#include "smz_tree_dev.cuh"
 
 namespace {
 
@@ -86,7 +86,6 @@ struct Smem {
   unsigned long long bbar;
   unsigned int tmem_base;
   float4 part[4][TM];       // per-row partial reductions of the head epilogues, one slot per column block
-  int rowtree[TM];          // tree id of every row of the tile (-1 = none): the fused tree phase works on these
 };
 
 // InstrDescriptor: D=f32 (bit 4), A=B=bf16 (bits 7, 10), both K-major, N>>3 at [17,23), M>>4 at [24,29)
@@ -113,16 +112,137 @@ __device__ __forceinline__ void a_store(unsigned char* a, int r, int kchunk, uin
 // the bf16 rounding the result gets next)
 __device__ __forceinline__ float elu_fast(float x) { return x > 0.f ? x : ex2f(x * 1.4426950408889634f) - 1.f; }
 
+// bulk copy of the weight tile of layer l of chain c into ring slot `slot` (w[slot]), completion on wbar[slot]
+__device__ __forceinline__ void load_weight_tile(const Chain& c, int l, unsigned long long* wbar, unsigned char (*w)[W_BYTES], int slot) {
+  const unsigned bytes = (unsigned)c.layer[l].K * TN * 2;
+  mbar_expect_tx(&wbar[slot], bytes);
+  bulk_g2s(w[slot], c.layer[l].w, bytes, &wbar[slot]);
+}
+
+// K-chunk kc (8 columns) of the one-hot block of a row whose action / code is act (-1 = none)
+__device__ __forceinline__ uint4 onehot_chunk(int act, int kc) {
+  unsigned w4[4] = {0, 0, 0, 0};
+  if (act >= kc * 8 && act < kc * 8 + 8) {
+    const int j = act - kc * 8;
+    w4[j >> 1] = (j & 1) ? 0x3F800000u : 0x00003F80u;   // bf16 1.0 in the high / low half
+  }
+  return make_uint4(w4[0], w4[1], w4[2], w4[3]);
+}
+
+// A CTA with nothing to do: it must not exit while a bulk copy into its shared memory is still in flight, so thread 0
+// waits for every copy it has issued (bbar: the bias table, or null; wbar[0] and, if wbar1, wbar[1]: the first weight
+// tiles); then the TMEM allocation is given back.
+__device__ __forceinline__ void idle_cta_exit(unsigned long long* bbar, unsigned long long* wbar, bool wbar1,
+                                              const unsigned& tmem_base, unsigned ncols) {
+  if (threadIdx.x == 0) {
+    if (bbar) mbar_wait(bbar, 0);
+    mbar_wait(&wbar[0], 0);
+    if (wbar1) mbar_wait(&wbar[1], 0);
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
+  if (threadIdx.x < 32) tmem_dealloc(tmem_base, ncols);
+}
+
+// ---- the head layer of a 128-row tile: thread (row r, column block cb) holds the 32 biased logits x of columns
+//      32cb .. 32cb+31.  Columns [0,64) = state or value logits, [64,128) = reward or policy logits.  Row-wise
+//      reductions span two column blocks: head_partials leaves this thread's partials in part[cb][r], the caller
+//      synchronises, head_finish combines them.
+__device__ __forceinline__ bool head_state_seg(int kind, int cb) { return (kind == LK_STATE || kind == LK_STATE_REWARD) && cb < 2; }
+__device__ __forceinline__ bool head_soft_seg(int kind, int cb) {
+  return (kind == LK_STATE_REWARD && cb >= 2) || (kind == LK_PRED && cb < 2);
+}
+
+__device__ __forceinline__ SoftPart head_partials(const float* x, int kind, int cb, int r, int S, float4 (*part)[TM]) {
+  SoftPart sp{-1e30f, 0.f, 0.f};
+  if (head_state_seg(kind, cb)) {
+    float lo = INFINITY, hi = -INFINITY;
+#pragma unroll
+    for (int j = 0; j < 32; ++j)
+      { lo = fminf(lo, x[j]); hi = fmaxf(hi, x[j]); }   // padded columns replicate column 0 (weight image)
+    part[cb][r] = make_float4(lo, hi, 0.f, 0.f);
+  } else if (head_soft_seg(kind, cb)) {
+    sp = soft_part(x, (cb * 32) & 63, S);
+    part[cb][r] = make_float4(sp.m, sp.z, sp.y, 0.f);
+  }
+  return sp;
+}
+
+// the bf16 state row piece of a head layer, whose global store the caller defers past its barrier (the proxy fence
+// before it would otherwise wait for the store to land)
+struct HeadStores {
+  uint4 v[4];
+  uint4* dst;               // -> the arena's bf16 hidden store, or null
+  __device__ __forceinline__ void flush() const {
+    if (dst) {             // the arena keeps hidden states in bf16: exactly what the next gather needs
+#pragma unroll
+      for (int q = 0; q < 4; ++q) dst[q] = v[q];
+    }
+  }
+};
+
+// second half: the state head becomes the next network's A operand (A: the tile's shared-memory operand) and leaves
+// the normalised state in x, the value / reward head its scalar, the policy / code head its softmax (+ argmax for
+// LK_CODE); index = output row (-1 = none)
+__device__ __forceinline__ HeadStores head_finish(float* x, int kind, int cb, int r, SoftPart sp, const float4 (*part)[TM],
+                                                  unsigned char* A, int index, const Job& job, int n_policy) {
+  HeadStores st;
+  st.dst = nullptr;
+  const int c0 = cb * 32;
+  if (head_state_seg(kind, cb)) {
+    // scale_to_bound_action (mlp:349-357): bf16 copy to HBM and into the next network's A operand
+    const float4 o = part[cb ^ 1][r];
+    const float lo = fminf(part[cb][r].x, o.x), hi = fmaxf(part[cb][r].y, o.y);
+    float scale = hi - lo;
+    if (scale < 1e-5f) scale += 1e-5f;
+    const float inv = 1.f / scale;
+#pragma unroll
+    for (int j = 0; j < 32; ++j) x[j] = (x[j] - lo) * inv;   // padded columns: finite copies, zero weights next
+    if (index >= 0 && job.hidden16_dst) st.dst = reinterpret_cast<uint4*>(job.hidden16_dst + (size_t)index * SMZ_SP + c0);
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      st.v[q] = make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
+                           pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7]));
+      a_store(A, r, cb * 4 + q, st.v[q]);
+    }
+  } else if (head_soft_seg(kind, cb) && (cb & 1) == 0) {
+    const float4 o = part[cb + 1][r];
+    const float v = support_scalar(sp, SoftPart{o.x, o.y, o.z});
+    float* dst = (kind == LK_PRED) ? job.value_dst : job.reward_dst;
+    if (index >= 0 && dst) dst[index] = v;
+  } else if ((kind == LK_PRED && cb == 2) || (kind == LK_CODE && cb == 0)) {
+    // policy softmax (muzero_model.py:837) / Encoder code distribution + argmax (mlp:209-250)
+    float m = -1e30f, z = 0.f;
+    int best = 0;
+#pragma unroll
+    for (int i = 0; i < 32; ++i)
+      if (x[i] > m) { m = x[i]; best = i; }             // padded logits sit at -1e30 (bias)
+#pragma unroll
+    for (int i = 0; i < 32; ++i) {
+      x[i] = ex2f((x[i] - m) * 1.4426950408889634f);
+      z += x[i];
+    }
+    if (index >= 0) {
+      if (job.policy_dst) {
+        float* dst = job.policy_dst + (size_t)index * job.pstride;
+        const float inv = 1.f / z;
+#pragma unroll
+        for (int i = 0; i < 32; ++i)
+          if (i < n_policy) dst[i] = x[i] * inv;
+      }
+      if (kind == LK_CODE && job.code_dst) job.code_dst[index] = best;
+    }
+  }
+  return st;
+}
+
 
 // ---------------------------------------------------------------------------------------------
 // the fused chain kernel: 512 threads = 16 warps; warp w owns TMEM lanes 32*(w%4).. (rows) and the
 // 32 accumulator columns 32*(w/4).. of every layer, so each SM sub-partition always has 4 warps to
 // interleave around the TMEM-load / MUFU latencies.
 // ---------------------------------------------------------------------------------------------
-// TREE = 0: network step only.  TREE = 1 / 2: the CTA also runs, for the 128 trees of its tile (4 lanes per
-// tree), the expansion + backup of simulation `sim` (1) and then the descent of simulation `sim + 1` (2) —
-// one launch per simulation instead of two, no second kernel ramp-up, outputs re-read from L1/L2.
-template <int TREE>
 __global__ void __launch_bounds__(NTHREADS, 1)
 k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   extern __shared__ unsigned char smem_raw[];
@@ -146,11 +266,6 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
 
   // ---- barriers + first weight tiles (one thread), TMEM allocation (warp 0): all of it overlaps the
   //      dependent global loads of the gather below; one barrier publishes everything ----------------
-  auto load_weights = [&](int l) {
-    const unsigned bytes = (unsigned)ch.layer[l].K * TN * 2;
-    mbar_expect_tx(&sm.wbar[l & 1], bytes);
-    bulk_g2s(sm.w[l & 1], ch.layer[l].w, bytes, &sm.wbar[l & 1]);
-  };
   if (tid == 0) {
     mbar_init(&sm.wbar[0], 1);
     mbar_init(&sm.wbar[1], 1);
@@ -160,15 +275,11 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
     const unsigned bbytes = (unsigned)ch.n_layers * TN * 4;
     mbar_expect_tx(&sm.bbar, bbytes);
     bulk_g2s(sm.bias, ch.bias, bbytes, &sm.bbar);
-    load_weights(0);
-    if (ch.n_layers > 1) load_weights(1);
+    load_weight_tile(ch, 0, sm.wbar, sm.w, 0);
+    if (ch.n_layers > 1) load_weight_tile(ch, 1, sm.wbar, sm.w, 1);
   }
   __syncwarp();
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(&sm.tmem_base)), "r"(TN)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 0) tmem_alloc(&sm.tmem_base, TN);
 
   // ---- everything above is independent of the previous kernel; from here on we read its results ---
   smz_pdl_wait();
@@ -179,17 +290,8 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   if (job.input_kind == IN_GATHER) count = a.branch_count[sim * 2 + branch];
   const int row = tile * TM + r;
   const bool valid = row < count;
-  if (tile * TM >= count) {        // nothing to do for this CTA: drain the prefetches, give TMEM back, leave
-    if (tid == 0) {
-      mbar_wait(&sm.bbar, 0);
-      mbar_wait(&sm.wbar[0], 0);
-      if (ch.n_layers > 1) mbar_wait(&sm.wbar[1], 0);
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    if (warp == 0)
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(sm.tmem_base), "r"(TN) : "memory");
+  if (tile * TM >= count) {
+    idle_cta_exit(&sm.bbar, sm.wbar, ch.n_layers > 1, sm.tmem_base, TN);
     return;
   }
 
@@ -236,17 +338,9 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
         }
         a_store(sm.a, r, kc, o);
       }
-      for (int kc = cb; kc < ch.onehot_pad / 8; kc += 4) {   // one-hot columns 64 + act
-        unsigned w4[4] = {0, 0, 0, 0};
-        if (valid && act >= kc * 8 && act < kc * 8 + 8) {
-          const int j = act - kc * 8;
-          w4[j >> 1] = (j & 1) ? 0x3F800000u : 0x00003F80u;   // bf16 1.0 in the high / low half
-        }
-        a_store(sm.a, r, 8 + kc, make_uint4(w4[0], w4[1], w4[2], w4[3]));
-      }
+      for (int kc = cb; kc < ch.onehot_pad / 8; kc += 4) a_store(sm.a, r, 8 + kc, onehot_chunk(act, kc));   // columns 64 + act
     }
   }
-  if (cb == 0) sm.rowtree[r] = index;
   fence_async_smem();
   tc_fence_before();
   __syncthreads();
@@ -281,12 +375,12 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
     __syncwarp();       // tcgen05.ld below is .sync.aligned: reconverge after the spin loop
     if (stamp) job.timeline[1 + l * 4 + 2] = clock64();
     tc_fence_after();
-    if (tid == 0 && l + 2 < ch.n_layers) load_weights(l + 2);   // ring slot l&1 is free again
+    if (tid == 0 && l + 2 < ch.n_layers) load_weight_tile(ch, l + 2, sm.wbar, sm.w, l & 1);   // ring slot l&1 is free again
     __syncwarp();
     const float* bias = sm.bias[l] + c0;
 
-    uint4 pend[4];                 // bf16 row pieces whose global store is deferred past the barrier
-    uint4* pend_dst = nullptr;
+    HeadStores pend;              // global stores deferred past the barrier
+    pend.dst = nullptr;
     float4* pend32_dst = nullptr;
     float x[32];
     {
@@ -316,70 +410,14 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
                 make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
                            pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7])));
     } else {
-      // head layer: columns [0,64) = state or value logits, [64,128) = reward or policy logits.
-      // Row-wise reductions span two column blocks: partials meet in shared memory.
-      const bool state_seg = (kind == LK_STATE || kind == LK_STATE_REWARD) && cb < 2;
-      const bool soft_seg = (kind == LK_STATE_REWARD && cb >= 2) || (kind == LK_PRED && cb < 2);
-      SoftPart sp{-INFINITY, 0.f, 0.f};
-      if (state_seg) {
-        float lo = INFINITY, hi = -INFINITY;
-#pragma unroll
-        for (int j = 0; j < 32; ++j)
-          { lo = fminf(lo, x[j]); hi = fmaxf(hi, x[j]); }   // padded columns replicate column 0 (weight image)
-        sm.part[cb][r] = make_float4(lo, hi, 0.f, 0.f);
-      } else if (soft_seg) {
-        sp = soft_part(x, c0 & 63, S);
-        sm.part[cb][r] = make_float4(sp.m, sp.z, sp.y, 0.f);
-      }
+      const SoftPart sp = head_partials(x, kind, cb, r, S, sm.part);
       if (hs) hs[1] = clock64();
       __syncthreads();
       if (hs) hs[2] = clock64();
-      if (state_seg) {
-        // scale_to_bound_action (mlp:349-357): fp32 copy to HBM, bf16 copy = the next network's A operand
-        const float4 o = sm.part[cb ^ 1][r];
-        const float lo = fminf(sm.part[cb][r].x, o.x), hi = fmaxf(sm.part[cb][r].y, o.y);
-        float scale = hi - lo;
-        if (scale < 1e-5f) scale += 1e-5f;
-        const float inv = 1.f / scale;
-#pragma unroll
-        for (int j = 0; j < 32; ++j) x[j] = (x[j] - lo) * inv;   // padded columns: finite copies, zero weights next
-        if (index >= 0 && job.hidden_dst) pend32_dst = reinterpret_cast<float4*>(job.hidden_dst + (size_t)index * SMZ_SP + c0);
-        if (index >= 0 && job.hidden16_dst) pend_dst = reinterpret_cast<uint4*>(job.hidden16_dst + (size_t)index * SMZ_SP + c0);
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          pend[q] = make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
-                               pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7]));
-          a_store(sm.a, r, cb * 4 + q, pend[q]);
-        }
-      } else if (soft_seg && (cb & 1) == 0) {
-        const float4 o = sm.part[cb + 1][r];
-        const float v = support_scalar(sp, SoftPart{o.x, o.y, o.z});
-        float* dst = (kind == LK_PRED) ? job.value_dst : job.reward_dst;
-        if (index >= 0 && dst) dst[index] = v;
-      } else if ((kind == LK_PRED && cb == 2) || (kind == LK_CODE && cb == 0)) {
-        // policy softmax (muzero_model.py:837) / Encoder code distribution + argmax (mlp:209-250)
-        const int n = ch.n_policy;
-        float m = -1e30f, z = 0.f;
-        int best = 0;
-#pragma unroll
-        for (int i = 0; i < 32; ++i)
-          if (x[i] > m) { m = x[i]; best = i; }             // padded logits sit at -1e30 (bias)
-#pragma unroll
-        for (int i = 0; i < 32; ++i) {
-          x[i] = ex2f((x[i] - m) * 1.4426950408889634f);
-          z += x[i];
-        }
-        if (index >= 0) {
-          if (job.policy_dst) {
-            float* dst = job.policy_dst + (size_t)index * job.pstride;
-            const float inv = 1.f / z;
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (i < n) dst[i] = x[i] * inv;
-          }
-          if (kind == LK_CODE && job.code_dst) job.code_dst[index] = best;
-        }
-      }
+      pend = head_finish(x, kind, cb, r, sp, sm.part, sm.a, index, job, ch.n_policy);
+      // stand-alone evaluation (only this kernel serves it) also returns the normalised state in fp32
+      if (head_state_seg(kind, cb) && index >= 0 && job.hidden_dst)
+        pend32_dst = reinterpret_cast<float4*>(job.hidden_dst + (size_t)index * SMZ_SP + cb * 32);
     }
     if (hs) hs[3] = clock64();
     // make the new A operand visible to the tensor core (async proxy) and retire the TMEM reads.
@@ -390,10 +428,7 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
       __syncthreads();
     }
     if (hs) hs[4] = clock64();
-    if (pend_dst) {           // the arena keeps hidden states in bf16: exactly what the next gather needs
-#pragma unroll
-      for (int q = 0; q < 4; ++q) pend_dst[q] = pend[q];
-    }
+    pend.flush();
     if (pend32_dst) {
 #pragma unroll
       for (int q = 0; q < 8; ++q) pend32_dst[q] = make_float4(x[q * 4], x[q * 4 + 1], x[q * 4 + 2], x[q * 4 + 3]);
@@ -403,24 +438,7 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
 
   tc_fence_before();
   __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TN) : "memory");
-  }
-  if constexpr (TREE > 0) {
-    // ---- tree phase for the trees of this tile: 4 lanes per tree, the policy / value / reward just written by
-    //      this CTA are visible after the barrier above ---------------------------------------------------------
-    using namespace smz_tree_dev;
-    Group<4> g;
-    int tree = sm.rowtree[tid >> 2];
-    const bool alive = tree >= 0;
-    if (!alive) tree = 0;
-    const SmzRng rng = smz_make_rng(a);
-    const TreeState ts = expand_backup_phase(g, a, rng, tree, alive, sim, a.out_policy, a.W, a.out_value, a.out_reward);
-    if constexpr (TREE > 1) {
-      __syncwarp();
-      select_phase(g, a, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr);
-    }
-  }
+  if (warp == 0) tmem_dealloc(tmem, TN);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -459,10 +477,109 @@ __device__ __forceinline__ void epi_sync() { __syncwarp(); asm volatile("bar.syn
 __device__ __forceinline__ void nb_arrive(int id) { __syncwarp(); asm volatile("bar.arrive %0, %1;" ::"r"(id), "n"(NPIPE) : "memory"); }
 __device__ __forceinline__ void nb_sync(int id) { __syncwarp(); asm volatile("bar.sync %0, %1;" ::"r"(id), "n"(NPIPE) : "memory"); }
 
-// NR = rounds per hidden layer: 2 = 64-column rounds, 16-column slices per warp (default: every round costs a proxy
-// fence, two rounds measured best); 4 = 32-column rounds, 8-column slices.  An uneven 96 + 32 split (fewer K-steps
-// left after the last round) measured slower than 64 + 64.
-template <int NR>
+// Row record {tree, parent slot, action, -} of position pos of the simulation's row array, and the NC 16-byte chunks
+// kc0 .. kc0+NC-1 of the parent's bf16 hidden row: copied next to the record by the descent (a.xin: one dependent load
+// less), else gathered from the arena.  Positions beyond the live rows hold stale but in-range records (zeroed at create).
+template <int NC>
+__device__ __forceinline__ int4 load_row(const SmzArena& a, int sim, int pos, int kc0, uint4* hrow) {
+  const size_t ri = (size_t)(sim & 1) * a.row_cap + pos;
+  int4 rec = a.rows4[ri];
+  if (a.xin) {
+#pragma unroll
+    for (int q = 0; q < NC; ++q) hrow[q] = a.xin[ri * 8 + kc0 + q];
+  } else {
+    rec.x = min(max(rec.x, 0), a.B - 1);
+    rec.y = min(max(rec.y, 0), a.N);
+    const __nv_bfloat16* src16 = reinterpret_cast<const __nv_bfloat16*>(a.hidden) + ((size_t)rec.y * a.B + rec.x) * SMZ_SP;
+#pragma unroll
+    for (int q = 0; q < NC; ++q) hrow[q] = *reinterpret_cast<const uint4*>(src16 + (kc0 + q) * 8);
+  }
+  return rec;
+}
+
+// The issuer warp's weight ring: layer l of the CTA's chain lives in slot (l + branch) & 1 (layer 0 of chain b was
+// prefetched into slot b before the branch was known).  The hidden layers of a network share ONE weight tile (the
+// reference ties them, mlp:31-37): a tile that is already resident in its slot is not streamed again — 6 bulk copies
+// per chain instead of 12.  nfill / nseen = fills issued to / waited for on each slot.  Every counter and resident-tile
+// pointer is a scalar member, kept in registers (an indexed array would not be).  The whole warp calls every method;
+// lane 0 issues the copies.
+struct WeightRing {
+  const Chain& ch;
+  unsigned long long* wbar;       // [2]
+  unsigned char (*w)[W_BYTES];    // [2]
+  int branch, lane;
+  unsigned nfill0, nfill1, nseen0, nseen1;
+  const __nv_bfloat16 *res0, *res1;
+
+  __device__ __forceinline__ WeightRing(const Chain& c, unsigned long long* bars, unsigned char (*slots)[W_BYTES], int lane_)
+      : ch(c), wbar(bars), w(slots), branch(0), lane(lane_), nfill0(1u), nfill1(1u), nseen0(0u), nseen1(0u),
+        res0(nullptr), res1(nullptr) {}
+  // slot `branch` holds layer 0 (fill 0); the other slot's fill 0 was the unused chain's layer 0: layer 1 replaces it
+  // as soon as it has landed
+  __device__ __forceinline__ void start(int branch_, int nl) {
+    branch = branch_;
+    if (branch) res1 = ch.layer[0].w; else res0 = ch.layer[0].w;
+    if (nl > 1) {
+      const int s1 = branch ^ 1;
+      mbar_wait(&wbar[s1], 0);
+      if (lane == 0) load_weight_tile(ch, 1, wbar, w, s1);
+      if (s1) { nseen1 = 1u; nfill1 = 2u; res1 = ch.layer[1].w; } else { nseen0 = 1u; nfill0 = 2u; res0 = ch.layer[1].w; }
+      __syncwarp();
+    }
+  }
+  // the slot of layer l, once its tile has landed
+  __device__ __forceinline__ int wait(int l) {
+    const int slot = (l + branch) & 1;
+    const unsigned seen = slot ? nseen1 : nseen0;
+    if (seen < (slot ? nfill1 : nfill0)) {
+      mbar_wait(&wbar[slot], seen & 1u);
+      if (slot) ++nseen1; else ++nseen0;
+    }
+    return slot;
+  }
+  // layer l + 2 goes into the slot of layer l — unless it is resident there already (stream_all: always) — once the
+  // MMAs that read that slot have completed: mbarrier `done`, phase `parity`
+  __device__ __forceinline__ void refill(int l, int nl, bool stream_all, unsigned long long* done, unsigned parity) {
+    const int slot = (l + branch) & 1;
+    if (l + 2 < nl && ((slot ? res1 : res0) != ch.layer[l + 2].w || stream_all)) {
+      mbar_wait(done, parity);
+      if (lane == 0) load_weight_tile(ch, l + 2, wbar, w, slot);
+      if (slot) { ++nfill1; res1 = ch.layer[l + 2].w; } else { ++nfill0; res0 = ch.layer[l + 2].w; }
+      __syncwarp();
+    }
+  }
+};
+
+// Hidden layer of a 128-row tile in NR = 2 rounds of 64 columns (every round costs a proxy fence; two rounds measured
+// best): this warp owns a 16-column slice of every round for its 32 rows.  All slices are requested at once (one exposed
+// TMEM latency per layer); each round then goes bias + ELU -> bf16 -> A operand and is handed to the issuer through
+// named barrier bar0 + round.  taddr: TMEM lane address of the tile's accumulator; bias: the layer's bias row.
+constexpr int NR = 2;
+__device__ __forceinline__ void hidden_rounds(unsigned char* A, unsigned taddr, const float* bias, int bar0, int r, int cb) {
+  constexpr int SL = 32 / NR;              // slice width: 16 columns
+  constexpr int RC = TN / NR;              // columns per round
+  const int j0 = cb * SL;
+  unsigned raw[NR][SL];
+#pragma unroll
+  for (int c = 0; c < NR; ++c) tmem_ld16_nowait(taddr + c * RC + j0, raw[c]);
+  tmem_wait_ld();
+#pragma unroll
+  for (int c = 0; c < NR; ++c) {
+    const float* b = bias + c * RC + j0;
+    float x[SL];
+#pragma unroll
+    for (int i = 0; i < SL; ++i) x[i] = elu_fast(__uint_as_float(raw[c][i]) + b[i]);
+#pragma unroll
+    for (int q = 0; q < SL / 8; ++q)
+      a_store(A, r, (c * RC + j0) / 8 + q,
+              make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
+                         pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7])));
+    fence_async_smem();
+    if (c == NR - 1) tc_fence_before();
+    nb_arrive(bar0 + c);
+  }
+}
+
 __global__ void __launch_bounds__(NPIPE, 1)
 k_bf16_chain_pipe(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   extern __shared__ unsigned char smem_raw[];
@@ -470,7 +587,7 @@ k_bf16_chain_pipe(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const bool is_issuer_warp = warp == NEPI / 32;
   const int r = (warp & 3) * 32 + lane;   // epilogue role: row of the tile == TMEM lane
-  const int cb = (warp >> 2) & 3;         // head layers: 32-column block; hidden layers: 8-column slice of a round
+  const int cb = (warp >> 2) & 3;         // head layers: 32-column block; hidden layers: 16-column slice of a round
 
   // CTA i owns positions [i * 128, (i + 1) * 128) of the simulation's row array (smz_common.cuh): afterstate rows from the
   // bottom, dynamics rows from the top, never both in one tile — no CTA is launched for an empty tile of the other branch
@@ -479,11 +596,6 @@ k_bf16_chain_pipe(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   long long* tl = (job.timeline && blockIdx.x == 0 && lane == 0) ? job.timeline : nullptr;   // debug stamps
   if (tl && tid == 0) tl[0] = clock64();
 
-  auto load_weights = [&](const Chain& c, int l, int slot) {
-    const unsigned bytes = (unsigned)c.layer[l].K * TN * 2;
-    mbar_expect_tx(&sm.wbar[slot], bytes);
-    bulk_g2s(sm.w[slot], c.layer[l].w, bytes, &sm.wbar[slot]);
-  };
   if (tid == 0) {
     mbar_init(&sm.wbar[0], 1); mbar_init(&sm.wbar[1], 1);
     mbar_init(&sm.dbar[0], 1); mbar_init(&sm.dbar[1], 1);
@@ -493,52 +605,25 @@ k_bf16_chain_pipe(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
     mbar_expect_tx(&sm.bbar, 2 * bbytes);
     bulk_g2s(sm.bias[0], chain0.bias, bbytes, &sm.bbar);
     bulk_g2s(sm.bias[1], chain1.bias, bbytes, &sm.bbar);
-    load_weights(chain0, 0, 0);              // the first weight tile of BOTH chains: the branch is not known yet
-    load_weights(chain1, 0, 1);
+    load_weight_tile(chain0, 0, sm.wbar, sm.w, 0);   // the first weight tile of BOTH chains: the branch is not known yet
+    load_weight_tile(chain1, 0, sm.wbar, sm.w, 1);
   }
   __syncwarp();
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(&sm.tmem_base)), "r"(2 * TN)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 0) tmem_alloc(&sm.tmem_base, 2 * TN);
   smz_pdl_wait();
   // only now may the tree kernel of this simulation start: its prologue mirrors the tree arena into shared memory,
   // which the PREVIOUS tree kernel (complete once the wait above returns) was still writing
   smz_pdl_launch_dependents();
-  // The row record and the parent's hidden row are requested together with the branch counts (one L2 round trip):
-  // positions beyond the live rows hold stale but in-range records (zeroed at create).
+  // The row record and the parent's hidden row are requested together with the branch counts (one L2 round trip).
   int4 rec = make_int4(0, 0, 0, 0);
   uint4 hrow[2] = {make_uint4(0, 0, 0, 0), make_uint4(0, 0, 0, 0)};
   const int pos = tile * TM + r;
-  if (!is_issuer_warp) {
-    const size_t ri = (size_t)(sim & 1) * a.row_cap + pos;
-    rec = a.rows4[ri];
-    if (a.xin) {
-#pragma unroll
-      for (int q = 0; q < 2; ++q) hrow[q] = a.xin[ri * 8 + cb * 2 + q];   // copied by the descent: one dependent load less
-    } else {
-      rec.x = min(max(rec.x, 0), a.B - 1);
-      rec.y = min(max(rec.y, 0), a.N);
-      const __nv_bfloat16* src16 = reinterpret_cast<const __nv_bfloat16*>(a.hidden) + ((size_t)rec.y * a.B + rec.x) * SMZ_SP;
-#pragma unroll
-      for (int q = 0; q < 2; ++q) hrow[q] = *reinterpret_cast<const uint4*>(src16 + (cb * 2 + q) * 8);
-    }
-  }
+  if (!is_issuer_warp) rec = load_row<2>(a, sim, pos, cb * 2, hrow);
   const int count0 = a.branch_count[sim * 2], count1 = a.branch_count[sim * 2 + 1];
   const int top1 = a.row_top - count1;      // dynamics rows occupy [top1, row_top)
   const int branch = tile * TM < count0 ? 0 : ((tile + 1) * TM > top1 ? 1 : -1);
-  if (branch < 0) {                // nothing to do for this CTA: drain the prefetches, give TMEM back, leave
-    if (tid == 0) {
-      mbar_wait(&sm.bbar, 0);
-      mbar_wait(&sm.wbar[0], 0);
-      mbar_wait(&sm.wbar[1], 0);
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    if (warp == 0)
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(sm.tmem_base), "r"(2 * TN) : "memory");
+  if (branch < 0) {
+    idle_cta_exit(&sm.bbar, sm.wbar, true, sm.tmem_base, 2 * TN);
     return;
   }
   const Chain& ch = branch ? chain1 : chain0;
@@ -551,26 +636,11 @@ k_bf16_chain_pipe(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   if (is_issuer_warp) {
     // =========================== issuer warp: weights ring + tcgen05.mma =======================================
     const unsigned long long ad = umma_desc(s32(sm.a), CHUNK_A, 128);
-    // weight ring: layer l lives in slot (l + branch) & 1 (layer 0 of chain b was prefetched into slot b); a tile that is
-    // already resident in its slot (the tied hidden layers) is not streamed again.  nfill / nseen = fills issued to /
-    // waited for on each slot.
-    unsigned nfill0 = 1u, nfill1 = 1u, nseen0 = 0u, nseen1 = 0u;        // per slot, kept in registers (no indexed arrays)
-    const __nv_bfloat16 *res0 = branch ? nullptr : ch.layer[0].w, *res1 = branch ? ch.layer[0].w : nullptr;
-    if (nl > 1) {                              // layer 1 replaces the unused chain's prefetched tile
-      const int s1 = branch ^ 1;
-      mbar_wait(&sm.wbar[s1], 0);
-      if (lane == 0) load_weights(ch, 1, s1);
-      if (s1) { nseen1 = 1u; nfill1 = 2u; res1 = ch.layer[1].w; } else { nseen0 = 1u; nfill0 = 2u; res0 = ch.layer[1].w; }
-      __syncwarp();
-    }
+    WeightRing ring(ch, sm.wbar, sm.w, lane);
+    ring.start(branch, nl);
     for (int l = 0; l < nl; ++l) {
       const int nk = ch.layer[l].K / 16;
-      const int slot = (l + branch) & 1;
-      const unsigned seen = slot ? nseen1 : nseen0;
-      if (seen < (slot ? nfill1 : nfill0)) {
-        mbar_wait(&sm.wbar[slot], seen & 1u);
-        if (slot) ++nseen1; else ++nseen0;
-      }
+      const int slot = ring.wait(l);
       const unsigned long long bd = umma_desc(s32(sm.w[slot]), CHUNK_W, 128);
       const unsigned d = tmem + (unsigned)((l & 1) * TN);
       for (int c = 0; c < NR; ++c) {
@@ -591,12 +661,7 @@ k_bf16_chain_pipe(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
       if (lane == 0) umma_commit(&sm.dbar[l & 1]);
       if (tl) tl[1 + l * 4 + 1] = clock64();
       __syncwarp();
-      if (l + 2 < nl && ((slot ? res1 : res0) != ch.layer[l + 2].w || job.stream_all)) {
-        mbar_wait(&sm.dbar[l & 1], (l >> 1) & 1);   // the slot is reusable once these MMAs have completed
-        if (lane == 0) load_weights(ch, l + 2, slot);
-        if (slot) { ++nfill1; res1 = ch.layer[l + 2].w; } else { ++nfill0; res0 = ch.layer[l + 2].w; }
-        __syncwarp();
-      }
+      ring.refill(l, nl, job.stream_all, &sm.dbar[l & 1], (l >> 1) & 1);   // the slot is reusable once these MMAs have completed
     }
   } else {
     // =========================== epilogue warps =================================================================
@@ -607,14 +672,7 @@ k_bf16_chain_pipe(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
       const int act = valid ? rec.z : -1;
 #pragma unroll
       for (int q = 0; q < 2; ++q) a_store(sm.a, r, cb * 2 + q, valid ? hrow[q] : make_uint4(0, 0, 0, 0));
-      for (int kc = cb; kc < ch.onehot_pad / 8; kc += 4) {
-        unsigned w4[4] = {0, 0, 0, 0};
-        if (valid && act >= kc * 8 && act < kc * 8 + 8) {
-          const int j = act - kc * 8;
-          w4[j >> 1] = (j & 1) ? 0x3F800000u : 0x00003F80u;
-        }
-        a_store(sm.a, r, 8 + kc, make_uint4(w4[0], w4[1], w4[2], w4[3]));
-      }
+      for (int kc = cb; kc < ch.onehot_pad / 8; kc += 4) a_store(sm.a, r, 8 + kc, onehot_chunk(act, kc));
     }
     fence_async_smem();
     for (int c = 0; c < NR; ++c) nb_arrive(2 + c);
@@ -630,118 +688,37 @@ k_bf16_chain_pipe(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
       __syncwarp();
       tc_fence_after();
       if (kind == LK_HIDDEN) {
-        // NR rounds of 128/NR columns; this warp owns a (32/NR)-column slice of every round for its 32 rows
-        constexpr int SL = 32 / NR;              // slice width: 8 or 16 columns
-        constexpr int RC = TN / NR;              // columns per round
-        const int j0 = cb * SL;
-        unsigned raw[NR][SL];
-        // all slices are requested at once (one exposed TMEM latency per layer)
-#pragma unroll
-        for (int c = 0; c < NR; ++c) {
-          if constexpr (NR == 4) tmem_ld8_nowait(lane_t + dcol + c * RC + j0, raw[c]);
-          else tmem_ld16_nowait(lane_t + dcol + c * RC + j0, raw[c]);
-        }
-        tmem_wait_ld();
-#pragma unroll
-        for (int c = 0; c < NR; ++c) {
-          const float* bias = cbias[l] + c * RC + j0;
-          float x[SL];
-#pragma unroll
-          for (int i = 0; i < SL; ++i) x[i] = elu_fast(__uint_as_float(raw[c][i]) + bias[i]);
-#pragma unroll
-          for (int q = 0; q < SL / 8; ++q)
-            a_store(sm.a, r, (c * RC + j0) / 8 + q,
-                    make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
-                               pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7])));
-          fence_async_smem();
-          if (c == NR - 1) tc_fence_before();
-          nb_arrive(2 + c);
-        }
+        hidden_rounds(sm.a, lane_t + dcol, cbias[l], 2, r, cb);
       } else {
-        // head layers are not pipelined: row-wise reductions need all columns.  Same code as k_bf16_chain,
-        // warp (quarter, cb) owns the 32-column block cb of its rows; barriers among the epilogue warps only.
+        // head layers are not pipelined: row-wise reductions need all columns.  Warp (quarter, cb) owns the 32-column
+        // block cb of its rows; barriers among the epilogue warps only.
         const int c0 = cb * 32;
         const float* bias = cbias[l] + c0;
-        uint4 pend[4];
-        uint4* pend_dst = nullptr;
         float x[32];
         tmem_ld32(lane_t + dcol + c0, x);
 #pragma unroll
         for (int i = 0; i < 32; ++i) x[i] += bias[i];
-        const bool state_seg = (kind == LK_STATE || kind == LK_STATE_REWARD) && cb < 2;
-        const bool soft_seg = (kind == LK_STATE_REWARD && cb >= 2) || (kind == LK_PRED && cb < 2);
-        SoftPart sp{-1e30f, 0.f, 0.f};
-        if (state_seg) {
-          float lo = INFINITY, hi = -INFINITY;
-#pragma unroll
-          for (int i = 0; i < 32; ++i) { lo = fminf(lo, x[i]); hi = fmaxf(hi, x[i]); }
-          sm.part[cb][r] = make_float4(lo, hi, 0.f, 0.f);
-        } else if (soft_seg) {
-          sp = soft_part(x, c0 & 63, S);
-          sm.part[cb][r] = make_float4(sp.m, sp.z, sp.y, 0.f);
-        }
+        const SoftPart sp = head_partials(x, kind, cb, r, S, sm.part);
         epi_sync();
-        if (state_seg) {
-          const float4 o = sm.part[cb ^ 1][r];
-          const float lo = fminf(sm.part[cb][r].x, o.x), hi = fmaxf(sm.part[cb][r].y, o.y);
-          float scale = hi - lo;
-          if (scale < 1e-5f) scale += 1e-5f;
-          const float inv = 1.f / scale;
-#pragma unroll
-          for (int i = 0; i < 32; ++i) x[i] = (x[i] - lo) * inv;
-          if (index >= 0 && job.hidden16_dst) pend_dst = reinterpret_cast<uint4*>(job.hidden16_dst + (size_t)index * SMZ_SP + c0);
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            pend[q] = make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
-                                 pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7]));
-            a_store(sm.a, r, cb * 4 + q, pend[q]);
-          }
-        } else if (soft_seg && (cb & 1) == 0) {
-          const float4 o = sm.part[cb + 1][r];
-          const float v = support_scalar(sp, SoftPart{o.x, o.y, o.z});
-          float* dst = (kind == LK_PRED) ? job.value_dst : job.reward_dst;
-          if (index >= 0 && dst) dst[index] = v;
-        } else if (kind == LK_PRED && cb == 2) {
-          const int n = ch.n_policy;
-          float m = -1e30f, z = 0.f;
-#pragma unroll
-          for (int i = 0; i < 32; ++i) m = fmaxf(m, x[i]);
-#pragma unroll
-          for (int i = 0; i < 32; ++i) {
-            x[i] = ex2f((x[i] - m) * 1.4426950408889634f);
-            z += x[i];
-          }
-          if (index >= 0 && job.policy_dst) {
-            float* dst = job.policy_dst + (size_t)index * job.pstride;
-            const float inv = 1.f / z;
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (i < n) dst[i] = x[i] * inv;
-          }
-        }
+        const HeadStores pend = head_finish(x, kind, cb, r, sp, sm.part, sm.a, index, job, ch.n_policy);
         if (l + 1 < nl) {
           // the next network's A operand (K = 64: column blocks 0, 1); the other two barriers are consumed as well
           fence_async_smem();
           tc_fence_before();
           for (int c = 0; c < NR; ++c) nb_arrive(2 + c);
         }
-        if (pend_dst) {
-#pragma unroll
-          for (int q = 0; q < 4; ++q) pend_dst[q] = pend[q];
-        }
+        pend.flush();
       }
       if (tl && warp == 0) tl[1 + l * 4 + 3] = clock64();
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(2 * TN) : "memory");
-  }
+  if (warp == 0) tmem_dealloc(tmem, 2 * TN);
 }
 
 // ---------------------------------------------------------------------------------------------
-// Two or four tiles per CTA for batches of more than one wave (k_bf16_chain_pipeN<2> / <4>).  With one 128-leaf tile per SM the tensor
+// Two tiles per CTA for batches of more than one wave (k_bf16_chain_pipeN<2>).  With one 128-leaf tile per SM the tensor
 // pipe idles while the 16 epilogue warps work through a layer (~1800 cycles, MUFU / issue bound) and the epilogue warps
 // idle while the layer's last K-steps complete (~600 cycles).  A CTA that owns TWO adjacent tiles of the row array (256
 // positions: never both branches, see smz_common.cuh) alternates them: the epilogue warps do (tile 0, layer l), (tile 1,
@@ -749,8 +726,7 @@ k_bf16_chain_pipe(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
 // epilogue — the contraction disappears behind the activation function.  Both tiles read the SAME weight tile
 // (one ring, one stream of bulk copies per group); accumulators: one per tile, NT x 128 TMEM columns.
 // ---------------------------------------------------------------------------------------------
-// NT = tiles per CTA: 2 by default; 4 (cfg4's 516 tiles = 129 quads, one wave instead of two waves of pairs) is kept
-// behind SMZ_PIPE2=4 — it measured slower.  One accumulator per tile is enough (NT x 128 TMEM columns): an epilogue loads all of
+// NT = tiles per CTA (2).  One accumulator per tile is enough (NT x 128 TMEM columns): an epilogue loads all of
 // its tile's accumulator before it hands the first round of columns to the issuer, so the next layer's K-steps never
 // overwrite values that are still to be read.
 template <int NT>
@@ -771,7 +747,6 @@ __global__ void __launch_bounds__(NPIPE, 1)
 k_bf16_chain_pipeN(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   extern __shared__ unsigned char smem_raw[];
   SmemPipeN<NT>& sm = *reinterpret_cast<SmemPipeN<NT>*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  constexpr int NR = 2;
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const bool is_issuer_warp = warp == NEPI / 32;
   const int r = (warp & 3) * 32 + lane;   // epilogue role: row of a tile == TMEM lane
@@ -779,26 +754,17 @@ k_bf16_chain_pipeN(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   const int group = blockIdx.x;           // positions [NT * 128 * group, NT * 128 * (group + 1)) of the row array
   const int nl = chain0.n_layers;
 
-  auto load_weights = [&](const Chain& c, int l, int slot) {
-    const unsigned bytes = (unsigned)c.layer[l].K * TN * 2;
-    mbar_expect_tx(&sm.wbar[slot], bytes);
-    bulk_g2s(sm.w[slot], c.layer[l].w, bytes, &sm.wbar[slot]);
-  };
   if (tid == 0) {
     mbar_init(&sm.wbar[0], 1); mbar_init(&sm.wbar[1], 1);
 #pragma unroll
     for (int t = 0; t < NT; ++t) mbar_init(&sm.dbar[t], 1);
     mbar_init(&sm.bbar, 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    load_weights(chain0, 0, 0);              // the first weight tile of BOTH chains: the branch is not known yet
-    load_weights(chain1, 0, 1);
+    load_weight_tile(chain0, 0, sm.wbar, sm.w, 0);   // the first weight tile of BOTH chains: the branch is not known yet
+    load_weight_tile(chain1, 0, sm.wbar, sm.w, 1);
   }
   __syncwarp();
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(&sm.tmem_base)), "r"(NT * TN)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 0) tmem_alloc(&sm.tmem_base, NT * TN);
   smz_pdl_wait();
   smz_pdl_launch_dependents();
   // row records + parent hidden rows of both tiles, requested together with the branch counts
@@ -808,35 +774,14 @@ k_bf16_chain_pipeN(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   for (int t = 0; t < NT; ++t) { rec[t] = make_int4(0, 0, 0, 0); hrow[t][0] = hrow[t][1] = make_uint4(0, 0, 0, 0); }
   if (!is_issuer_warp) {
 #pragma unroll
-    for (int t = 0; t < NT; ++t) {
-      const size_t ri = (size_t)(sim & 1) * a.row_cap + (size_t)(NT * group + t) * TM + r;
-      rec[t] = a.rows4[ri];
-      if (a.xin) {
-#pragma unroll
-        for (int q = 0; q < 2; ++q) hrow[t][q] = a.xin[ri * 8 + cb * 2 + q];
-      } else {
-        rec[t].x = min(max(rec[t].x, 0), a.B - 1);
-        rec[t].y = min(max(rec[t].y, 0), a.N);
-        const __nv_bfloat16* src16 = reinterpret_cast<const __nv_bfloat16*>(a.hidden) + ((size_t)rec[t].y * a.B + rec[t].x) * SMZ_SP;
-#pragma unroll
-        for (int q = 0; q < 2; ++q) hrow[t][q] = *reinterpret_cast<const uint4*>(src16 + (cb * 2 + q) * 8);
-      }
-    }
+    for (int t = 0; t < NT; ++t) rec[t] = load_row<2>(a, sim, (NT * group + t) * TM + r, cb * 2, hrow[t]);
   }
   const int count0 = a.branch_count[sim * 2], count1 = a.branch_count[sim * 2 + 1];
   const int top1 = a.row_top - count1;      // dynamics rows occupy [top1, row_top)
   const int lo = NT * group * TM;
   const int branch = lo < count0 ? 0 : (lo + NT * TM > top1 ? 1 : -1);
-  if (branch < 0) {                // nothing to do for this CTA: drain the prefetches, give TMEM back, leave
-    if (tid == 0) {
-      mbar_wait(&sm.wbar[0], 0);
-      mbar_wait(&sm.wbar[1], 0);
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    if (warp == 0)
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(sm.tmem_base), "r"(NT * TN) : "memory");
+  if (branch < 0) {                // the bias table has not been requested yet
+    idle_cta_exit(nullptr, sm.wbar, true, sm.tmem_base, NT * TN);
     return;
   }
   // which tiles carry rows (CTA-uniform bit mask): afterstate rows fill the group from below, dynamics rows from above
@@ -858,23 +803,11 @@ k_bf16_chain_pipeN(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
 
   if (is_issuer_warp) {
     // =========================== issuer warp: one weight ring, two tiles ======================================
-    unsigned nfill0 = 1u, nfill1 = 1u, nseen0 = 0u, nseen1 = 0u;
-    const __nv_bfloat16 *res0 = branch ? nullptr : ch.layer[0].w, *res1 = branch ? ch.layer[0].w : nullptr;
-    if (nl > 1) {                              // layer 1 replaces the unused chain's prefetched tile
-      const int s1 = branch ^ 1;
-      mbar_wait(&sm.wbar[s1], 0);
-      if (lane == 0) load_weights(ch, 1, s1);
-      if (s1) { nseen1 = 1u; nfill1 = 2u; res1 = ch.layer[1].w; } else { nseen0 = 1u; nfill0 = 2u; res0 = ch.layer[1].w; }
-      __syncwarp();
-    }
+    WeightRing ring(ch, sm.wbar, sm.w, lane);
+    ring.start(branch, nl);
     for (int l = 0; l < nl; ++l) {
       const int nk = ch.layer[l].K / 16;
-      const int slot = (l + branch) & 1;
-      const unsigned seen = slot ? nseen1 : nseen0;
-      if (seen < (slot ? nfill1 : nfill0)) {
-        mbar_wait(&sm.wbar[slot], seen & 1u);
-        if (slot) ++nseen1; else ++nseen0;
-      }
+      const int slot = ring.wait(l);
       const unsigned long long bd = umma_desc(s32(sm.w[slot]), CHUNK_W, 128);
 #pragma unroll 1
       for (int t = 0; t < NT; ++t) {
@@ -896,13 +829,8 @@ k_bf16_chain_pipeN(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
         if (lane == 0) umma_commit(&sm.dbar[t]);
         __syncwarp();
       }
-      if (l + 2 < nl && ((slot ? res1 : res0) != ch.layer[l + 2].w || job.stream_all)) {
-        // the slot is reusable once the MMAs of ALL tiles have completed (commits complete in issue order)
-        mbar_wait(&sm.dbar[t_last], l & 1);
-        if (lane == 0) load_weights(ch, l + 2, slot);
-        if (slot) { ++nfill1; res1 = ch.layer[l + 2].w; } else { ++nfill0; res0 = ch.layer[l + 2].w; }
-        __syncwarp();
-      }
+      // the slot is reusable once the MMAs of ALL tiles have completed (commits complete in issue order)
+      ring.refill(l, nl, job.stream_all, &sm.dbar[t_last], l & 1);
     }
   } else {
     // =========================== epilogue warps: (tile 0, l), (tile 1, l), (tile 0, l + 1), ... =====================
@@ -916,14 +844,7 @@ k_bf16_chain_pipeN(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
         const int act = valid ? rec[t].z : -1;
 #pragma unroll
         for (int q = 0; q < 2; ++q) a_store(sm.a[t], r, cb * 2 + q, valid ? hrow[t][q] : make_uint4(0, 0, 0, 0));
-        for (int kc = cb; kc < ch.onehot_pad / 8; kc += 4) {
-          unsigned w4[4] = {0, 0, 0, 0};
-          if (valid && act >= kc * 8 && act < kc * 8 + 8) {
-            const int j = act - kc * 8;
-            w4[j >> 1] = (j & 1) ? 0x3F800000u : 0x00003F80u;
-          }
-          a_store(sm.a[t], r, 8 + kc, make_uint4(w4[0], w4[1], w4[2], w4[3]));
-        }
+        for (int kc = cb; kc < ch.onehot_pad / 8; kc += 4) a_store(sm.a[t], r, 8 + kc, onehot_chunk(act, kc));
       }
     }
     fence_async_smem();
@@ -948,108 +869,32 @@ k_bf16_chain_pipeN(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
         __syncwarp();
         tc_fence_after();
         if (kind == LK_HIDDEN) {
-          constexpr int SL = 32 / NR;              // 16-column slice of every round
-          constexpr int RC = TN / NR;              // 64 columns per round
-          const int j0 = cb * SL;
-          unsigned raw[NR][SL];
-#pragma unroll
-          for (int c = 0; c < NR; ++c) tmem_ld16_nowait(lane_t + c * RC + j0, raw[c]);
-          tmem_wait_ld();
-#pragma unroll
-          for (int c = 0; c < NR; ++c) {
-            const float* bias = cbias[l] + c * RC + j0;
-            float x[SL];
-#pragma unroll
-            for (int i = 0; i < SL; ++i) x[i] = elu_fast(__uint_as_float(raw[c][i]) + bias[i]);
-#pragma unroll
-            for (int q = 0; q < SL / 8; ++q)
-              a_store(A, r, (c * RC + j0) / 8 + q,
-                      make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
-                                 pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7])));
-            fence_async_smem();
-            if (c == NR - 1) tc_fence_before();
-            nb_arrive(2 + 2 * t + c);
-          }
+          hidden_rounds(A, lane_t, cbias[l], 2 + 2 * t, r, cb);
         } else {
           // head layers: row-wise reductions need all columns; warp (quarter, cb) owns the 32-column block cb of its rows
           const int c0 = cb * 32;
           const float* bias = cbias[l] + c0;
           float4 (*part)[TM] = sm.part[t & 1];
-          uint4 pend[4];
-          uint4* pend_dst = nullptr;
           float x[32];
           tmem_ld32(lane_t + c0, x);
 #pragma unroll
           for (int i = 0; i < 32; ++i) x[i] += bias[i];
-          const bool state_seg = (kind == LK_STATE || kind == LK_STATE_REWARD) && cb < 2;
-          const bool soft_seg = (kind == LK_STATE_REWARD && cb >= 2) || (kind == LK_PRED && cb < 2);
-          SoftPart sp{-1e30f, 0.f, 0.f};
-          if (state_seg) {
-            float lo_ = INFINITY, hi_ = -INFINITY;
-#pragma unroll
-            for (int i = 0; i < 32; ++i) { lo_ = fminf(lo_, x[i]); hi_ = fmaxf(hi_, x[i]); }
-            part[cb][r] = make_float4(lo_, hi_, 0.f, 0.f);
-          } else if (soft_seg) {
-            sp = soft_part(x, c0 & 63, S);
-            part[cb][r] = make_float4(sp.m, sp.z, sp.y, 0.f);
-          }
+          const SoftPart sp = head_partials(x, kind, cb, r, S, part);
           epi_sync();
-          if (state_seg) {
-            const float4 o = part[cb ^ 1][r];
-            const float lo_ = fminf(part[cb][r].x, o.x), hi_ = fmaxf(part[cb][r].y, o.y);
-            float scale = hi_ - lo_;
-            if (scale < 1e-5f) scale += 1e-5f;
-            const float inv = 1.f / scale;
-#pragma unroll
-            for (int i = 0; i < 32; ++i) x[i] = (x[i] - lo_) * inv;
-            if (index_t >= 0 && job.hidden16_dst) pend_dst = reinterpret_cast<uint4*>(job.hidden16_dst + (size_t)index_t * SMZ_SP + c0);
-#pragma unroll
-            for (int q = 0; q < 4; ++q) {
-              pend[q] = make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
-                                   pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7]));
-              a_store(A, r, cb * 4 + q, pend[q]);
-            }
-          } else if (soft_seg && (cb & 1) == 0) {
-            const float4 o = part[cb + 1][r];
-            const float v = support_scalar(sp, SoftPart{o.x, o.y, o.z});
-            float* dst = (kind == LK_PRED) ? job.value_dst : job.reward_dst;
-            if (index_t >= 0 && dst) dst[index_t] = v;
-          } else if (kind == LK_PRED && cb == 2) {
-            const int n = ch.n_policy;
-            float m = -1e30f, z = 0.f;
-#pragma unroll
-            for (int i = 0; i < 32; ++i) m = fmaxf(m, x[i]);
-#pragma unroll
-            for (int i = 0; i < 32; ++i) {
-              x[i] = ex2f((x[i] - m) * 1.4426950408889634f);
-              z += x[i];
-            }
-            if (index_t >= 0 && job.policy_dst) {
-              float* dst = job.policy_dst + (size_t)index_t * job.pstride;
-              const float inv = 1.f / z;
-#pragma unroll
-              for (int i = 0; i < 32; ++i)
-                if (i < n) dst[i] = x[i] * inv;
-            }
-          }
+          const HeadStores pend = head_finish(x, kind, cb, r, sp, part, A, index_t, job, ch.n_policy);
           if (l + 1 < nl) {
             fence_async_smem();
             tc_fence_before();
             for (int c = 0; c < NR; ++c) nb_arrive(2 + 2 * t + c);
           }
-          if (pend_dst) {
-#pragma unroll
-            for (int q = 0; q < 4; ++q) pend_dst[q] = pend[q];
-          }
+          pend.flush();
         }
       }
     }
   }
   tc_fence_before();
   __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(NT * TN) : "memory");
-  }
+  if (warp == 0) tmem_dealloc(tmem, NT * TN);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1101,18 +946,15 @@ __device__ __forceinline__ void a64_tstore(unsigned taddr, const unsigned* pa, c
   for (int i = 0; i < N; ++i) { r[2 * i] = pa[i]; r[2 * i + 1] = pb[i]; }
   if constexpr (N == 1) {
     tmem_st16x128_x1(taddr, r[0], r[1]);
-  } else if constexpr (N == 2) {
-    tmem_st16x128_x2(taddr, r);
   } else if constexpr (N == 3) {
     tmem_st16x128_x2(taddr, r);
     tmem_st16x128_x1(taddr + 8, r[4], r[5]);
   } else {
-    static_assert(N == 4, "a64_tstore: 1 .. 4 groups");
+    static_assert(N == 4, "a64_tstore: 1, 3 or 4 groups");
     tmem_st16x128_x4(taddr, r);
   }
 }
 
-// R0 = columns of the first hidden-layer round (64: two even rounds; 96: 96 + 32, two K-steps left for the tail).
 // HALF = 32 leaves per tile instead of 64: the leaves sit in the accumulator rows m with m % 16 < 8, i.e. in the FIRST
 // row of every thread's 16x256b fragment (thread t: rows t/4 and t/4 + 8), so the epilogue — bound by the MUFU pipe and
 // by instruction issue, not by the contraction — does half the work per SM with all 32 lanes of every warp busy, on
@@ -1121,10 +963,11 @@ __device__ __forceinline__ void a64_tstore(unsigned taddr, const unsigned* pa, c
 // from the bottom, dynamics rows from the top, never both in one tile), so the row records are requested together with
 // the branch counts — one L2 round trip after the dependency wait — and no CTA is launched for an empty tile of
 // the "other" branch.  The first weight tile of BOTH chains is prefetched before the wait.
-template <int R0, bool HALF>
+template <bool HALF>
 __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& chain0, const Chain& chain1, const Job& job, int sim) {
   extern __shared__ unsigned char smem_raw[];
   Smem64& sm = *reinterpret_cast<Smem64*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
+  constexpr int R0 = 96;                   // hidden layers: rounds of 96 + 32 columns (two K-steps left for the tail)
   constexpr int TV = HALF ? 32 : 64;       // leaves per tile
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const bool is_issuer_warp = warp == NEPI / 32;
@@ -1138,11 +981,6 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
   long long* tl = (job.timeline && blockIdx.x == 0 && lane == 0) ? job.timeline : nullptr;   // debug stamps
   if (tl && tid == 0) tl[0] = clock64();
 
-  auto load_weights = [&](const Chain& c, int l, int slot) {
-    const unsigned bytes = (unsigned)c.layer[l].K * TN * 2;
-    mbar_expect_tx(&sm.wbar[slot], bytes);
-    bulk_g2s(sm.w[slot], c.layer[l].w, bytes, &sm.wbar[slot]);
-  };
   if (tid == 0) {
     mbar_init(&sm.wbar[0], 1); mbar_init(&sm.wbar[1], 1);
     mbar_init(&sm.dbar[0], 1); mbar_init(&sm.dbar[1], 1);
@@ -1152,15 +990,11 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
     mbar_expect_tx(&sm.bbar, 2 * bbytes);
     bulk_g2s(sm.bias[0], chain0.bias, bbytes, &sm.bbar);
     bulk_g2s(sm.bias[1], chain1.bias, bbytes, &sm.bbar);
-    load_weights(chain0, 0, 0);
-    load_weights(chain1, 0, 1);
+    load_weight_tile(chain0, 0, sm.wbar, sm.w, 0);
+    load_weight_tile(chain1, 0, sm.wbar, sm.w, 1);
   }
   __syncwarp();
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(&sm.tmem_base)), "r"(2 * TN)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
+  if (warp == 0) tmem_alloc(&sm.tmem_base, 2 * TN);
   smz_pdl_wait();
   smz_pdl_launch_dependents();
   smz_stamp_min(a.dbg, sim, 2);
@@ -1172,37 +1006,15 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
   const int pos = tile * TV + srow;
   int4 rec = make_int4(0, 0, 0, 0);
   uint4 hrow = make_uint4(0, 0, 0, 0);
-  if (stager) {
-    const size_t ri = (size_t)(sim & 1) * a.row_cap + pos;
-    rec = a.rows4[ri];
-    if (a.xin) {
-      hrow = a.xin[ri * 8 + skc];              // the descent copied the parent's row: no dependent second load
-    } else {
-      rec.x = min(max(rec.x, 0), a.B - 1);
-      rec.y = min(max(rec.y, 0), a.N);
-      hrow = *reinterpret_cast<const uint4*>(reinterpret_cast<const __nv_bfloat16*>(a.hidden) +
-                                             ((size_t)rec.y * a.B + rec.x) * SMZ_SP + skc * 8);
-    }
-  }
+  if (stager) rec = load_row<1>(a, sim, pos, skc, &hrow);
   const int count0 = a.branch_count[sim * 2], count1 = a.branch_count[sim * 2 + 1];
   const int top1 = a.row_top - count1;      // dynamics rows occupy [top1, row_top)
   const int branch = tile * TV < count0 ? 0 : ((tile + 1) * TV > top1 ? 1 : -1);
   if (branch < 0) {
-    if (tid == 0) {
-      mbar_wait(&sm.bbar, 0);
-      mbar_wait(&sm.wbar[0], 0);
-      mbar_wait(&sm.wbar[1], 0);
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    if (warp == 0)
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(sm.tmem_base), "r"(2 * TN) : "memory");
+    idle_cta_exit(&sm.bbar, sm.wbar, true, sm.tmem_base, 2 * TN);
     return;
   }
   const Chain& ch = branch ? chain1 : chain0;
-  // weight ring: layer l lives in slot (l + branch) & 1 (layer 0 of chain b was prefetched into slot b); the other
-  // slot's first fill was the unused chain's tile, so the fill that carries layer l is number (l + 1) >> 1 of its slot
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
@@ -1210,27 +1022,11 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
 
   if (is_issuer_warp) {
     const unsigned long long ad = umma_desc(s32(sm.a), CHUNK_A64, 128);
-    // Weight ring.  The hidden layers of a network share ONE weight tile (the reference ties them, mlp:31-37): a tile
-    // that is already resident in its slot is not streamed again — 6 bulk copies per chain instead of 12.
-    // nfill / nseen = fills issued to / waited for on each slot; slot `branch` holds layer 0 (fill 0, prefetched),
-    // the other slot's fill 0 was the unused chain's layer 0 and is replaced by layer 1 as soon as it has landed.
-    unsigned nfill0 = 1u, nfill1 = 1u, nseen0 = 0u, nseen1 = 0u;        // per slot, kept in registers (no indexed arrays)
-    const __nv_bfloat16 *res0 = branch ? nullptr : ch.layer[0].w, *res1 = branch ? ch.layer[0].w : nullptr;
-    if (nl > 1) {
-      const int s1 = branch ^ 1;
-      mbar_wait(&sm.wbar[s1], 0);
-      if (lane == 0) load_weights(ch, 1, s1);
-      if (s1) { nseen1 = 1u; nfill1 = 2u; res1 = ch.layer[1].w; } else { nseen0 = 1u; nfill0 = 2u; res0 = ch.layer[1].w; }
-      __syncwarp();
-    }
+    WeightRing ring(ch, sm.wbar, sm.w, lane);
+    ring.start(branch, nl);
     for (int l = 0; l < nl; ++l) {
       const int nk = ch.layer[l].K / 16;
-      const int slot = (l + branch) & 1;
-      const unsigned seen = slot ? nseen1 : nseen0;
-      if (seen < (slot ? nfill1 : nfill0)) {
-        mbar_wait(&sm.wbar[slot], seen & 1u);
-        if (slot) ++nseen1; else ++nseen0;
-      }
+      const int slot = ring.wait(l);
       const unsigned long long bd = umma_desc(s32(sm.w[slot]), CHUNK_W, 128);
       for (int c = 0; c < 2; ++c) {
         nb_sync(2 + c);
@@ -1254,12 +1050,7 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
       if (lane == 0) umma_commit(&sm.dbar[l & 1]);
       if (tl) tl[1 + l * 4 + 1] = clock64();
       __syncwarp();
-      if (l + 2 < nl && ((slot ? res1 : res0) != ch.layer[l + 2].w || job.stream_all)) {
-        mbar_wait(&sm.dbar[l & 1], (l >> 1) & 1);            // the slot is free once these MMAs have completed
-        if (lane == 0) load_weights(ch, l + 2, slot);
-        if (slot) { ++nfill1; res1 = ch.layer[l + 2].w; } else { ++nfill0; res0 = ch.layer[l + 2].w; }
-        __syncwarp();
-      }
+      ring.refill(l, nl, job.stream_all, &sm.dbar[l & 1], (l >> 1) & 1);   // the slot is free once these MMAs have completed
     }
   } else {
     {   // stage the first A operand
@@ -1269,14 +1060,9 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
                      "r"(valid ? hrow.y : 0u), "r"(valid ? hrow.z : 0u), "r"(valid ? hrow.w : 0u)
                      : "memory");
         if (skc < ch.onehot_pad / 8) {
-          const int act = valid ? rec.z : -1;
-          unsigned w4[4] = {0, 0, 0, 0};
-          if (act >= skc * 8 && act < skc * 8 + 8) {
-            const int j = act - skc * 8;
-            w4[j >> 1] = (j & 1) ? 0x3F800000u : 0x00003F80u;
-          }
-          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(s32(sm.a + (8 + skc) * CHUNK_A64 + mrow * 16)), "r"(w4[0]),
-                       "r"(w4[1]), "r"(w4[2]), "r"(w4[3])
+          const uint4 oh = onehot_chunk(valid ? rec.z : -1, skc);
+          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(s32(sm.a + (8 + skc) * CHUNK_A64 + mrow * 16)), "r"(oh.x),
+                       "r"(oh.y), "r"(oh.z), "r"(oh.w)
                        : "memory");
         }
         if (skc == 0) sm.rowidx[mrow] = valid ? rec.x : -1;
@@ -1319,14 +1105,9 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
         // two rounds: columns [0, R0) and [R0, 128); this warp owns a quarter of each round for its 16 rows.  All the
         // arithmetic of both rounds first (independent chains: the MUFU latencies overlap), then stores + hand-off per round.
         unsigned raw[4 * (G0 + G1)];
-        if constexpr (R0 == 64) {
-          tmem_ld16x256_x2(lane_t + cb * 16, raw);
-          tmem_ld16x256_x2(lane_t + 64 + cb * 16, raw + 8);
-        } else {
-          tmem_ld16x256_x2(lane_t + cb * 24, raw);
-          tmem_ld16x256_x1(lane_t + cb * 24 + 16, raw + 8);
-          tmem_ld16x256_x1(lane_t + 96 + cb * 8, raw + 12);
-        }
+        tmem_ld16x256_x2(lane_t + cb * 24, raw);
+        tmem_ld16x256_x1(lane_t + cb * 24 + 16, raw + 8);
+        tmem_ld16x256_x1(lane_t + R0 + cb * 8, raw + 12);
         tmem_wait_ld();
         const bool fine = tl && warp == 0 && l == 2;
         if (fine) tl[1 + 4 * MAXL + 2] = clock64();
@@ -1518,307 +1299,19 @@ __device__ __forceinline__ void chain_m64_body(const SmzArena& a, const Chain& c
   tc_fence_before();
   __syncthreads();
   smz_stamp_max(a.dbg, sim, 3);
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(2 * TN) : "memory");
-  }
+  if (warp == 0) tmem_dealloc(tmem, 2 * TN);
 }
 
-template <int R0>
 __global__ void __maxnreg__(80)      // see k_bf16_chain_m32: measured 1.33 vs 1.50 ms per search at 6144 trees (98 CTAs)
 k_bf16_chain_m64(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
-  chain_m64_body<R0, false>(a, chain0, chain1, job, sim);
+  chain_m64_body<false>(a, chain0, chain1, job, sim);
 }
 // 32-leaf tiles: 80 registers per thread, so that a block of the tree step (4 warps x 88 registers) still fits next to
 // the 17 warps of this CTA in every SM sub-partition (16 K registers each; sub-partition 0 holds 5 of the 17 warps) —
 // with one network CTA on nearly every SM the tree step launched under it (PDL) has nowhere else to go
 __global__ void __maxnreg__(80)
 k_bf16_chain_m32(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
-  chain_m64_body<96, true>(a, chain0, chain1, job, sim);
-}
-
-// ---------------------------------------------------------------------------------------------
-// The whole search loop of 128 trees in ONE persistent CTA (no inter-CTA dependency exists in the search:
-// trees are independent, so nothing but this tile's own progress gates the next simulation).
-// Per simulation: [expansion + backup of the previous one, descent of this one] on 4 lanes per tree ->
-// rows sorted by branch (afterstate leaves first) -> gather -> the 2(L+2)-layer chain with BOTH weight sets
-// resident per layer (afterstate-net tile and dynamics-net tile, accumulators in TMEM columns [0,128) and
-// [128,256)); each row's epilogue reads the accumulator half of its own branch.  No kernel boundary, no
-// per-launch prologue (TMEM, barriers, first weight tiles), no compaction atomics, no waiting for the deepest
-// tree of the whole batch.  Needs policy widths <= 4 (4 lanes per tree).
-// ---------------------------------------------------------------------------------------------
-struct SmemMega {
-  alignas(1024) unsigned char a[A_BYTES];
-  alignas(1024) unsigned char w[2][2][W_BYTES];   // [ring slot][0 = afterstate pair, 1 = dynamics pair]
-  float bias[2][MAXL][TN];
-  unsigned long long wbar[2];
-  unsigned long long mbar;
-  unsigned long long bbar;
-  unsigned int tmem_base;
-  float4 part[4][TM];
-  int rowtree[TM], rowslot[TM], rowact[TM];        // indexed by tile ROW (after the per-simulation sort)
-  int lslot[TM], lact[TM], lbranch[TM];            // indexed by LOCAL tree, written by the descent
-  int wcount[2][4];
-  int n_after;
-};
-
-__global__ void __launch_bounds__(NTHREADS, 1)
-k_search_mega(SmzArena a, Chain chA, Chain chD, int n_trees, int first, int n_sims, int S, long long* timeline) {
-  using namespace smz_tree_dev;
-  extern __shared__ unsigned char smem_raw[];
-  SmemMega& sm = *reinterpret_cast<SmemMega*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int r = (warp & 3) * 32 + lane;   // chain role: row of the tile == TMEM lane
-  const int cb = warp >> 2;               // chain role: accumulator column block
-  const int c0 = cb * 32;
-  const int tile_base = blockIdx.x * TM;
-  const int nl = chA.n_layers, total = n_sims * nl;
-
-  auto load_weights = [&](int gl) {
-    const int l = gl % nl, slot = gl & 1;
-    const unsigned bytes = (unsigned)chA.layer[l].K * TN * 2;
-    mbar_expect_tx(&sm.wbar[slot], 2 * bytes);
-    bulk_g2s(sm.w[slot][0], chA.layer[l].w, bytes, &sm.wbar[slot]);
-    bulk_g2s(sm.w[slot][1], chD.layer[l].w, bytes, &sm.wbar[slot]);
-  };
-  if (tid == 0) {
-    mbar_init(&sm.wbar[0], 1);
-    mbar_init(&sm.wbar[1], 1);
-    mbar_init(&sm.mbar, 1);
-    mbar_init(&sm.bbar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    const unsigned bbytes = (unsigned)nl * TN * 4;
-    mbar_expect_tx(&sm.bbar, 2 * bbytes);
-    bulk_g2s(sm.bias[0], chA.bias, bbytes, &sm.bbar);
-    bulk_g2s(sm.bias[1], chD.bias, bbytes, &sm.bbar);
-    load_weights(0);
-    if (total > 1) load_weights(1);
-  }
-  __syncwarp();
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(&sm.tmem_base)), "r"(2 * TN)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-
-  // ---- tree role: 4 lanes per tree, the per-tree state stays in registers across the whole loop -----------
-  Group<4> g;
-  const int ltree = tid >> 2;
-  int tree = tile_base + ltree;
-  const bool alive = tree < n_trees;
-  if (!alive) tree = n_trees - 1;
-  const SmzRng rng = smz_make_rng(a);
-  TreeState ts;
-  ts.cursor = a.ucursor[tree];
-  ts.mm = a.minmax[tree];
-  { const int4 rs = a.stat[(size_t)tree * a.M]; ts.root = make_int2(rs.x, rs.y); }
-
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const unsigned tmem = sm.tmem_base;
-  mbar_wait(&sm.bbar, 0);
-  if (tid == 0) mbar_wait(&sm.wbar[0], 0);
-
-  for (int it = 0; it < n_sims; ++it) {
-    const int sim = first + it;
-    const bool stamp = timeline && blockIdx.x == 0 && tid == 0 && it == n_sims - 1;
-    if (stamp) timeline[0] = clock64();
-    // ---- 1. tree phase -------------------------------------------------------------------------------------
-    if (it > 0) {
-      ts = expand_backup_phase(g, a, rng, tree, alive, sim - 1, a.out_policy, a.W, a.out_value, a.out_reward);
-      __syncwarp();
-    }
-    select_phase<4, false>(g, a, rng, tree, alive, sim, ts, sm.lslot - tile_base, sm.lact - tile_base, sm.lbranch - tile_base);
-    if (tid < TM) sm.rowtree[tid] = -1;
-    if (stamp) timeline[1 + 4 * MAXL + 0] = clock64();
-    __syncthreads();
-    if (stamp) timeline[1 + 4 * MAXL + 1] = clock64();
-    // ---- 2. sort the rows of the tile by branch: afterstate leaves first ---------------------------------------
-    unsigned m0 = 0, m1 = 0;
-    int mybranch = 2;
-    if (tid < TM) {
-      if (tile_base + tid < n_trees) mybranch = sm.lbranch[tid];
-      m0 = __ballot_sync(0xffffffffu, mybranch == 0);
-      m1 = __ballot_sync(0xffffffffu, mybranch == 1);
-      if (lane == 0) { sm.wcount[0][warp] = __popc(m0); sm.wcount[1][warp] = __popc(m1); }
-    }
-    __syncthreads();
-    if (tid < TM) {
-      int n0 = 0, pre0 = 0, pre1 = 0;
-      for (int w2 = 0; w2 < 4; ++w2) {
-        if (w2 < warp) { pre0 += sm.wcount[0][w2]; pre1 += sm.wcount[1][w2]; }
-        n0 += sm.wcount[0][w2];
-      }
-      const unsigned lt = (1u << lane) - 1u;
-      if (mybranch < 2) {
-        const int pos = mybranch == 0 ? pre0 + __popc(m0 & lt) : n0 + pre1 + __popc(m1 & lt);
-        sm.rowtree[pos] = tile_base + tid;
-        sm.rowslot[pos] = sm.lslot[tid];
-        sm.rowact[pos] = sm.lact[tid];
-      }
-      if (tid == 0) sm.n_after = n0;
-    }
-    __syncthreads();
-    // ---- 3. gather the parent hidden states (bf16 arena rows) + one-hot action into the A operand --------------
-    const int index = sm.rowtree[r];
-    const int n_after = sm.n_after;
-    const int br = r >= n_after;                     // this row's branch (rows beyond the last leaf: don't care)
-    {
-      const bool valid = index >= 0;
-      const __nv_bfloat16* src16 = valid
-          ? reinterpret_cast<const __nv_bfloat16*>(a.hidden) + ((size_t)sm.rowslot[r] * a.B + index) * SMZ_SP : nullptr;
-      const int act = valid ? sm.rowact[r] : -1;
-#pragma unroll
-      for (int q = 0; q < 2; ++q) {
-        const int kc = cb * 2 + q;
-        a_store(sm.a, r, kc, valid ? *reinterpret_cast<const uint4*>(src16 + kc * 8) : make_uint4(0, 0, 0, 0));
-      }
-      for (int kc = cb; kc < chA.onehot_pad / 8; kc += 4) {
-        unsigned w4[4] = {0, 0, 0, 0};
-        if (valid && act >= kc * 8 && act < kc * 8 + 8) {
-          const int j = act - kc * 8;
-          w4[j >> 1] = (j & 1) ? 0x3F800000u : 0x00003F80u;
-        }
-        a_store(sm.a, r, 8 + kc, make_uint4(w4[0], w4[1], w4[2], w4[3]));
-      }
-    }
-    fence_async_smem();
-    tc_fence_before();
-    __syncthreads();
-    if (stamp) timeline[1 + 4 * MAXL + 2] = clock64();
-    // this warp's 32 rows all take the same branch unless the boundary falls inside them
-    const int q0 = (warp & 3) * 32;
-    const bool mixed = n_after > q0 && n_after < q0 + 32;
-    const unsigned taddr0 = tmem + ((unsigned)q0 << 16) + (unsigned)c0;
-
-    // ---- 4. the layer chain, both weight sets per layer -------------------------------------------------------
-    for (int l = 0; l < nl; ++l) {
-      const int gl = it * nl + l;
-      const int K = chA.layer[l].K;
-      const int kindA = chA.layer[l].kind;
-      if (tid == 0) {
-        if (stamp) timeline[1 + l * 4 + 0] = clock64();
-        tc_fence_after();
-        const unsigned long long ad = umma_desc(s32(sm.a), CHUNK_A, 128);
-        const int nk = K / 16;
-#pragma unroll
-        for (int net = 0; net < 2; ++net) {
-          const unsigned long long bd = umma_desc(s32(sm.w[gl & 1][net]), CHUNK_W, 128);
-          umma(tmem + net * TN, ad, bd, 0u);
-#pragma unroll
-          for (int k = 1; k < 8; ++k)
-            if (k < nk)
-              umma(tmem + net * TN, ad + (unsigned long long)(k * ((2 * CHUNK_A) >> 4)),
-                   bd + (unsigned long long)(k * ((2 * CHUNK_W) >> 4)), 1u);
-        }
-        umma_commit(&sm.mbar);
-        if (stamp) timeline[1 + l * 4 + 1] = clock64();
-        if (gl + 1 < total) mbar_wait(&sm.wbar[(gl + 1) & 1], ((gl + 1) >> 1) & 1);
-      }
-      mbar_wait(&sm.mbar, gl & 1);
-      __syncwarp();
-      if (stamp) timeline[1 + l * 4 + 2] = clock64();
-      tc_fence_after();
-      if (tid == 0 && gl + 2 < total) load_weights(gl + 2);
-      __syncwarp();
-      const float* bias = sm.bias[br][l] + c0;
-
-      uint4 pend[4];
-      uint4* pend_dst = nullptr;
-      float x[32];
-      if (!mixed) {
-        tmem_ld32(taddr0 + (unsigned)(br * TN), x);
-      } else {
-        float y[32];
-        tmem_ld32(taddr0, x);
-        tmem_ld32(taddr0 + TN, y);
-#pragma unroll
-        for (int j = 0; j < 32; ++j) x[j] = br ? y[j] : x[j];
-      }
-#pragma unroll
-      for (int j = 0; j < 32; ++j) x[j] += bias[j];
-
-      if (kindA == LK_HIDDEN) {
-#pragma unroll
-        for (int j = 0; j < 32; ++j) x[j] = elu_fast(x[j]);
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          a_store(sm.a, r, cb * 4 + q,
-                  make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
-                             pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7])));
-      } else {
-        // head layers: LK_STATE / LK_STATE_REWARD (end of the dynamics nets) or LK_PRED (end of the prediction nets)
-        const bool is_pred = kindA == LK_PRED;
-        const bool state_seg = !is_pred && cb < 2;
-        const bool soft_seg = (is_pred && cb < 2) || (!is_pred && br == 1 && cb >= 2);     // reward: dynamics rows only
-        SoftPart sp{-1e30f, 0.f, 0.f};
-        if (state_seg) {
-          float lo = INFINITY, hi = -INFINITY;
-#pragma unroll
-          for (int j = 0; j < 32; ++j) { lo = fminf(lo, x[j]); hi = fmaxf(hi, x[j]); }
-          sm.part[cb][r] = make_float4(lo, hi, 0.f, 0.f);
-        } else if (soft_seg) {
-          sp = soft_part(x, c0 & 63, S);
-          sm.part[cb][r] = make_float4(sp.m, sp.z, sp.y, 0.f);
-        }
-        __syncthreads();
-        if (state_seg) {
-          const float4 o = sm.part[cb ^ 1][r];
-          const float lo = fminf(sm.part[cb][r].x, o.x), hi = fmaxf(sm.part[cb][r].y, o.y);
-          float scale = hi - lo;
-          if (scale < 1e-5f) scale += 1e-5f;
-          const float inv = 1.f / scale;
-#pragma unroll
-          for (int j = 0; j < 32; ++j) x[j] = (x[j] - lo) * inv;
-          if (index >= 0)
-            pend_dst = reinterpret_cast<uint4*>(reinterpret_cast<__nv_bfloat16*>(a.hidden) +
-                                                ((size_t)(sim + 1) * a.B + index) * SMZ_SP + c0);
-#pragma unroll
-          for (int q = 0; q < 4; ++q) {
-            pend[q] = make_uint4(pack_bf16(x[q * 8 + 0], x[q * 8 + 1]), pack_bf16(x[q * 8 + 2], x[q * 8 + 3]),
-                                 pack_bf16(x[q * 8 + 4], x[q * 8 + 5]), pack_bf16(x[q * 8 + 6], x[q * 8 + 7]));
-            a_store(sm.a, r, cb * 4 + q, pend[q]);
-          }
-        } else if (soft_seg && (cb & 1) == 0) {
-          const float4 o = sm.part[cb + 1][r];
-          const float v = support_scalar(sp, SoftPart{o.x, o.y, o.z});
-          if (index >= 0) (is_pred ? a.out_value : a.out_reward)[index] = v;
-        } else if (is_pred && cb == 2) {
-          const int n = br ? chD.n_policy : chA.n_policy;
-          float m = -1e30f, z = 0.f;
-#pragma unroll
-          for (int i = 0; i < 32; ++i) m = fmaxf(m, x[i]);
-#pragma unroll
-          for (int i = 0; i < 32; ++i) {
-            x[i] = ex2f((x[i] - m) * 1.4426950408889634f);
-            z += x[i];
-          }
-          if (index >= 0) {
-            float* dst = a.out_policy + (size_t)index * a.W;
-            const float inv = 1.f / z;
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (i < n) dst[i] = x[i] * inv;
-          }
-        }
-      }
-      fence_async_smem();
-      tc_fence_before();
-      __syncthreads();
-      if (pend_dst) {
-#pragma unroll
-        for (int q = 0; q < 4; ++q) pend_dst[q] = pend[q];
-      }
-      if (stamp) timeline[1 + l * 4 + 3] = clock64();
-    }
-  }
-  // ---- expansion + backup of the last simulation ------------------------------------------------------------
-  expand_backup_phase(g, a, rng, tree, alive, first + n_sims - 1, a.out_policy, a.W, a.out_value, a.out_reward);
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(2 * TN) : "memory");
-  }
+  chain_m64_body<true>(a, chain0, chain1, job, sim);
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -1878,13 +1371,11 @@ struct SmzBf16Image {
   size_t pool_bytes;
   int smem_bytes;
   long long* timeline;    // device debug buffer or null (SMZ_BF16_TIMELINE=1)
-  int pipe_rounds;        // 2 (default) or 4 rounds per hidden layer in the pipelined kernel (SMZ_PIPE_ROUNDS)
   int use_m64;            // 64-row tiles: -1 = by batch size (busy CTAs fit one wave of SMs), SMZ_M64=0/1 forces
   int use_m32;            // 32 leaves per 64-row tile: -1 = while those tiles fit one wave of SMs, SMZ_M32=0/1 forces
   int n_sms;
-  int timeline_mega;
   int use_pipe;           // K-pipelined chain for the simulation step (SMZ_NO_PIPE=1 turns it off)
-  int use_pipe2;          // 128-leaf tiles per CTA: -1 = by batch size (1 / 2 / 4), SMZ_PIPE2 = 0 / 1 (= 2) / 2 / 4 forces
+  int use_pipe2;          // 128-leaf tiles per CTA: -1 = by batch size (1 / 2), SMZ_PIPE2 = 0 / 1 forces one / two
 };
 
 static int round16(int v) { return (v + 15) / 16 * 16; }
@@ -1929,11 +1420,9 @@ int smz_bf16_create(const SmzNetShape& sh, const SmzArena&, SmzBf16Image** out, 
   }
   im->bias_pool = (float*)p;
   im->smem_bytes = (int)sizeof(Smem) + 1024;
-  cudaFuncSetAttribute((const void*)k_bf16_chain_pipe<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemPipe) + 1024);
-  cudaFuncSetAttribute((const void*)k_bf16_chain_pipe<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemPipe) + 1024);
+  cudaFuncSetAttribute((const void*)k_bf16_chain_pipe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemPipe) + 1024);
   im->use_pipe = getenv("SMZ_NO_PIPE") ? 0 : 1;
   cudaFuncSetAttribute((const void*)k_bf16_chain_pipeN<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemPipeN<2>) + 1024);
-  cudaFuncSetAttribute((const void*)k_bf16_chain_pipeN<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(SmemPipeN<4>) + 1024);
   im->use_pipe2 = getenv("SMZ_PIPE2") ? atoi(getenv("SMZ_PIPE2")) : -1;
   im->use_m64 = getenv("SMZ_M64") ? atoi(getenv("SMZ_M64")) : -1;
   {
@@ -1941,8 +1430,7 @@ int smz_bf16_create(const SmzNetShape& sh, const SmzArena&, SmzBf16Image** out, 
     cudaGetDevice(&dev);
     if (cudaDeviceGetAttribute(&im->n_sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || im->n_sms <= 0) im->n_sms = 148;
   }
-  cudaFuncSetAttribute((const void*)k_bf16_chain_m64<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem64) + 1024);
-  cudaFuncSetAttribute((const void*)k_bf16_chain_m64<96>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem64) + 1024);
+  cudaFuncSetAttribute((const void*)k_bf16_chain_m64, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem64) + 1024);
   cudaFuncSetAttribute((const void*)k_bf16_chain_m32, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem64) + 1024);
   im->use_m32 = getenv("SMZ_M32") ? atoi(getenv("SMZ_M32")) : -1;
   // The small-batch network CTAs share their SMs with the blocks of the shared-memory tree step that is launched while
@@ -1950,16 +1438,13 @@ int smz_bf16_create(const SmzNetShape& sh, const SmzArena&, SmzBf16Image** out, 
   // of them alone and the other's blocks wait for it to drain (measured: 156 vs 176 M sims/s on cfg2).  NOT set on the
   // arena-only tree kernels of the large batches — they live on the L1 (cfg4: 534 -> 480 M sims/s with it).
   if (!getenv("SMZ_NO_CARVEOUT"))
-    for (const void* f : {(const void*)k_bf16_chain_m64<64>, (const void*)k_bf16_chain_m64<96>, (const void*)k_bf16_chain_m32})
+    for (const void* f : {(const void*)k_bf16_chain_m64, (const void*)k_bf16_chain_m32})
       cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  im->pipe_rounds = getenv("SMZ_PIPE_ROUNDS") ? atoi(getenv("SMZ_PIPE_ROUNDS")) : 2;
   if (getenv("SMZ_BF16_TIMELINE")) {
     cudaMalloc(&im->timeline, (1 + 4 * MAXL + 32) * sizeof(long long));
     cudaMemset(im->timeline, 0, (1 + 4 * MAXL + 32) * sizeof(long long));
   }
-  cudaFuncSetAttribute((const void*)k_bf16_chain<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, im->smem_bytes);
-  cudaFuncSetAttribute((const void*)k_bf16_chain<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, im->smem_bytes);
-  cudaFuncSetAttribute((const void*)k_bf16_chain<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, im->smem_bytes);
+  cudaFuncSetAttribute((const void*)k_bf16_chain, cudaFuncAttributeMaxDynamicSharedMemorySize, im->smem_bytes);
   *out = im;
   return SMZ_OK;
 }
@@ -1975,10 +1460,7 @@ void smz_bf16_destroy(SmzBf16Image* im) {
                 t[1 + l * 4] - t[0], t[1 + l * 4 + 1] - t[1 + l * 4], t[1 + l * 4 + 2] - t[1 + l * 4 + 1],
                 t[1 + l * 4 + 3] - t[1 + l * 4 + 2]);
       const long long* h = t + 1 + 4 * MAXL;
-      if (im->timeline_mega)
-        fprintf(stderr, "  persistent kernel, last simulation: tree phase %lld | barrier %lld | sort+gather %lld | to first layer +%lld\n",
-                h[0] - t[0], h[1] - h[0], h[2] - h[1], t[1] - h[2]);
-      else if (h[0] && !h[1]) {
+      if (h[0] && !h[1]) {
         fprintf(stderr, "  pipelined kernel: dependency wait returned at +%lld (A operand of layer 0 complete %lld cycles later)\n",
                 h[0] - t[0], t[1] - h[0]);
         if (h[2])
@@ -2087,11 +1569,11 @@ void smz_bf16_root(SmzBf16Image* im, const SmzArena& a, const SmzNetShape& sh, i
   job.input_kind = IN_OBS; job.n_rows = n_trees; job.in = obs; job.obs = sh.obs; job.S = sh.S;
   job.hidden16_dst = reinterpret_cast<__nv_bfloat16*>(a.hidden);
   job.policy_dst = a.out_policy; job.value_dst = a.out_value; job.pstride = a.W;
-  k_bf16_chain<0><<<(n_trees + TM - 1) / TM, NTHREADS, im->smem_bytes, s>>>(a, im->chain_root, im->chain_root, job, 0);
+  k_bf16_chain<<<(n_trees + TM - 1) / TM, NTHREADS, im->smem_bytes, s>>>(a, im->chain_root, im->chain_root, job, 0);
 }
 
 void smz_bf16_sim(SmzBf16Image* im, const SmzArena& a, const SmzNetShape& sh, int n_trees, int sim, bool pdl,
-                  int tree_mode, cudaStream_t s) {
+                  cudaStream_t s) {
   Job job{};
   job.input_kind = IN_GATHER; job.n_rows = n_trees; job.S = sh.S;
   job.hidden16_dst = reinterpret_cast<__nv_bfloat16*>(a.hidden) + (size_t)(sim + 1) * a.B * SMZ_SP;
@@ -2105,50 +1587,24 @@ void smz_bf16_sim(SmzBf16Image* im, const SmzArena& a, const SmzNetShape& sh, in
   // "other" branch, so the one-wave condition is on row_top / tile
   const bool m64 = im->use_m64 < 0 ? a.row_top / TM64 <= im->n_sms : im->use_m64 != 0;
   const bool m32 = m64 && (im->use_m32 < 0 ? a.row_top / 32 <= im->n_sms : im->use_m32 != 0);
-  if (tree_mode == 0 && im->use_pipe && m64) {
-    const bool uneven = getenv("SMZ_M64_EVEN") == nullptr;     // 96 + 32 columns measured 2.7 % faster than 64 + 64
-    auto* k64 = m32 ? k_bf16_chain_m32 : (uneven ? k_bf16_chain_m64<96> : k_bf16_chain_m64<64>);
+  if (im->use_pipe && m64) {
+    auto* k64 = m32 ? k_bf16_chain_m32 : k_bf16_chain_m64;
     smz_launch(k64, dim3(a.row_top / (m32 ? 32 : TM64)), dim3(NPIPE), sizeof(Smem64) + 1024, s, pdl, a, im->chain_after,
                im->chain_dyn, job, sim);
     return;
   }
-  // tiles per CTA: 1 while the tiles fit one wave of SMs, else 2 (SMZ_PIPE2 = 0 / 1 / 2 / 4 forces).  Four per CTA put cfg4
-  // into ONE wave of 129 CTAs but measured slower than two waves of pairs (65536 trees 5.76 vs 5.16 ms, 32768 trees 4.02 vs 2.50)
+  // tiles per CTA: 1 while the tiles fit one wave of SMs, else 2 (SMZ_PIPE2 = 0 / 1 forces one / two)
   const int tiles = a.row_top / TM;
-  int nt = im->use_pipe2 < 0 ? (tiles <= im->n_sms ? 1 : 2) : (im->use_pipe2 == 1 ? 2 : im->use_pipe2);
-  if (nt != 2 && nt != 4) nt = 1;
-  if (tree_mode == 0 && im->use_pipe && nt > 1 && a.row_top % (nt * TM) == 0) {
-    if (nt == 2)
-      smz_launch(k_bf16_chain_pipeN<2>, dim3(tiles / 2), dim3(NPIPE), sizeof(SmemPipeN<2>) + 1024, s, pdl, a, im->chain_after, im->chain_dyn, job, sim);
-    else
-      smz_launch(k_bf16_chain_pipeN<4>, dim3(tiles / 4), dim3(NPIPE), sizeof(SmemPipeN<4>) + 1024, s, pdl, a, im->chain_after, im->chain_dyn, job, sim);
+  const bool two = im->use_pipe2 < 0 ? tiles > im->n_sms : im->use_pipe2 == 1;
+  if (im->use_pipe && two && a.row_top % (2 * TM) == 0) {
+    smz_launch(k_bf16_chain_pipeN<2>, dim3(tiles / 2), dim3(NPIPE), sizeof(SmemPipeN<2>) + 1024, s, pdl, a, im->chain_after, im->chain_dyn, job, sim);
     return;
   }
-  if (tree_mode == 0 && im->use_pipe) {
-    auto* kp = im->pipe_rounds == 4 ? k_bf16_chain_pipe<4> : k_bf16_chain_pipe<2>;
-    smz_launch(kp, dim3(a.row_top / TM), dim3(NPIPE), sizeof(SmemPipe) + 1024, s, pdl, a, im->chain_after, im->chain_dyn, job, sim);
+  if (im->use_pipe) {
+    smz_launch(k_bf16_chain_pipe, dim3(a.row_top / TM), dim3(NPIPE), sizeof(SmemPipe) + 1024, s, pdl, a, im->chain_after, im->chain_dyn, job, sim);
     return;
   }
-  auto* k = tree_mode == 2 ? k_bf16_chain<2> : (tree_mode == 1 ? k_bf16_chain<1> : k_bf16_chain<0>);
-  smz_launch(k, grid, block, (size_t)im->smem_bytes, s, pdl, a, im->chain_after, im->chain_dyn, job, sim);
-}
-
-bool smz_bf16_mega_supported(const SmzBf16Image* im, const SmzArena& a, int lanes) {
-  return im != nullptr && lanes == 4 && a.A <= 4 && a.C <= 4 && im->chain_after.n_layers == im->chain_dyn.n_layers;
-}
-
-// the whole simulation loop [first, first + n_sims) as one persistent launch, one CTA per 128 trees
-void smz_bf16_mega(SmzBf16Image* im, const SmzArena& a, const SmzNetShape& sh, int n_trees, int first, int n_sims,
-                   cudaStream_t s) {
-  const int smem = (int)sizeof(SmemMega) + 1024;
-  static bool attr_set = false;
-  if (!attr_set) {
-    cudaFuncSetAttribute((const void*)k_search_mega, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    attr_set = true;
-  }
-  k_search_mega<<<(n_trees + TM - 1) / TM, NTHREADS, smem, s>>>(a, im->chain_after, im->chain_dyn, n_trees, first, n_sims, sh.S,
-                                                                    im->timeline);
-  im->timeline_mega = 1;
+  smz_launch(k_bf16_chain, grid, block, (size_t)im->smem_bytes, s, pdl, a, im->chain_after, im->chain_dyn, job, sim);
 }
 
 void smz_bf16_eval(SmzBf16Image* im, const SmzNetShape& sh, int which, int n_rows, const float* in, const int* idx,
@@ -2160,5 +1616,5 @@ void smz_bf16_eval(SmzBf16Image* im, const SmzNetShape& sh, int which, int n_row
   job.hidden_dst = hidden_out; job.policy_dst = policy_out; job.value_dst = value_out; job.reward_dst = reward_out;
   job.code_dst = code_out; job.pstride = policy_stride;
   SmzArena dummy{};
-  k_bf16_chain<0><<<(n_rows + TM - 1) / TM, NTHREADS, im->smem_bytes, s>>>(dummy, im->chain_single[which], im->chain_single[which], job, 0);
+  k_bf16_chain<<<(n_rows + TM - 1) / TM, NTHREADS, im->smem_bytes, s>>>(dummy, im->chain_single[which], im->chain_single[which], job, 0);
 }

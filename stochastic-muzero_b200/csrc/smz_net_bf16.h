@@ -13,17 +13,10 @@ int smz_bf16_pack(SmzBf16Image* im, const SmzNetShape& sh, const float* blob_dev
                   size_t err_len);
 void smz_bf16_root(SmzBf16Image* im, const SmzArena& a, const SmzNetShape& sh, int n_trees, const float* obs,
                    cudaStream_t s);
-// tree_mode: 0 = network step only; 1 = + expansion/backup of `sim` in the kernel tail; 2 = + descent of sim+1
-// (1 and 2 need 4 lanes per tree, i.e. policy widths <= 4)
 void smz_bf16_sim(SmzBf16Image* im, const SmzArena& a, const SmzNetShape& sh, int n_trees, int sim, bool pdl,
-                  int tree_mode, cudaStream_t s);
+                  cudaStream_t s);
 void smz_bf16_eval(SmzBf16Image* im, const SmzNetShape& sh, int which, int n_rows, const float* in, const int* idx,
                    float* hidden_out, float* policy_out, float* value_out, float* reward_out, int* code_out,
                    int policy_stride, cudaStream_t s);
 // bf16 mode keeps the arena's hidden-state store in bf16 ([slot][B][64]); this widens one slot to fp32 rows
 void smz_bf16_read_hidden(const SmzArena& a, int slot, int n_trees, float* out, cudaStream_t s);
-// Persistent per-tile search kernel: the whole loop of simulations [first, first + n_sims) in one launch (needs
-// 4 lanes per tree, i.e. policy widths <= 4)
-bool smz_bf16_mega_supported(const SmzBf16Image* im, const SmzArena& a, int lanes);
-void smz_bf16_mega(SmzBf16Image* im, const SmzArena& a, const SmzNetShape& sh, int n_trees, int first, int n_sims,
-                   cudaStream_t s);

@@ -1,6 +1,6 @@
 // smz_tc_ptx.cuh — PTX wrappers shared by the tensor-core network-step kernels (smz_net_bf16.cu, smz_net_tc32.cu):
 // mbarriers, bulk (TMA) copies, proxy / tcgen05 fences, UMMA shared-memory descriptors, the tensor-memory-A form of
-// tcgen05.mma, tcgen05.commit, the tcgen05.ld / tcgen05.st shapes the epilogues use, and the head-layer reductions (softmax expectation over the categorical
+// tcgen05.mma, TMEM allocation, tcgen05.commit, the tcgen05.ld / tcgen05.st shapes the epilogues use, and the head-layer reductions (softmax expectation over the categorical
 // support, muzero_model.py:575-591).
 #pragma once
 #include <cuda_bf16.h>
@@ -75,6 +75,14 @@ __device__ __forceinline__ void umma_ts(unsigned tmem_d, unsigned tmem_a, unsign
       "tcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}" ::"r"(tmem_d),
       "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accum)
       : "memory");
+}
+// whole warp: ncols TMEM columns, their address written to *base in shared memory; then give up the allocation permit
+__device__ __forceinline__ void tmem_alloc(unsigned* base, unsigned ncols) {
+  asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(s32(base)), "r"(ncols) : "memory");
+  asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+__device__ __forceinline__ void tmem_dealloc(unsigned base, unsigned ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "r"(ncols) : "memory");
 }
 __device__ __forceinline__ void umma_commit(unsigned long long* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(s32(bar)) : "memory");

@@ -75,7 +75,7 @@ __global__ void k_select(SmzArena a, int n_trees, int sim, int* __restrict__ o_s
   ts.mm = a.minmax[tree];
   const int4 rs = a.stat[(size_t)tree * a.M];
   ts.root = make_int2(rs.x, rs.y);
-  select_phase<G, true, false, true>(g, a, rng, tree, alive, sim, ts, o_slot, o_action, o_branch);
+  select_phase<G>(g, a, rng, tree, alive, sim, ts, o_slot, o_action, o_branch);
 }
 
 template <int G>
@@ -106,7 +106,7 @@ __global__ void k_backup_select(SmzArena a, int n_trees, int sim) {
   const TreeState ts = expand_backup_phase(g, a, rng, tree, alive, sim, a.out_policy, a.W, a.out_value, a.out_reward);
   __syncwarp();
   if (stamp) a.dbg[1] = clock64();
-  select_phase<G, true, false, true>(g, a, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr);
+  select_phase<G>(g, a, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr);
   if (stamp) { a.dbg[2] = clock64(); a.dbg[3] = a.path_len[tree]; }
 }
 
@@ -173,7 +173,7 @@ __global__ void k_backup_select_sm(SmzArena a, int n_trees, int sim, int n_tab) 
                                                     sst, slk);
   __syncwarp();
   if (stamp) a.dbg[1] = clock64();
-  select_phase<G, true, true, true>(g, al, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr, sst, slk, srp);
+  select_phase<G, true>(g, al, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr, sst, slk, srp);
   if (stamp) { a.dbg[2] = clock64(); a.dbg[3] = a.path_len[tree]; }
   if (a.dbg) {
     __syncthreads();

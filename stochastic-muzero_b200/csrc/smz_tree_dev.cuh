@@ -1,5 +1,4 @@
-// smz_tree_dev.cuh — device-side tree phases shared by the stand-alone tree kernels (smz_tree.cu) and the
-// network-step kernel that runs them in its tail (smz_net_bf16.cu).  Everything that decides a visit order uses
+// smz_tree_dev.cuh — device-side tree phases of the tree kernels (smz_tree.cu).  Everything that decides a visit order uses
 // explicit round-to-nearest intrinsics, so the translation unit's -fmad setting does not matter here.
 #pragma once
 #include "smz_common.cuh"
@@ -219,9 +218,9 @@ struct TreeState {
 
 // The search path is kept as one int4 record per level {node, visit_count, value_sum, reward} captured
 // while descending, so the backup needs ONE round trip (the record) instead of two (index -> stat).
-// COMPACT: append the tree to the per-branch row list of the simulation (one atomic per tree) for kernels that
-// re-tile the leaves by branch; the persistent per-tile kernel sorts its own rows instead.
-template <int G, bool COMPACT = true, bool MIRROR = false, bool BLOCKAGG = false>
+// The tree is appended to the per-branch row list of the simulation, from which the network step tiles its leaves.
+// Called by every thread of the block: the row reservation below synchronises the block.
+template <int G, bool MIRROR = false>
 __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& a, const SmzRng& rng, int tree, bool alive,
                                              int sim, TreeState ts, int* __restrict__ o_slot, int* __restrict__ o_action,
                                              int* __restrict__ o_branch, const int4* __restrict__ sst = nullptr,
@@ -339,15 +338,15 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
     ++level;
   }
   if (a.dbg && blockIdx.x == 0 && threadIdx.x == 0) { a.dbg[4] = clock64(); a.dbg[5] = level; }
-  // ---- leaf record.  The row compaction and the depth statistic are aggregated per warp: one atomic per branch
-  //      (and one for the depth sum) per warp instead of one per tree — thousands of same-address atomics per
+  // ---- leaf record.  The row compaction is aggregated per block (one global atomic per branch per block) and the
+  //      depth statistic per warp, instead of one atomic per tree — thousands of same-address atomics per
   //      simulation serialise in the L2 and their return value is on the critical path of the kernel.
   const bool lead = alive && g.gl == 0;
   const int branch = ((depth >> 1) & 1) ? SMZ_BRANCH_DYNAMICS : SMZ_BRANCH_AFTERSTATE;
   const int slot = (cbase == 1) ? 0 : (cbase - 1 - a.A) / a.Kmax + 1;
   // the parent's hidden row is requested now and stored once the row index is known (bf16 network: a.xin)
   uint4 hcopy[(G < 8) ? 8 / G : 1], hcopy2[(G < 8) ? 8 / G : 1];
-  const bool copy_row = COMPACT && a.xin != nullptr && alive;
+  const bool copy_row = a.xin != nullptr && alive;
   const bool wide_row = a.xin_q > 8;          // fp16 hi + lo rows (SMZ_NET_TC32): a second batch of 8 pieces
   if (copy_row) {
     const uint4* src = reinterpret_cast<const uint4*>(a.hidden) + ((size_t)slot * a.B + tree) * a.xin_q;
@@ -358,53 +357,37 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
       if (wide_row) hcopy2[j] = idx < 8 ? src[8 + idx] : make_uint4(0, 0, 0, 0);
     }
   }
+  // warps reserve ranks in shared memory, two threads reserve the block's rows globally
   int r = 0;
-  if (COMPACT) {
+  {
     const unsigned lane = threadIdx.x & 31u;
-    if constexpr (BLOCKAGG) {
-      // whole-block kernels: warps reserve ranks in shared memory, two threads reserve the block's rows globally
-      __shared__ int s_cnt[2], s_base[2];
-      if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
-      __syncthreads();
+    __shared__ int s_cnt[2], s_base[2];
+    if (threadIdx.x < 2) s_cnt[threadIdx.x] = 0;
+    __syncthreads();
 #pragma unroll
-      for (int b = 0; b < 2; ++b) {
-        const unsigned m = __ballot_sync(FULL, lead && branch == b);
-        if (m) {
-          const int leader = __ffs(m) - 1;
-          int base = 0;
-          if ((int)lane == leader) base = atomicAdd(&s_cnt[b], __popc(m));
-          base = __shfl_sync(FULL, base, leader);
-          if (lead && branch == b) r = base + __popc(m & ((1u << lane) - 1u));
-        }
-      }
-      __syncthreads();
-      if (threadIdx.x < 2) s_base[threadIdx.x] = s_cnt[threadIdx.x] ? atomicAdd(&a.branch_count[sim * 2 + threadIdx.x], s_cnt[threadIdx.x]) : 0;
-      __syncthreads();
-      r += s_base[branch];
-    } else {
-#pragma unroll
-      for (int b = 0; b < 2; ++b) {
-        const unsigned m = __ballot_sync(FULL, lead && branch == b);
-        if (m) {
-          const int leader = __ffs(m) - 1;
-          int base = 0;
-          if ((int)lane == leader) base = atomicAdd(&a.branch_count[sim * 2 + b], __popc(m));
-          base = __shfl_sync(FULL, base, leader);
-          if (lead && branch == b) r = base + __popc(m & ((1u << lane) - 1u));
-        }
+    for (int b = 0; b < 2; ++b) {
+      const unsigned m = __ballot_sync(FULL, lead && branch == b);
+      if (m) {
+        const int leader = __ffs(m) - 1;
+        int base = 0;
+        if ((int)lane == leader) base = atomicAdd(&s_cnt[b], __popc(m));
+        base = __shfl_sync(FULL, base, leader);
+        if (lead && branch == b) r = base + __popc(m & ((1u << lane) - 1u));
       }
     }
+    __syncthreads();
+    if (threadIdx.x < 2) s_base[threadIdx.x] = s_cnt[threadIdx.x] ? atomicAdd(&a.branch_count[sim * 2 + threadIdx.x], s_cnt[threadIdx.x]) : 0;
+    __syncthreads();
+    r += s_base[branch];
   }
-  if (COMPACT) {
-    const int rg = g.bcast(r, 0);
-    if (copy_row) {
-      uint4* dst = a.xin + smz_row_index(a, sim, branch, rg) * a.xin_q;
+  const int rg = g.bcast(r, 0);
+  if (copy_row) {
+    uint4* dst = a.xin + smz_row_index(a, sim, branch, rg) * a.xin_q;
 #pragma unroll
-      for (int j = 0; j < ((G < 8) ? 8 / G : 1); ++j) {
-        const int idx = g.gl + j * G;
-        if (idx < 8) dst[idx] = hcopy[j];
-        if (wide_row && idx < 8) dst[8 + idx] = hcopy2[j];
-      }
+    for (int j = 0; j < ((G < 8) ? 8 / G : 1); ++j) {
+      const int idx = g.gl + j * G;
+      if (idx < 8) dst[idx] = hcopy[j];
+      if (wide_row && idx < 8) dst[8 + idx] = hcopy2[j];
     }
   }
   {
@@ -423,10 +406,8 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
     if (o_slot) o_slot[tree] = slot;
     if (o_action) o_action[tree] = child_key;
     if (o_branch) o_branch[tree] = branch;
-    if (COMPACT) {
-      a.rows[smz_row_index(a, sim, branch, r)] = tree;
-      a.rows4[smz_row_index(a, sim, branch, r)] = make_int4(tree, slot, child_key, 0);
-    }
+    a.rows[smz_row_index(a, sim, branch, r)] = tree;
+    a.rows4[smz_row_index(a, sim, branch, r)] = make_int4(tree, slot, child_key, 0);
   }
 }
 

@@ -811,10 +811,7 @@ def test_api_misuse_is_reported_not_executed():
 _VARIANTS = {
     "chain_one_thread_issue": {"SMZ_NO_PIPE": "1"},
     "chain_128_rows_2_rounds": {"SMZ_M64": "0"},
-    "chain_128_rows_4_rounds": {"SMZ_M64": "0", "SMZ_PIPE_ROUNDS": "4"},
-    "chain_128_rows_two_tiles_per_cta": {"SMZ_M64": "0", "SMZ_PIPE2": "2"},
-    "chain_128_rows_four_tiles_per_cta": {"SMZ_M64": "0", "SMZ_PIPE2": "4"},
-    "chain_64_rows_even_rounds": {"SMZ_M64": "1", "SMZ_M32": "0", "SMZ_M64_EVEN": "1"},
+    "chain_128_rows_two_tiles_per_cta": {"SMZ_M64": "0", "SMZ_PIPE2": "1"},
     "chain_64_rows_64_leaves": {"SMZ_M64": "1", "SMZ_M32": "0"},
     "chain_64_rows_32_leaves": {"SMZ_M64": "1", "SMZ_M32": "1"},
     "chain_32_leaves_every_tile_streamed": {"SMZ_M64": "1", "SMZ_M32": "1", "SMZ_STREAM_ALL": "1"},
@@ -823,7 +820,7 @@ _VARIANTS = {
 
 
 def _bf16_search_record(monkeypatch, env, B=300, N=50):
-    for k in ("SMZ_NO_PIPE", "SMZ_M64", "SMZ_M32", "SMZ_PIPE2", "SMZ_STREAM_ALL", "SMZ_PIPE_ROUNDS", "SMZ_M64_EVEN", "SMZ_NO_TREE_SMEM"):
+    for k in ("SMZ_NO_PIPE", "SMZ_M64", "SMZ_M32", "SMZ_PIPE2", "SMZ_STREAM_ALL", "SMZ_NO_TREE_SMEM"):
         monkeypatch.delenv(k, raising=False)
     for k, v in env.items():
         monkeypatch.setenv(k, v)
