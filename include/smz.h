@@ -77,7 +77,8 @@ typedef struct smz_config {
   double root_exploration_fraction;
   /* MLP shape (muzero_model.py ctor: observation/state_space_dimensions, hidden_layer_dimensions,
    * number_of_hidden_layer).  Ignored when net_mode == SMZ_NET_EXTERNAL. */
-  int32_t obs_dim;
+  int32_t obs_dim;           /* flattened observation width, 1..8192 for the MLP modes (the first layer streams its K
+                              * through the tensor / CUDA cores in slices of 128); 3*98*98 for SMZ_NET_VISION */
   int32_t state_dim;         /* S: hidden-state width and categorical-support size */
   int32_t hidden_dim;        /* H */
   int32_t num_hidden_layers; /* L (weight-tied, neural_network_mlp_model.py:31-37) */

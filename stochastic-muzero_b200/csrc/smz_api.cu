@@ -130,9 +130,12 @@ int smz_create(const smz_config* cfg, smz_engine** out) {
   } else if (c.net_mode != SMZ_NET_EXTERNAL) {
     if (c.obs_dim < 1 || c.state_dim < 2 || c.hidden_dim < 1 || c.num_hidden_layers < 0)
       return fail(SMZ_E_INVALID_ARG, "smz_create: model shape out of range");
-    if (c.hidden_dim > SMZ_HP || c.state_dim > SMZ_SP || c.obs_dim > SMZ_HP)
-      return fail(SMZ_E_CAPACITY, "smz_create: fused MLP tiles hold H<=%d, S<=%d, obs<=%d (got %d, %d, %d)",
-                  SMZ_HP, SMZ_SP, SMZ_HP, c.hidden_dim, c.state_dim, c.obs_dim);
+    if (c.hidden_dim > SMZ_HP || c.state_dim > SMZ_SP)
+      return fail(SMZ_E_CAPACITY, "smz_create: fused MLP tiles hold H<=%d, S<=%d (got %d, %d)",
+                  SMZ_HP, SMZ_SP, c.hidden_dim, c.state_dim);
+    if (c.obs_dim > SMZ_MAX_OBS)
+      return fail(SMZ_E_CAPACITY, "smz_create: observations of the MLP family are limited to obs_dim<=%d (got %d)",
+                  SMZ_MAX_OBS, c.obs_dim);
   }
   int need = pow2ceil(c.action_dim > c.chance_dim ? c.action_dim : c.chance_dim);
   if (need < 2) need = 2;

@@ -17,6 +17,7 @@
 #define SMZ_MAX_POLICY 32   // widest policy head handled by the lane-per-entry tree kernels
 #define SMZ_HP 128          // padded hidden width of the MLP tiles
 #define SMZ_SP 64           // padded state width
+#define SMZ_MAX_OBS 8192    // widest observation of the MLP family (an 84 x 84 frame flattened is 7056)
 #define SMZ_VISION_SP 160   // hidden-row stride of the vision family: 3*7*7 = 147 floats padded to 160
 
 struct SmzArena {

@@ -119,6 +119,17 @@ __device__ __forceinline__ void load_weight_tile(const Chain& c, int l, unsigned
   bulk_g2s(w[slot], c.layer[l].w, bytes, &wbar[slot]);
 }
 
+// k_bf16_chain streams the K of a first layer wider than KMAX (an observation of more than 128 features) in slices of
+// KMAX through the same ring: ring tile t < ns is slice t of layer 0, tile ns - 1 + l is layer l >= 1.  The image is
+// K-major, so a slice is one contiguous piece of it.
+__device__ __forceinline__ void load_ring_tile(const Chain& c, int t, int ns, unsigned long long* wbar, unsigned char (*w)[W_BYTES],
+                                               int slot) {
+  if (t >= ns) { load_weight_tile(c, t - ns + 1, wbar, w, slot); return; }
+  const unsigned bytes = (unsigned)min(KMAX, c.layer[0].K - t * KMAX) * TN * 2;
+  mbar_expect_tx(&wbar[slot], bytes);
+  bulk_g2s(w[slot], c.layer[0].w + (size_t)t * KMAX * TN, bytes, &wbar[slot]);
+}
+
 // K-chunk kc (8 columns) of the one-hot block of a row whose action / code is act (-1 = none)
 __device__ __forceinline__ uint4 onehot_chunk(int act, int kc) {
   unsigned w4[4] = {0, 0, 0, 0};
@@ -263,6 +274,10 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
     tile -= branch * T;
   }
   const Chain& ch = branch ? chain1 : chain0;
+  // K slices of the first layer (1 unless an observation is wider than KMAX); see load_ring_tile.  Ring tile and
+  // accumulator-barrier phase of layer l: t = l + ns - 1.
+  const int ns = (ch.kin + KMAX - 1) / KMAX;
+  const int n_tiles = ch.n_layers + ns - 1;
 
   // ---- barriers + first weight tiles (one thread), TMEM allocation (warp 0): all of it overlaps the
   //      dependent global loads of the gather below; one barrier publishes everything ----------------
@@ -275,8 +290,8 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
     const unsigned bbytes = (unsigned)ch.n_layers * TN * 4;
     mbar_expect_tx(&sm.bbar, bbytes);
     bulk_g2s(sm.bias, ch.bias, bbytes, &sm.bbar);
-    load_weight_tile(ch, 0, sm.wbar, sm.w, 0);
-    if (ch.n_layers > 1) load_weight_tile(ch, 1, sm.wbar, sm.w, 1);
+    load_ring_tile(ch, 0, ns, sm.wbar, sm.w, 0);
+    if (n_tiles > 1) load_ring_tile(ch, 1, ns, sm.wbar, sm.w, 1);
   }
   __syncwarp();
   if (warp == 0) tmem_alloc(&sm.tmem_base, TN);
@@ -291,24 +306,40 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   const int row = tile * TM + r;
   const bool valid = row < count;
   if (tile * TM >= count) {
-    idle_cta_exit(&sm.bbar, sm.wbar, ch.n_layers > 1, sm.tmem_base, TN);
+    idle_cta_exit(&sm.bbar, sm.wbar, n_tiles > 1, sm.tmem_base, TN);
     return;
   }
+
+  // K slice s of this thread's observation row, K-chunks cb, cb + 4, cb + 8, cb + 12 (8 columns each), packed to bf16;
+  // loaded into registers first, so that the next slice's loads are in flight while the tensor core works on this one
+  auto load_obs_slice = [&](int s, uint4 (&o)[4]) {
+    const int k0 = s * KMAX;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      float v[8];
+#pragma unroll
+      for (int j = 0; j < 8; ++j) {
+        const int c = k0 + (cb + 4 * i) * 8 + j;
+        v[j] = (valid && c < job.obs) ? job.in[(size_t)row * job.obs + c] : 0.f;
+      }
+      o[i] = make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7]));
+    }
+  };
+  auto store_obs_slice = [&](int s, const uint4 (&o)[4]) {
+    const int kw = min(KMAX, ch.kin - s * KMAX);
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+      if ((cb + 4 * i) * 8 < kw) a_store(sm.a, r, cb + 4 * i, o[i]);
+  };
 
   // ---- stage the first A operand: bf16, canonical K-major layout; thread (r, cb) fills its K-chunks ---
   int index = -1;      // tree id (gather) or caller row: where this row's outputs go
   {
     if (job.input_kind == IN_OBS) {
       index = valid ? row : -1;
-      for (int kc = cb; kc < ch.kin / 8; kc += 4) {
-        float v[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          const int c = kc * 8 + j;
-          v[j] = (valid && c < job.obs) ? job.in[(size_t)row * job.obs + c] : 0.f;
-        }
-        a_store(sm.a, r, kc, make_uint4(pack_bf16(v[0], v[1]), pack_bf16(v[2], v[3]), pack_bf16(v[4], v[5]), pack_bf16(v[6], v[7])));
-      }
+      uint4 o[4];
+      load_obs_slice(0, o);
+      store_obs_slice(0, o);
     } else {
       const float* src = nullptr;
       const __nv_bfloat16* src16 = nullptr;   // arena rows are already bf16: copied straight into the operand
@@ -346,6 +377,33 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   __syncthreads();
   tc_fence_after();
   const unsigned tmem = sm.tmem_base;
+
+  // ---- a first layer wider than KMAX: every K slice but the last accumulates into the layer-0 accumulator; the
+  //      last one is layer 0 of the loop below -------------------------------------------------------------------
+  if (tid == 0) mbar_wait(&sm.wbar[0], 0);
+  for (int s = 0; s + 1 < ns; ++s) {
+    if (tid == 0) {
+      tc_fence_after();
+      const unsigned long long ad = umma_desc(s32(sm.a), CHUNK_A, 128), bd = umma_desc(s32(sm.w[s & 1]), CHUNK_W, 128);
+#pragma unroll
+      for (int k = 0; k < 8; ++k)
+        umma(tmem, ad + (unsigned long long)(k * ((2 * CHUNK_A) >> 4)), bd + (unsigned long long)(k * ((2 * CHUNK_W) >> 4)),
+             (s > 0 || k > 0) ? 1u : 0u);
+      umma_commit(&sm.mbar);
+      mbar_wait(&sm.wbar[(s + 1) & 1], ((s + 1) >> 1) & 1);
+    }
+    uint4 o[4];
+    load_obs_slice(s + 1, o);
+    mbar_wait(&sm.mbar, s & 1);
+    __syncwarp();
+    tc_fence_after();
+    if (tid == 0 && s + 2 < n_tiles) load_ring_tile(ch, s + 2, ns, sm.wbar, sm.w, s & 1);   // ring slot s&1 is free again
+    store_obs_slice(s + 1, o);
+    fence_async_smem();
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+  }
   mbar_wait(&sm.bbar, 0);
 
   const unsigned taddr = tmem + ((unsigned)((warp & 3) * 32) << 16) + (unsigned)(cb * 32);
@@ -353,29 +411,29 @@ k_bf16_chain(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   const int c0 = cb * 32;
 
   // ---- the layer loop ---------------------------------------------------------------------------------
-  if (tid == 0) mbar_wait(&sm.wbar[0], 0);
   for (int l = 0; l < ch.n_layers; ++l) {
-    const int K = ch.layer[l].K, kind = ch.layer[l].kind;
+    const int K = l ? ch.layer[l].K : ch.kin - (ns - 1) * KMAX, kind = ch.layer[l].kind;
+    const int t = l + ns - 1;          // ring tile of this layer (= completed accumulator phases before it)
     if (tid == 0) {
       if (stamp) job.timeline[1 + l * 4 + 0] = clock64();
       tc_fence_after();
       // descriptors advance by two K-chunks per MMA: only the 14-bit start-address field changes
-      const unsigned long long ad = umma_desc(s32(sm.a), CHUNK_A, 128), bd = umma_desc(s32(sm.w[l & 1]), CHUNK_W, 128);
+      const unsigned long long ad = umma_desc(s32(sm.a), CHUNK_A, 128), bd = umma_desc(s32(sm.w[t & 1]), CHUNK_W, 128);
       const int nk = K / 16;
-      umma(tmem, ad, bd, 0u);
+      umma(tmem, ad, bd, (l == 0 && ns > 1) ? 1u : 0u);
 #pragma unroll
       for (int k = 1; k < 8; ++k)
         if (k < nk) umma(tmem, ad + (unsigned long long)(k * ((2 * CHUNK_A) >> 4)), bd + (unsigned long long)(k * ((2 * CHUNK_W) >> 4)), 1u);
       umma_commit(&sm.mbar);
       if (stamp) job.timeline[1 + l * 4 + 1] = clock64();
       // the next layer's weights were requested two layers ago: absorb that wait while the MMAs run
-      if (l + 1 < ch.n_layers) mbar_wait(&sm.wbar[(l + 1) & 1], ((l + 1) >> 1) & 1);
+      if (l + 1 < ch.n_layers) mbar_wait(&sm.wbar[(t + 1) & 1], ((t + 1) >> 1) & 1);
     }
-    mbar_wait(&sm.mbar, l & 1);
+    mbar_wait(&sm.mbar, t & 1);
     __syncwarp();       // tcgen05.ld below is .sync.aligned: reconverge after the spin loop
     if (stamp) job.timeline[1 + l * 4 + 2] = clock64();
     tc_fence_after();
-    if (tid == 0 && l + 2 < ch.n_layers) load_weight_tile(ch, l + 2, sm.wbar, sm.w, l & 1);   // ring slot l&1 is free again
+    if (tid == 0 && l + 2 < ch.n_layers) load_weight_tile(ch, l + 2, sm.wbar, sm.w, t & 1);   // ring slot t&1 is free again
     __syncwarp();
     const float* bias = sm.bias[l] + c0;
 

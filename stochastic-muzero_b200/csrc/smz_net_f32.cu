@@ -102,6 +102,74 @@ __device__ void dense(const float* __restrict__ wt, int K, const float* __restri
   __syncthreads();
 }
 
+// First layer of a network that reads caller rows of any width (the observation of repr / enc):
+// out[r][c] = elu( sum_k in[row0 + r][k] * Wt[k][c] + b[c] ).  The input streams through xs in slices of SMZ_HP
+// columns, re-staged whenever the k-slab ring crosses into the next slice, and the products are accumulated in the
+// same order as dense() does over a staged row — so for in_w <= SMZ_HP the result is bit-identical to staging the
+// whole row and calling dense().
+__device__ void dense_wide_in(const SmzNetF32& net, const float* __restrict__ in, int in_w, int row0, int n_rows,
+                              float (*xs)[LD], float (*out)[LD], float (*wbuf)[KC][SMZ_HP]) {
+  const int tid = threadIdx.x, tx = tid & 15, ty = tid >> 4;
+  float acc[2][8];
+#pragma unroll
+  for (int i = 0; i < 2; ++i)
+#pragma unroll
+    for (int j = 0; j < 8; ++j) acc[i][j] = 0.f;
+  const int nchunks = net.kin_pad / KC;
+  auto issue = [&](int c) {
+    const float* src = net.in_wt + (size_t)c * KC * SMZ_HP;
+    float* dst = &wbuf[c & 1][0][0];
+#pragma unroll
+    for (int i = 0; i < (KC * SMZ_HP / 4) / NT; ++i) {
+      const int e = (i * NT + tid) * 4;
+      cp_async16(dst + e, src + e);
+    }
+    cp_async_commit();
+  };
+  issue(0);
+  for (int c = 0; c < nchunks; ++c) {
+    const int kc = (c * KC) % SMZ_HP;          // column of this k-slab inside the staged slice
+    if (kc == 0) {                             // every thread is past the previous slice (barrier ending the last slab)
+      const int k0 = c * KC, w = min(SMZ_HP, net.kin_pad - k0);
+      for (int e = tid; e < R * w; e += NT) {
+        const int r = e / w, k = e % w;
+        xs[r][k] = (row0 + r < n_rows && k0 + k < in_w) ? in[(size_t)(row0 + r) * in_w + k0 + k] : 0.f;
+      }
+    }
+    if (c + 1 < nchunks) { issue(c + 1); cp_async_wait<1>(); } else { cp_async_wait<0>(); }
+    __syncthreads();
+    const float(*w)[SMZ_HP] = wbuf[c & 1];
+#pragma unroll
+    for (int kk = 0; kk < KC; kk += 4) {
+      const float4 a0 = *reinterpret_cast<const float4*>(&xs[ty * 2][kc + kk]);
+      const float4 a1 = *reinterpret_cast<const float4*>(&xs[ty * 2 + 1][kc + kk]);
+      const float av0[4] = {a0.x, a0.y, a0.z, a0.w}, av1[4] = {a1.x, a1.y, a1.z, a1.w};
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const float4 b0 = *reinterpret_cast<const float4*>(&w[kk + q][tx * 8]);
+        const float4 b1 = *reinterpret_cast<const float4*>(&w[kk + q][tx * 8 + 4]);
+        const float bv[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {
+          acc[0][j] = fmaf(av0[q], bv[j], acc[0][j]);
+          acc[1][j] = fmaf(av1[q], bv[j], acc[1][j]);
+        }
+      }
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int i = 0; i < 2; ++i) {
+    const int r = ty * 2 + i;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const int c = tx * 8 + j;
+      out[r][c] = elu(acc[i][j] + net.in_b[c]);
+    }
+  }
+  __syncthreads();
+}
+
 // in-layer + L tied hidden layers + concatenated heads.  Returns the buffer holding the head tile;
 // *free_buf receives the other one.
 __device__ float (*run_net(const SmzNetF32& net, int L, float (*in)[LD], float (*other)[LD], const int* idx_s,
@@ -110,6 +178,22 @@ __device__ float (*run_net(const SmzNetF32& net, int L, float (*in)[LD], float (
   float(*nxt)[LD] = other;
   dense(net.in_wt, net.kin_pad, net.in_b, net.emb, idx_s, cur, nxt, true, wbuf);
   { auto t = cur; cur = nxt; nxt = t; }
+  for (int l = 0; l < L; ++l) {
+    dense(net.mid_wt, SMZ_HP, net.mid_b, nullptr, nullptr, cur, nxt, true, wbuf);
+    auto t = cur; cur = nxt; nxt = t;
+  }
+  dense(net.head_wt, SMZ_HP, net.head_b, nullptr, nullptr, cur, nxt, false, wbuf);
+  *free_buf = cur;
+  return nxt;
+}
+
+// run_net for a network whose input is caller rows [n_rows][in_w] in global memory (the observation):
+// the first layer streams them through x, the result lands in y.
+__device__ float (*run_net_wide_in(const SmzNetF32& net, int L, const float* in, int in_w, int row0, int n_rows,
+                                   float (*x)[LD], float (*y)[LD], float (*wbuf)[KC][SMZ_HP], float (**free_buf)[LD]))[LD] {
+  dense_wide_in(net, in, in_w, row0, n_rows, x, y, wbuf);
+  float(*cur)[LD] = y;
+  float(*nxt)[LD] = x;
   for (int l = 0; l < L; ++l) {
     dense(net.mid_wt, SMZ_HP, net.mid_b, nullptr, nullptr, cur, nxt, true, wbuf);
     auto t = cur; cur = nxt; nxt = t;
@@ -236,13 +320,8 @@ __global__ void __launch_bounds__(NT) k_net_root(SmzArena a, SmzNetShape sh, Smz
   extern __shared__ __align__(16) unsigned char smem_raw[];
   Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, row0 = blockIdx.x * R;
-  for (int e = tid; e < R * sh.obs_pad; e += NT) {
-    const int r = e / sh.obs_pad, c = e % sh.obs_pad;
-    sm.x[r][c] = (row0 + r < n_trees && c < sh.obs) ? obs[(size_t)(row0 + r) * sh.obs + c] : 0.f;
-  }
-  __syncthreads();
   float(*fre)[LD];
-  float(*head)[LD] = run_net(img.repr, sh.L, sm.x, sm.y, nullptr, sm.w, &fre);
+  float(*head)[LD] = run_net_wide_in(img.repr, sh.L, obs, sh.obs, row0, n_trees, sm.x, sm.y, sm.w, &fre);
   for (int r = warp; r < R; r += NT / 32) {
     const int tree = row0 + r;
     state_epilogue(head[r], sh.S, fre[r], tree < n_trees ? a.hidden + (size_t)tree * SMZ_SP : nullptr);
@@ -268,16 +347,18 @@ __global__ void __launch_bounds__(NT) k_net_eval(SmzNetShape sh, SmzNetImageF32 
   Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
   const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, row0 = blockIdx.x * R;
   const bool from_obs = (which == 0 || which == 5);
-  const int in_w = from_obs ? sh.obs : SMZ_SP, in_pad = from_obs ? sh.obs_pad : SMZ_SP;
-  for (int e = tid; e < R * in_pad; e += NT) {
-    const int r = e / in_pad, c = e % in_pad;
-    sm.x[r][c] = (row0 + r < n_rows && c < in_w) ? in[(size_t)(row0 + r) * in_w + c] : 0.f;
+  if (!from_obs) {
+    for (int e = tid; e < R * SMZ_SP; e += NT) {
+      const int r = e / SMZ_SP, c = e % SMZ_SP;
+      sm.x[r][c] = row0 + r < n_rows ? in[(size_t)(row0 + r) * SMZ_SP + c] : 0.f;
+    }
   }
   if (tid < R) sm.idx[tid] = (idx && row0 + tid < n_rows) ? idx[row0 + tid] : -1;
   __syncthreads();
   const SmzNetF32* nets[6] = {&img.repr, &img.pred, &img.adyn, &img.apred, &img.dyn, &img.enc};
   float(*fre)[LD];
-  float(*head)[LD] = run_net(*nets[which], sh.L, sm.x, sm.y, (which == 2 || which == 4) ? sm.idx : nullptr, sm.w, &fre);
+  float(*head)[LD] = from_obs ? run_net_wide_in(*nets[which], sh.L, in, sh.obs, row0, n_rows, sm.x, sm.y, sm.w, &fre)
+                              : run_net(*nets[which], sh.L, sm.x, sm.y, (which == 2 || which == 4) ? sm.idx : nullptr, sm.w, &fre);
   for (int r = warp; r < R; r += NT / 32) {
     const int row = row0 + r;
     const bool ok = row < n_rows;

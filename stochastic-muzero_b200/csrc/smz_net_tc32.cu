@@ -113,6 +113,7 @@ struct SmemT {
   float4 part[4][TM];       // head layers, first exchange: row min / max (state) or row max (softmax) per column block
   float4 part2[4][TM];      // second exchange: softmax sums.  A later head layer reuses both only after every warp has
                             // passed the named-barrier arrivals that follow its reads (the accumulator wait implies them)
+  unsigned long long sbar;  // WIDE: "the MMAs of a K slice of the first layer have completed"
 };
 
 template <bool STACKED>
@@ -186,7 +187,12 @@ __device__ __forceinline__ float act32(float x) { return RELU ? fmaxf(x, 0.f) : 
 // one product; "f16" throughput mode: 11-bit significands instead of bf16's 8, same speed class as the bf16 chain;
 // arena rows are then 64 fp16 = 128 B and the head exponentials use ex2.approx).
 // RELU: the vision heads use nn.ReLU between their Linear layers (the MLP family nn.ELU).
-template <int NPROD, bool EXACT, bool RELU, int KA>
+// WIDE: the observation of an IN_OBS job is wider than KMAX.  The first layer's K then streams in ns slices of KMAX
+// through the same weight ring and A operand, all accumulated into the layer-0 accumulator: ring tile t < ns is slice t,
+// tile ns - 1 + l is layer l >= 1.  The epilogue stages slice s + 1 once the MMAs of slice s have completed (sbar); the
+// last slice is issued as layer 0 of the ordinary loop.  A separate instantiation, so the simulation step's code is
+// untouched by it.
+template <int NPROD, bool EXACT, bool RELU, int KA, bool WIDE>
 __global__ void __launch_bounds__(NTHR, 1)
 k_tc32_chain_m64(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   constexpr bool SPLIT = NPROD == 3;
@@ -225,12 +231,21 @@ k_tc32_chain_m64(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   }
   const Chain& ch = *chp;
   const int nl = ch.n_layers;
+  const int ns = WIDE ? (ch.kin + KMAX - 1) / KMAX : 1;     // K slices of the first layer (>= 2 when WIDE)
 
   auto load_weights = [&](int l) {
     const unsigned bytes = (unsigned)ch.layer[l].K * TN * 2;          // one part (hi or lo)
     mbar_expect_tx(&sm.wbar[l & 1], (SPLIT ? 2 : 1) * bytes);
     bulk_g2s(sm.w[l & 1][0], ch.layer[l].w, bytes, &sm.wbar[l & 1]);
     if (SPLIT) bulk_g2s(sm.w[l & 1][1], ch.layer[l].w + (size_t)ch.layer[l].K * TN, bytes, &sm.wbar[l & 1]);
+  };
+  auto load_tile = [&](int t) {                                      // WIDE: ring tile t into slot t & 1
+    const int l = t < ns ? 0 : t - ns + 1;
+    const int K = ch.layer[l].K, k0 = t < ns ? t * KMAX : 0;
+    const unsigned bytes = (unsigned)(t < ns ? min(KMAX, K - k0) : K) * TN * 2;
+    mbar_expect_tx(&sm.wbar[t & 1], (SPLIT ? 2 : 1) * bytes);
+    bulk_g2s(sm.w[t & 1][0], ch.layer[l].w + (size_t)k0 * TN, bytes, &sm.wbar[t & 1]);
+    if (SPLIT) bulk_g2s(sm.w[t & 1][1], ch.layer[l].w + (size_t)(K + k0) * TN, bytes, &sm.wbar[t & 1]);
   };
   if (tid == 0) {
     mbar_init(&sm.wbar[0], 1); mbar_init(&sm.wbar[1], 1);
@@ -240,8 +255,15 @@ k_tc32_chain_m64(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
     const unsigned bbytes = (unsigned)nl * TN * 4;
     mbar_expect_tx(&sm.bbar, bbytes);
     bulk_g2s(sm.bias, ch.bias, bbytes, &sm.bbar);
-    load_weights(0);
-    if (nl > 1) load_weights(1);
+    if (WIDE) {
+      mbar_init(&sm.sbar, 1);
+      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+      load_tile(0);
+      load_tile(1);
+    } else {
+      load_weights(0);
+      if (nl > 1) load_weights(1);
+    }
   }
   __syncwarp();
   if (warp == 0) {
@@ -333,11 +355,37 @@ k_tc32_chain_m64(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
   if (is_issuer_warp) {
     // =========================== issuer warp: weight ring + 3 x tcgen05.mma per K-step ==========================
     const unsigned long long ad = umma_desc(s32(sm.a[0]), CH, 128);
+    if (WIDE) {
+      for (int s = 0; s + 1 < ns; ++s) {      // every K slice of the first layer but the last
+        mbar_wait(&sm.wbar[s & 1], (s >> 1) & 1);
+        const unsigned long long bd_hi = umma_desc(s32(sm.w[s & 1][0]), CHUNK_W, 128);
+        const unsigned long long bd_lo = umma_desc(s32(sm.w[s & 1][1]), CHUNK_W, 128);
+        nb_sync(2);                         // slice s is in shared memory (the epilogue arrives on both round barriers)
+        nb_sync(3);
+        tc_fence_after();
+        if (elect_one()) {
+#pragma unroll
+          for (int k = 0; k < KMAX / 16; ++k) {
+            const unsigned long long oa = (unsigned long long)(k * ((2 * CH) >> 4));
+            const unsigned long long ow = (unsigned long long)(k * ((2 * CHUNK_W) >> 4));
+            umma<SPLIT>(tmem, ad + oa, bd_hi + ow, (s > 0 || k > 0) ? 1u : 0u);
+            if (SPLIT) umma<SPLIT>(tmem, ad + oa, bd_lo + ow, 1u);
+          }
+        }
+        __syncwarp();
+        if (lane == 0) umma_commit(&sm.sbar);
+        __syncwarp();
+        mbar_wait(&sm.sbar, s & 1);         // slot s & 1 and the A operand are free again
+        if (lane == 0) load_tile(s + 2);    // s + 2 <= ns: the last slice or layer 1
+        __syncwarp();
+      }
+    }
     for (int l = 0; l < nl; ++l) {
-      const int nk = ch.layer[l].K / 16;
-      mbar_wait(&sm.wbar[l & 1], (l >> 1) & 1);
-      const unsigned long long bd_hi = umma_desc(s32(sm.w[l & 1][0]), CHUNK_W, 128);
-      const unsigned long long bd_lo = umma_desc(s32(sm.w[l & 1][1]), CHUNK_W, 128);
+      const int t = WIDE ? l + ns - 1 : l;  // ring tile of layer l
+      const int nk = (WIDE && l == 0) ? (ch.kin - (ns - 1) * KMAX) / 16 : ch.layer[l].K / 16;
+      mbar_wait(&sm.wbar[t & 1], (t >> 1) & 1);
+      const unsigned long long bd_hi = umma_desc(s32(sm.w[t & 1][0]), CHUNK_W, 128);
+      const unsigned long long bd_lo = umma_desc(s32(sm.w[t & 1][1]), CHUNK_W, 128);
       const unsigned d = tmem + (unsigned)((l & 1) * TN);
       for (int c = 0; c < 2; ++c) {
         nb_sync(2 + c);                     // the A columns of round c are in shared memory
@@ -348,7 +396,7 @@ k_tc32_chain_m64(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
             if (k >= (c ? R0 / 16 : 0) && k < (c ? KA / 16 : R0 / 16) && k < nk) {
               const unsigned long long oa = (unsigned long long)(k * ((2 * CH) >> 4));
               const unsigned long long ow = (unsigned long long)(k * ((2 * CHUNK_W) >> 4));
-              umma<SPLIT>(d, ad + oa, bd_hi + ow, k > 0 ? 1u : 0u);
+              umma<SPLIT>(d, ad + oa, bd_hi + ow, (k > 0 || (WIDE && l == 0)) ? 1u : 0u);
               if (SPLIT) umma<SPLIT>(d, ad + oa, bd_lo + ow, 1u);
             }
         }
@@ -358,7 +406,9 @@ k_tc32_chain_m64(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
       __syncwarp();
       if (l + 2 < nl) {                     // ring slot l&1 is reusable once these MMAs have completed
         mbar_wait(&sm.dbar[l & 1], (l >> 1) & 1);
-        if (lane == 0) load_weights(l + 2);
+        if (lane == 0) {
+          if (WIDE) load_tile(t + 2); else load_weights(l + 2);
+        }
         __syncwarp();
       }
     }
@@ -394,6 +444,41 @@ k_tc32_chain_m64(SmzArena a, Chain chain0, Chain chain1, Job job, int sim) {
     }
     fence_async_smem();
     for (int c = 0; c < 2; ++c) nb_arrive(2 + c);
+    if (WIDE) {
+      // the remaining K slices of the observation: the next slice's loads are in flight while the MMAs of the last run
+      const int row = tile * TM + srow;
+      const bool valid = row < count;
+      const uint4 z = make_uint4(0, 0, 0, 0);
+      unsigned char* const ph = sm.a[0] + (SPLIT ? 32 * (srow >> 4) + (srow & 15) : srow) * 16;
+      unsigned char* const pl = ph + 16 * 16;
+      for (int s = 1; s < ns; ++s) {
+        const int k0 = s * KMAX, kw = min(KMAX, ch.kin - k0);
+#pragma unroll
+        for (int half = 0; half < 2; ++half) {
+          const int kc = skc + 8 * half;
+          float v[8];
+#pragma unroll
+          for (int j = 0; j < 8; ++j) {
+            const int c = k0 + kc * 8 + j;
+            v[j] = (valid && c < job.obs) ? job.in[(size_t)row * job.obs + c] : 0.f;
+          }
+          if (half) split8(v, h1, l1); else split8(v, h0, l0);
+        }
+        mbar_wait(&sm.sbar, (s - 1) & 1);
+        __syncwarp();
+        tc_fence_after();
+        if (skc * 8 < kw) {
+          sts16(ph + skc * CH, valid ? h0 : z);
+          if (SPLIT) sts16(pl + skc * CH, valid ? l0 : z);
+        }
+        if ((skc + 8) * 8 < kw) {
+          sts16(ph + (skc + 8) * CH, valid ? h1 : z);
+          if (SPLIT) sts16(pl + (skc + 8) * CH, valid ? l1 : z);
+        }
+        fence_async_smem();
+        for (int c = 0; c < 2; ++c) nb_arrive(2 + c);
+      }
+    }
     mbar_wait(&sm.bbar, 0);
     epi_sync();                              // rowidx is read by other threads from here on
     const unsigned lane_t = tmem + ((unsigned)(q * 32) << 16);
@@ -808,9 +893,10 @@ int smz_tc32_create(const SmzNetShape& sh, int nprod, SmzTc32Image** out, char* 
   im->smem_bytes = (int)sizeof(SmemT<KMAX>) + 1024;
   im->nprod = nprod == 1 ? 1 : 3;
   im->exact_elu = (im->nprod == 3 && getenv("SMZ_TC32_POLY")) ? atoi(getenv("SMZ_TC32_POLY")) : 0;
-  cudaFuncSetAttribute((const void*)k_tc32_chain_m64<3, false, false, KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, im->smem_bytes);
-  cudaFuncSetAttribute((const void*)k_tc32_chain_m64<3, true, false, KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, im->smem_bytes);
-  cudaFuncSetAttribute((const void*)k_tc32_chain_m64<1, false, false, KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, im->smem_bytes);
+  for (const void* f : {(const void*)k_tc32_chain_m64<3, false, false, KMAX, false>, (const void*)k_tc32_chain_m64<3, true, false, KMAX, false>,
+                        (const void*)k_tc32_chain_m64<1, false, false, KMAX, false>, (const void*)k_tc32_chain_m64<3, false, false, KMAX, true>,
+                        (const void*)k_tc32_chain_m64<3, true, false, KMAX, true>, (const void*)k_tc32_chain_m64<1, false, false, KMAX, true>})
+    cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, im->smem_bytes);
   *out = im;
   return SMZ_OK;
 }
@@ -929,8 +1015,12 @@ void smz_tc32_read_hidden(const SmzArena& a, int slot, int n_trees, float* out, 
 static void launch(SmzTc32Image* im, dim3 grid, cudaStream_t s, bool pdl, const SmzArena& a, const Chain& c0, const Chain& c1,
                    Job job, int sim) {
   job.exact_elu = im->exact_elu;
-  auto* k = im->nprod == 1 ? k_tc32_chain_m64<1, false, false, KMAX>
-                           : (im->exact_elu ? k_tc32_chain_m64<3, true, false, KMAX> : k_tc32_chain_m64<3, false, false, KMAX>);
+  // observations wider than one K tile: the instantiation that streams the first layer's K in slices
+  const bool wide = job.input_kind == IN_OBS && c0.kin > KMAX;
+  auto* k = wide ? (im->nprod == 1 ? k_tc32_chain_m64<1, false, false, KMAX, true>
+                                   : (im->exact_elu ? k_tc32_chain_m64<3, true, false, KMAX, true> : k_tc32_chain_m64<3, false, false, KMAX, true>))
+                 : (im->nprod == 1 ? k_tc32_chain_m64<1, false, false, KMAX, false>
+                                   : (im->exact_elu ? k_tc32_chain_m64<3, true, false, KMAX, false> : k_tc32_chain_m64<3, false, false, KMAX, false>));
   smz_launch(k, grid, dim3(NTHR), (size_t)im->smem_bytes, s, pdl, a, c0, c1, job, sim);
 }
 
@@ -1004,7 +1094,7 @@ int smz_tc32_vision_create(int A, int S, int H, int L, SmzTc32VisionHeads** out,
   }
   im->bias_pool = (float*)p;
   im->smem_bytes = (int)sizeof(SmemT<KVIS>) + 1024;
-  if (cudaFuncSetAttribute((const void*)k_tc32_chain_m64<3, false, true, KVIS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+  if (cudaFuncSetAttribute((const void*)k_tc32_chain_m64<3, false, true, KVIS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                            im->smem_bytes) != cudaSuccess) {
     snprintf(err, err_len, "vision heads on tcgen05: %d bytes of shared memory per CTA are not available", im->smem_bytes);
     smz_tc32_vision_destroy(im);
@@ -1087,6 +1177,6 @@ void smz_tc32_vision_heads(SmzTc32VisionHeads* im, const SmzArena& a, int n_tree
   job.feat = feat; job.vchains = im->chains_dev;
   job.policy_dst = a.out_policy; job.value_dst = a.out_value; job.reward_dst = a.out_reward; job.pstride = a.W;
   Chain none{};
-  smz_launch(k_tc32_chain_m64<3, false, true, KVIS>, dim3(5 * ((n_trees + TM - 1) / TM)), dim3(NTHR), (size_t)im->smem_bytes, s, pdl,
+  smz_launch(k_tc32_chain_m64<3, false, true, KVIS, false>, dim3(5 * ((n_trees + TM - 1) / TM)), dim3(NTHR), (size_t)im->smem_bytes, s, pdl,
              a, none, none, job, sim);
 }
