@@ -147,6 +147,22 @@ int smz_set_weights(smz_engine* e, const float* blob, uint64_t n_floats, int32_t
  * fresh draws).  Stream-ordered; does not invalidate the captured simulation graph. */
 int smz_set_seed(smz_engine* e, uint64_t seed, uint64_t tree_id_offset, void* stream);
 
+/* Which nodes of the tree are chance nodes.  The kind of a node at depth d is (d >> 1) & 1 (1 = chance) under
+ * SMZ_PATTERN_REFERENCE, the reference's F,F,T,T,F,F,... (monte_carlo_tree_search.py:211, :333-345), and d & 1 under
+ * SMZ_PATTERN_PAPER, the Stochastic MuZero alternation F,T,F,T,...: the root's children are afterstates, so
+ * afterstate_dynamics is applied to states and dynamics to afterstates, pUCT runs over actions and sampling over
+ * chance codes.  In both patterns a leaf whose parent is a decision node is evaluated by the afterstate pair and gets
+ * min(K, C) children, any other by the dynamics pair (min(K, A) children and a reward); a chance child keeps its
+ * parent's to_play, a decision child gets the next player.  Any other value returns SMZ_E_INVALID_ARG.
+ * The setting applies from the next smz_root, which copies it into the arena; a search already rooted keeps its
+ * pattern.  Default: SMZ_PATTERN_REFERENCE.  A caller that supplies its own smz_set_player_tables must build the
+ * to_play / sign tables with the same pattern (the per-depth player step follows the node kinds). */
+enum {
+  SMZ_PATTERN_REFERENCE = 0,
+  SMZ_PATTERN_PAPER = 1
+};
+int smz_set_node_pattern(smz_engine* e, int32_t pattern);
+
 /* Tape inputs (rng_mode == SMZ_RNG_TAPE): uniforms_dev is double[n_trees][stride]. */
 int smz_set_uniform_tape(smz_engine* e, const double* uniforms_dev, int32_t stride);
 

@@ -10,6 +10,7 @@ SMZ_ABI_VERSION = 2
 SMZ_OK, SMZ_E_INVALID_ARG, SMZ_E_CUDA, SMZ_E_CAPACITY, SMZ_E_STATE = 0, -1, -2, -3, -4
 NET_EXTERNAL, NET_FP32, NET_BF16, NET_VISION, NET_TC32, NET_F16 = 0, 1, 2, 3, 4, 5
 RNG_PHILOX, RNG_TAPE = 0, 1
+PATTERN_REFERENCE, PATTERN_PAPER = 0, 1
 
 
 class smz_config(C.Structure):
@@ -56,6 +57,7 @@ SIGNATURES = {
     "smz_set_weights": (C.c_int, [_P, _P, C.c_uint64, C.c_int32, _P]),
     "smz_set_seed": (C.c_int, [_P, C.c_uint64, C.c_uint64, _P]),
     "smz_set_uniform_tape": (C.c_int, [_P, _P, C.c_int32]),
+    "smz_set_node_pattern": (C.c_int, [_P, C.c_int32]),
     "smz_root": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
     "smz_simulate": (C.c_int, [_P, C.c_int32, _P]),
     "smz_select": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P]),

@@ -74,6 +74,7 @@ struct smz_engine {
   int graph_trees, graph_sims, graph_first, graph_launches;
   cudaStream_t capture_stream;
   int use_pdl;
+  int32_t node_pattern;  // SMZ_PATTERN_*, copied into the arena (a.kind_shift) by the next smz_root
 };
 
 const char* smz_last_error(void) { return g_err; }
@@ -165,6 +166,8 @@ int smz_create(const smz_config* cfg, smz_engine** out) {
   a.Sp = c.net_mode == SMZ_NET_VISION ? SMZ_VISION_SP : SMZ_SP;
   a.path_stride = a.N + 2;
   a.n_phases = 1;
+  a.kind_shift = 1;
+  e->node_pattern = SMZ_PATTERN_REFERENCE;
   a.rng_mode = c.rng_mode;
   a.discount = (float)c.discount;
   a.one_minus_frac_f32 = (float)(1.0 - c.root_exploration_fraction);
@@ -366,6 +369,15 @@ int smz_set_uniform_tape(smz_engine* e, const double* u, int32_t stride) {
   return SMZ_OK;
 }
 
+int smz_set_node_pattern(smz_engine* e, int32_t pattern) {
+  if (!e) return fail(SMZ_E_INVALID_ARG, "smz_set_node_pattern: null engine");
+  if (pattern != SMZ_PATTERN_REFERENCE && pattern != SMZ_PATTERN_PAPER)
+    return fail(SMZ_E_INVALID_ARG, "smz_set_node_pattern: pattern %d is neither SMZ_PATTERN_REFERENCE (0) nor SMZ_PATTERN_PAPER (1)",
+                pattern);
+  e->node_pattern = pattern;
+  return SMZ_OK;
+}
+
 int smz_root(smz_engine* e, int32_t n_trees, const float* obs, const float* root_policy, const int32_t* root_to_play,
              int32_t train, const double* dirichlet, void* stream) {
   if (!e) return fail(SMZ_E_INVALID_ARG, "smz_root: null engine");
@@ -378,6 +390,11 @@ int smz_root(smz_engine* e, int32_t n_trees, const float* obs, const float* root
   cudaStream_t s = (cudaStream_t)stream;
   ON_DEVICE(e);
   SmzArena& a = e->a;
+  const int kind_shift = e->node_pattern == SMZ_PATTERN_PAPER ? 0 : 1;
+  if (a.kind_shift != kind_shift) {   // the captured simulation graph holds the arena by value
+    a.kind_shift = kind_shift;
+    drop_graph(e);
+  }
   smz_launch_begin_search(a, s);       // row counters, error flag, depth statistic
   if (a.dbg) {      // wall-clock stamps: "first" slots start at all-ones (atomicMin), "last" slots at zero (atomicMax)
     std::vector<unsigned long long> init(4 * ((size_t)a.N + 2));

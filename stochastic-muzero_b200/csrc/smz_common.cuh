@@ -24,6 +24,7 @@ struct SmzArena {
   // shape
   int B, N, A, C, K, Kd, Kc, Kmax, M, W, Sp, path_stride, n_phases;
   int row_cap, row_top;   // compacted-row arrays: row_cap positions per parity; the current search uses [0, row_top)
+  int kind_shift;         // node kind at depth d = (d >> kind_shift) & 1 (1 = chance): 1 = reference F,F,T,T,...  0 = paper F,T,F,T,...
   // tree columns
   int4* stat;
   int2* link;

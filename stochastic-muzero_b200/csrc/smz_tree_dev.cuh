@@ -247,7 +247,7 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
   int level = 0;
   while (__any_sync(FULL, going)) {
     const bool act = going && g.gl < nch;
-    const bool chance = (level >> 1) & 1;
+    const bool chance = (level >> a.kind_shift) & 1;
     const int ci = act ? cbase + g.gl : 0;                     // idle lanes read node 0 and discard it
     int4 st;
     int2 lk;
@@ -342,7 +342,7 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
   //      depth statistic per warp, instead of one atomic per tree — thousands of same-address atomics per
   //      simulation serialise in the L2 and their return value is on the critical path of the kernel.
   const bool lead = alive && g.gl == 0;
-  const int branch = ((depth >> 1) & 1) ? SMZ_BRANCH_DYNAMICS : SMZ_BRANCH_AFTERSTATE;
+  const int branch = ((depth >> a.kind_shift) & 1) ? SMZ_BRANCH_DYNAMICS : SMZ_BRANCH_AFTERSTATE;   // the leaf's parent's kind
   const int slot = (cbase == 1) ? 0 : (cbase - 1 - a.A) / a.Kmax + 1;
   // the parent's hidden row is requested now and stored once the row index is known (bf16 network: a.xin)
   uint4 hcopy[(G < 8) ? 8 / G : 1], hcopy2[(G < 8) ? 8 / G : 1];

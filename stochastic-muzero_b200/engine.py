@@ -25,14 +25,16 @@ class SmzError(RuntimeError):
     pass
 
 
-def _is_chance(depth: int) -> bool:
-    """Depth pattern of the reference: F,F,T,T,F,F,... (monte_carlo_tree_search.py:211, :333-345)."""
-    return bool((depth >> 1) & 1)
+def _is_chance(depth: int, paper_alternation: bool = False) -> bool:
+    """Node kind by depth: the reference's F,F,T,T,F,F,... (monte_carlo_tree_search.py:211, :333-345), or with
+    ``paper_alternation`` the Stochastic MuZero alternation F,T,F,T,... (smz_set_node_pattern in include/smz.h)."""
+    return bool((depth >> (0 if paper_alternation else 1)) & 1)
 
 
-def player_tables(number_of_player: int, custom_loop: Optional[str], n_depth: int):
+def player_tables(number_of_player: int, custom_loop: Optional[str], n_depth: int, paper_alternation: bool = False):
     """Player_cycle (monte_carlo_tree_search.py:38-72) flattened per (root_to_play phase, depth):
-    to_play of a node and the sign its backed-up value gets (:302-305)."""
+    to_play of a node and the sign its backed-up value gets (:302-305).  A chance node keeps its parent's
+    to_play, a decision node gets the next player, so the tables follow the node pattern."""
     if custom_loop is not None:
         cycle = [float(i) for i in custom_loop.split(">")]
     else:
@@ -44,7 +46,7 @@ def player_tables(number_of_player: int, custom_loop: Optional[str], n_depth: in
         tp = p
         for d in range(n_depth):
             if d >= 1:
-                tp = tp if _is_chance(d) else (tp + 1) % n      # :210, :296
+                tp = tp if _is_chance(d, paper_alternation) else (tp + 1) % n      # :210, :296
             to_play[p, d] = tp
             sign[p, d] = 1 if cycle[p % n] == cycle[tp % n] else -1
     return sign, to_play
@@ -61,7 +63,9 @@ class SearchEngine:
     def __init__(self, search: Dict, action_dim: int, chance_dim: Optional[int] = None, max_trees: int = 1,
                  model_shape: Optional[ModelShape] = None, net: str = "external", rng: str = "philox",
                  seed: int = 0, tree_id_offset: int = 0, device: Optional[int] = None, lanes_per_tree: int = 0,
-                 record: bool = False):
+                 record: bool = False, paper_alternation: bool = False):
+        """``paper_alternation``: search with the Stochastic MuZero node alternation instead of the reference's depth
+        pattern (smz_set_node_pattern in include/smz.h); ``set_node_pattern`` changes it for later searches."""
         if not torch.cuda.is_available():
             raise SmzError("SearchEngine needs a CUDA device; the search path has no CPU fallback")
         self.lib = _lib.load()
@@ -118,12 +122,28 @@ class SearchEngine:
         base, init = int(search["pb_c_base"]), float(search["pb_c_init"])
         pbc = np.array([np.sqrt(n) * (np.log((n + base + 1) / base) + init) for n in range(self.N + 2)], np.float64)
         self._check(self.lib.smz_set_pbc_table(self._h, pbc.ctypes.data_as(C.POINTER(C.c_double)), len(pbc)))
-        sign, to_play = player_tables(int(search.get("number_of_player", 1)), search.get("custom_loop"), self.N + 2)
+        self.paper_alternation = None         # pattern of the current search and of the uploaded player tables
+        self._next_paper = bool(paper_alternation)
+        self._apply_node_pattern()
+
+    def set_node_pattern(self, paper_alternation: bool):
+        """Node pattern of the searches started by the following root() calls; a search already rooted keeps its own."""
+        self._next_paper = bool(paper_alternation)
+
+    def _apply_node_pattern(self):
+        """Engine setting and player tables of the pending pattern, before a root step (the tables follow the pattern)."""
+        paper = self._next_paper
+        if paper == self.paper_alternation:
+            return
+        self._check(self.lib.smz_set_node_pattern(self._h, _lib.PATTERN_PAPER if paper else _lib.PATTERN_REFERENCE))
+        sign, to_play = player_tables(int(self.search.get("number_of_player", 1)), self.search.get("custom_loop"),
+                                      self.N + 2, paper)
         self.to_play_table = to_play
         self.n_phases = sign.shape[0]
         sign, to_play = np.ascontiguousarray(sign), np.ascontiguousarray(to_play)
         self._check(self.lib.smz_set_player_tables(self._h, sign.ctypes.data_as(C.POINTER(C.c_int8)),
                                                    to_play.ctypes.data_as(C.POINTER(C.c_int32)), self.n_phases))
+        self.paper_alternation = paper
 
     # ------------------------------------------------------------------------------------------
     def _check(self, rc):
@@ -198,6 +218,7 @@ class SearchEngine:
             pol_t = self._pad_policy(self._dev(root_policy, torch.float32, "root_policy"), "root_policy")
         rtp = self._dev(root_to_play, torch.int32, "root_to_play")
         dr = self._dev(dirichlet, torch.float64, "dirichlet")
+        self._apply_node_pattern()
         self._check(self.lib.smz_root(self._h, n, self._ptr(obs_t), self._ptr(pol_t), self._ptr(rtp), int(bool(train)),
                                       self._ptr(dr), self._stream))
         self.n_trees = n
@@ -354,10 +375,10 @@ class SearchEngine:
 
     def n_children(self, depth: int) -> int:
         """Children of an expanded node at `depth`: A at the root, else min(K, width of the head that
-        expanded it) — dynamics pair (width A) iff its parent is a chance node (T2)."""
+        expanded it) — dynamics pair (width A) iff its parent is a chance node (T2), in either node pattern."""
         if depth == 0:
             return self.A
-        return min(self.K, self.A) if _is_chance(depth - 1) else min(self.K, self.Cdim)
+        return min(self.K, self.A) if _is_chance(depth - 1, self.paper_alternation) else min(self.K, self.Cdim)
 
     def export_tree(self, tree: int) -> Dict[str, np.ndarray]:
         """Canonical dump: depth-first, children in ascending key order (same format as the oracle's
@@ -371,7 +392,8 @@ class SearchEngine:
             cb = int(ar["child_base"][n])
             prior = 0.0 if n == 0 else (ar["root_prior"][n - 1] if d == 1 else np.float64(ar["prior"][n]))
             rows.append((d, -1 if n == 0 else int(ar["key"][n]), int(ar["visit"][n]), ar["value_sum"][n],
-                         ar["reward"][n], prior, _is_chance(d), int(self.to_play_table[phase, d]), cb != 0, n))
+                         ar["reward"][n], prior, _is_chance(d, self.paper_alternation), int(self.to_play_table[phase, d]),
+                         cb != 0, n))
             if cb:
                 k = self.n_children(d)
                 stack.extend((cb + i, d + 1) for i in reversed(range(k)))

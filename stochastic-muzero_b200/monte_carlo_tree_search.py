@@ -23,7 +23,7 @@ import numpy as np
 import torch
 
 from . import batched_model
-from .engine import SearchEngine, _is_chance
+from .engine import SearchEngine
 from .weights import (PackedModel, VisionShape, pack_vision_weights, pack_weights, shape_of, weights_version)
 
 
@@ -128,13 +128,14 @@ def _node_tree(dump, hidden_fetch=None):
             node = Node(np.float64(prior) if d == 1 else np.float32(prior))
         node.visit_count = int(dump["visit"][i])
         node.value_sum = np.float32(dump["value_sum"][i]) if node.visit_count else 0
-        node.reward = np.float32(dump["reward"][i]) if d >= 1 and _is_chance(d - 1) and dump["expanded"][i] else 0
         node.to_play = int(dump["to_play"][i])
         node.is_chance = bool(dump["is_chance"][i])
         if dump["expanded"][i] and hidden_fetch is not None:
             node._hidden_fetch = (lambda n=int(dump["node"][i]): hidden_fetch(n))
         while stack and stack[-1][0] >= d:
             stack.pop()
+        # only a node evaluated by the dynamics pair, i.e. one whose parent is a chance node, carries a reward (:333-337)
+        node.reward = np.float32(dump["reward"][i]) if stack and stack[-1][1].is_chance and dump["expanded"][i] else 0
         if stack:
             stack[-1][1].children[np.int64(dump["key"][i])] = node
         stack.append((d, node))
@@ -238,7 +239,7 @@ class Monte_carlo_tree_search():
                  maxium_action_sample=2,
                  number_of_player=1,
                  custom_loop=None,
-                 *, net="tc32", device=None, seed=None, max_batch=None, tree_id_offset=None):
+                 *, net="tc32", device=None, seed=None, max_batch=None, tree_id_offset=None, paper_alternation=False):
         """Same nine arguments as the reference (:76-85).  Keyword-only extras: ``net`` — the fused MLP network step:
         "tc32" (default: the reference's fp32 precision on the tensor cores, fp16 hi/lo split operands, 1e-5 against the
         reference's inference), "fp32" (the same precision on CUDA cores), "bf16" / "f16" (throughput modes with
@@ -247,8 +248,11 @@ class Monte_carlo_tree_search():
         ``max_batch`` (arena capacity reserved for ``run_batch``), ``tree_id_offset`` (global id of local tree 0:
         the Philox streams are keyed by (seed, global tree id), so ranks of a sharded self-play that seed
         numpy identically still draw different noise; default rank * max_batch when torch.distributed is
-        initialised, else 0)."""
+        initialised, else 0), ``paper_alternation`` (search with the Stochastic MuZero node alternation — decision,
+        chance, decision, ... from the root, so afterstate_dynamics sees states and dynamics sees afterstates —
+        instead of the reference's depth pattern F,F,T,T,...; default off: the reference's search)."""
         self._net, self._device, self._seed, self._max_batch = net, device, seed, max_batch
+        self._paper = bool(paper_alternation)
         self._tree_id_offset = tree_id_offset
         self._engines = {}
         self._weights_seen = {}
@@ -317,7 +321,8 @@ class Monte_carlo_tree_search():
             if eng is not None:
                 eng.close()
             eng = SearchEngine(self.search_config(), action_dim, chance_dim, max_trees=cap, model_shape=shape,
-                               net=kind, rng="philox", seed=self._base_seed(), device=self._device)
+                               net=kind, rng="philox", seed=self._base_seed(), device=self._device,
+                               paper_alternation=self._paper)
             self._engines[key] = eng
             self._weights_seen.pop(key, None)
         return eng, key
