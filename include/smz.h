@@ -105,8 +105,9 @@ typedef struct smz_dims {
 } smz_dims;
 
 /* One tree copied out in arena order (host memory owned by the caller, nodes_per_tree entries each).
- * Node 0 is the root, nodes 1..A its children; a node expanded by simulation s owns the children
- * block starting at 1 + A + s*Kmax. */
+ * Node 0 is the root, nodes 1..A its children (node 1 + a = action a); a node expanded by simulation s owns the
+ * children block starting at 1 + A + s*Kmax.  A root child whose action was illegal (smz_root_legal) is a sentinel:
+ * key -1, prior 0, child_base 0, never visited. */
 typedef struct smz_tree_host {
   int32_t* visit;
   float* value_sum;
@@ -177,6 +178,20 @@ int smz_set_uniform_tape(smz_engine* e, const double* uniforms_dev, int32_t stri
 int smz_root(smz_engine* e, int32_t n_trees, const float* obs_dev, const float* root_policy_dev,
              const int32_t* root_to_play_dev, int32_t train, const double* dirichlet_dev, void* stream);
 
+/* smz_root with the root of each tree restricted to the legal actions of its position.  legal_dev: uint32[n_trees]
+ * (bit a set = action a is legal; A <= 32), or NULL for every action (then this is smz_root).  A tree's root behaves
+ * exactly as the reference's root would if its action space were L = the set bits in ascending order: the policy is
+ * compacted to policy[L] before normalisation and the draws of root expansion, children are created for L only,
+ * Dirichlet noise covers L only (device noise: Gamma draws for the legal actions in ascending order; given noise:
+ * the entries at L are used), and the root's pUCT consumes one draw per legal child.  Illegal actions keep their
+ * arena slot 1 + a with key -1 (see smz_export_tree), and read out as 0 visits, 0 reward and prior 0.0; smz_select_
+ * actions applies its rule to the legal children and never returns an illegal action.  A mask that is empty or has
+ * a bit >= A set raises error flag 3 (smz_read_roots) and that tree is searched with every action legal.  The mask
+ * is read by the kernels this call enqueues only: the captured smz_simulate graph stays valid. */
+int smz_root_legal(smz_engine* e, int32_t n_trees, const float* obs_dev, const float* root_policy_dev,
+                   const int32_t* root_to_play_dev, const uint32_t* legal_dev, int32_t train,
+                   const double* dirichlet_dev, void* stream);
+
 /* n_sims full simulations (:325-347) with the internal network (net_mode FP32/BF16). */
 int smz_simulate(smz_engine* e, int32_t n_sims, void* stream);
 
@@ -214,7 +229,7 @@ int smz_net_eval(smz_engine* e, int32_t which, int32_t n_rows, const float* in_d
  * visits int32[n][A], root_values float[n] (= Node.value() of the root), priors double[n][A],
  * rewards float[n][A]; error_dev int32[1] = the search's error flag (0 ok, 1 uniform tape exhausted,
  * 2 NaN / all-zero policy met during an expansion — where np.random.choice raises in the reference,
- * monte_carlo_tree_search.py:208/:294), delivered with the same read-out so that the host needs no extra
+ * monte_carlo_tree_search.py:208/:294, 3 a legal-action mask of smz_root_legal was empty or had a bit >= A set), delivered with the same read-out so that the host needs no extra
  * synchronisation to learn about it.  Any pointer may be NULL. */
 int smz_read_roots(smz_engine* e, int32_t* visits_dev, float* root_values_dev, double* priors_dev,
                    float* rewards_dev, int32_t* error_dev, void* stream);
@@ -237,7 +252,8 @@ int smz_read_record(smz_engine* e, float* policy_dev, float* value_dev, float* r
                     int8_t* branch_dev, double* dirichlet_dev, float* root_policy_dev, void* stream);
 /* Synchronises `stream`.  Mean leaf depth and kernel-launch count of the last smz_root + smz_simulate, and the
  * number of kernels this engine has launched since smz_create (bench bookkeeping: `gpu_launches`).  Returns
- * SMZ_E_CAPACITY / SMZ_E_STATE when the last search raised its error flag (see smz_read_roots). */
+ * SMZ_E_CAPACITY / SMZ_E_STATE / SMZ_E_INVALID_ARG when the last search raised its error flag 1 / 2 / 3 (see
+ * smz_read_roots). */
 int smz_stats(smz_engine* e, double* mean_leaf_depth, int64_t* launches, int64_t* launches_total, void* stream);
 
 #ifdef __cplusplus

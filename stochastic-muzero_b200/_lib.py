@@ -59,6 +59,7 @@ SIGNATURES = {
     "smz_set_uniform_tape": (C.c_int, [_P, _P, C.c_int32]),
     "smz_set_node_pattern": (C.c_int, [_P, C.c_int32]),
     "smz_root": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
+    "smz_root_legal": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "smz_simulate": (C.c_int, [_P, C.c_int32, _P]),
     "smz_select": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P]),
     "smz_net_step": (C.c_int, [_P, C.c_int32, _P]),

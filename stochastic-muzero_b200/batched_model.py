@@ -84,16 +84,18 @@ def is_batched_backend(model) -> bool:
     return all(callable(getattr(model, n, None)) for n in BATCHED_METHODS)
 
 
-def run_search(engine, backend, observations, n_sims, root_to_play=None, train=True):
+def run_search(engine, backend, observations, n_sims, root_to_play=None, train=True, legal=None):
     """Drive one batched search with an external batched network: the engine's select / expand_backup
-    hooks around torch calls.  Returns the hidden-state store [N+1, B, ...] (slot-major like the arena's)."""
+    hooks around torch calls.  ``legal``: optional legal-action mask [B, A] of the roots (SearchEngine.root).
+    Returns the hidden-state store [N+1, B, ...] (slot-major like the arena's)."""
     dev = torch.device("cuda", engine.device)
     h0 = backend.representation(observations)
     B = h0.shape[0]
     policy, _value = backend.prediction(h0)
     store = torch.zeros((n_sims + 1,) + tuple(h0.shape), dtype=h0.dtype, device=dev)
     store[0] = h0
-    engine.root(root_policy=policy.float(), root_to_play=root_to_play, train=train)
+    engine.root(root_policy=policy.float(), root_to_play=root_to_play, train=train,
+                **({} if legal is None else {"legal": legal}))
     W = engine.dims.policy_stride
     rows = torch.arange(B, device=dev)
     for sim in range(n_sims):

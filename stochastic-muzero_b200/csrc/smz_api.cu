@@ -380,6 +380,12 @@ int smz_set_node_pattern(smz_engine* e, int32_t pattern) {
 
 int smz_root(smz_engine* e, int32_t n_trees, const float* obs, const float* root_policy, const int32_t* root_to_play,
              int32_t train, const double* dirichlet, void* stream) {
+  return smz_root_legal(e, n_trees, obs, root_policy, root_to_play, nullptr, train, dirichlet, stream);
+}
+
+int smz_root_legal(smz_engine* e, int32_t n_trees, const float* obs, const float* root_policy,
+                   const int32_t* root_to_play, const uint32_t* legal, int32_t train, const double* dirichlet,
+                   void* stream) {
   if (!e) return fail(SMZ_E_INVALID_ARG, "smz_root: null engine");
   if (n_trees < 1 || n_trees > e->a.B) return fail(SMZ_E_CAPACITY, "smz_root: n_trees %d not in [1, %d]", n_trees, e->a.B);
   if ((obs == nullptr) == (root_policy == nullptr))
@@ -417,11 +423,11 @@ int smz_root(smz_engine* e, int32_t n_trees, const float* obs, const float* root
     if (dirichlet) {
       CU(cudaMemcpyAsync(a.dirichlet, dirichlet, (size_t)n_trees * a.A * sizeof(double), cudaMemcpyDeviceToDevice, s));
     } else {
-      smz_launch_dirichlet(a, n_trees, s);
+      smz_launch_dirichlet(a, n_trees, legal, s);
       count_launches(e, 1);
     }
   }
-  smz_launch_root_expand(a, e->cfg.lanes_per_tree, n_trees, policy, a.W, root_to_play, train, a.dirichlet, s);
+  smz_launch_root_expand(a, e->cfg.lanes_per_tree, n_trees, policy, a.W, root_to_play, train, a.dirichlet, legal, s);
   count_launches(e, 1);
   CU(cudaGetLastError());
   e->n_trees = n_trees;
@@ -683,5 +689,8 @@ int smz_stats(smz_engine* e, double* mean_leaf_depth, int64_t* launches, int64_t
   if (launches_total) *launches_total = e->launches_total;
   if (err == 1) return fail(SMZ_E_CAPACITY, "uniform tape exhausted during the search");
   if (err == 2) return fail(SMZ_E_STATE, "degenerate (NaN / all-zero) policy met during expansion");
+  if (err == 3)
+    return fail(SMZ_E_INVALID_ARG, "a legal-action mask was empty or named an action >= action_dim; that tree was "
+                "searched with every action legal");
   return SMZ_OK;
 }

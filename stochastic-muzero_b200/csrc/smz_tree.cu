@@ -21,34 +21,57 @@ namespace {
 using namespace smz_tree_dev;
 
 // ------------------------------------------------------------------------------------------------
+// Legal set of a tree's root: bit a = action a may be played.  No mask means every action.  A mask that is empty or
+// names an action >= A is `bad`: the tree is then searched with every action legal (k_root_expand raises flag 3).
+__device__ __forceinline__ unsigned root_legal_set(const uint32_t* __restrict__ legal, int tree, int A, bool& bad) {
+  const unsigned all = A >= 32 ? 0xffffffffu : (1u << A) - 1u;
+  const unsigned m = legal ? legal[tree] : all;
+  bad = m == 0u || (m & ~all) != 0u;
+  return bad ? all : m;
+}
+
 template <int G>
 __global__ void k_root_expand(SmzArena a, int n_trees, const float* __restrict__ policy, int pstride,
                               const int* __restrict__ root_to_play, int train,
-                              const double* __restrict__ dirichlet) {
+                              const double* __restrict__ dirichlet, const uint32_t* __restrict__ legal) {
   Group<G> g;
   int tree = (blockIdx.x * blockDim.x + threadIdx.x) / G;
   const bool alive = tree < n_trees;
   if (!alive) tree = n_trees - 1;
   const size_t tb = (size_t)tree * a.M;
-  const int n = a.A;
+  bool bad;
+  const unsigned lm = root_legal_set(legal, tree, a.A, bad);
+  // the root's action space is the legal set L: lane i works on its i-th action, so the policy is compacted before
+  // it is normalised and drawn from (with every action legal, lane i is action i)
+  const int n = __popc(lm);
+  const int act = g.gl < n ? (int)__fns(lm, 0, g.gl + 1) : 0;
   int cursor = 0;
-  const float pol = (g.gl < n) ? policy[(size_t)tree * pstride + g.gl] : 0.f;
+  const float pol = (g.gl < n) ? policy[(size_t)tree * pstride + act] : 0.f;
   const float p = normalise_policy(g, pol, n);
-  // all A actions become children (ascending); the call still consumes its draws (T5)
+  // all legal actions become children (ascending); the call still consumes its draws (T5)
   const SmzRng rng = smz_make_rng(a);
   choice_without_replacement(g, a, rng, alive, tree, p, n, n, cursor);
   if (!alive) return;
   if (g.gl < n) {
     double prior = (double)p;
     if (train) {
-      const double nz = dirichlet[(size_t)tree * a.A + g.gl];
+      const double nz = dirichlet[(size_t)tree * a.A + act];
       prior = __dadd_rn((double)__fmul_rn(p, a.one_minus_frac_f32), __dmul_rn(nz, a.frac));
     }
-    a.root_prior[(size_t)tree * a.A + g.gl] = prior;
-    a.stat[tb + 1 + g.gl] = make_int4(0, 0, 0, __float_as_int(p));
-    a.link[tb + 1 + g.gl] = make_int2(0, g.gl);
+    a.root_prior[(size_t)tree * a.A + act] = prior;
+    a.stat[tb + 1 + act] = make_int4(0, 0, 0, __float_as_int(p));
+    a.link[tb + 1 + act] = make_int2(0, act);
+  }
+  // root-child slots stay indexed by action: the slot of an illegal action holds the sentinel key -1, prior 0, and
+  // is never expanded; its recorded noise reads 0
+  if (g.gl < a.A && !((lm >> g.gl) & 1u)) {
+    a.root_prior[(size_t)tree * a.A + g.gl] = 0.0;
+    a.stat[tb + 1 + g.gl] = make_int4(0, 0, 0, 0);
+    a.link[tb + 1 + g.gl] = make_int2(0, -1);
+    if (train) a.dirichlet[(size_t)tree * a.A + g.gl] = 0.0;
   }
   if (g.gl == 0) {
+    if (bad) *a.error_flag = 3;
     a.stat[tb] = make_int4(0, 0, 0, 0);
     a.link[tb] = make_int2(1, -1);
     a.minmax[tree] = make_float2(__int_as_float(0x7f800000), __int_as_float(0xff800000));
@@ -58,7 +81,7 @@ __global__ void k_root_expand(SmzArena a, int n_trees, const float* __restrict__
     a.root_to_play[tree] = rtp < 0 ? rtp + a.n_phases : rtp;
     a.path_len[tree] = 0;
     if (a.rec_root_policy)
-      for (int i = 0; i < a.W; ++i) a.rec_root_policy[(size_t)tree * a.W + i] = i < n ? policy[(size_t)tree * pstride + i] : 0.f;
+      for (int i = 0; i < a.W; ++i) a.rec_root_policy[(size_t)tree * a.W + i] = i < a.A ? policy[(size_t)tree * pstride + i] : 0.f;
   }
 }
 
@@ -226,16 +249,27 @@ __global__ void k_select_actions(SmzArena a, int n_trees, double temperature, co
   const int tree = blockIdx.x * blockDim.x + threadIdx.x;
   if (tree >= n_trees) return;
   const size_t tb = (size_t)tree * a.M;
-  const int n = a.A;
+  const int A = a.A;
+  // the reference's rule over the legal children only (key -1 marks an illegal action's slot): compacted vectors,
+  // results scattered back with 0 for illegal actions
   double v[SMZ_MAX_POLICY], pr[SMZ_MAX_POLICY], p[SMZ_MAX_POLICY];
-  for (int i = 0; i < n; ++i) {
-    v[i] = (double)a.stat[tb + 1 + i].x;
-    pr[i] = a.root_prior[(size_t)tree * n + i];
+  int act[SMZ_MAX_POLICY];
+  int n = 0;
+  for (int i = 0; i < A; ++i) {
+    if (a.link[tb + 1 + i].y < 0) {
+      if (stored_out) stored_out[(size_t)tree * A + i] = 0.0;
+      if (policy_out) policy_out[(size_t)tree * A + i] = 0.0;
+      continue;
+    }
+    act[n] = i;
+    v[n] = (double)a.stat[tb + 1 + i].x;
+    pr[n] = a.root_prior[(size_t)tree * A + i];
+    ++n;
   }
   const double sv = np_sum_f64(v, n);
   if (stored_out) {
     const double sp = np_sum_f64(pr, n);
-    for (int i = 0; i < n; ++i) stored_out[(size_t)tree * n + i] = sv >= 3.0 ? __ddiv_rn(v[i], sv) : __ddiv_rn(pr[i], sp);
+    for (int i = 0; i < n; ++i) stored_out[(size_t)tree * A + act[i]] = sv >= 3.0 ? __ddiv_rn(v[i], sv) : __ddiv_rn(pr[i], sp);
   }
   const double e = 1.0 / temperature;
   for (int i = 0; i < n; ++i) {
@@ -248,7 +282,7 @@ __global__ void k_select_actions(SmzArena a, int n_trees, double temperature, co
   for (int i = 0; i < n; ++i) {
     p[i] = __ddiv_rn(p[i], s);
     flat = flat && p[i] == p[0];
-    if (policy_out) policy_out[(size_t)tree * n + i] = p[i];
+    if (policy_out) policy_out[(size_t)tree * A + act[i]] = p[i];
   }
   int pick = 0;
   if (temperature > 0.1 || flat) {
@@ -260,19 +294,26 @@ __global__ void k_select_actions(SmzArena a, int n_trees, double temperature, co
   } else {
     for (int i = 1; i < n; ++i) if (p[i] > p[pick]) pick = i;
   }
-  if (action_out) action_out[tree] = a.link[tb + 1 + pick].y;
+  if (action_out) action_out[tree] = act[pick];
 }
 
 // Dirichlet(alpha) per tree on the device: Gamma(alpha) by Marsaglia-Tsang (alpha+1 boost), Philox
 // stream 1.  Production mode only; parity runs pass recorded noise (np.random.dirichlet, mcts.py:220).
-__global__ void k_dirichlet(SmzArena a, int n_trees) {
+// Draws are taken for the legal actions of the root only, in ascending order; an illegal action's noise is 0.
+__global__ void k_dirichlet(SmzArena a, int n_trees, const uint32_t* __restrict__ legal) {
   const int tree = blockIdx.x * blockDim.x + threadIdx.x;
   if (tree >= n_trees) return;
+  bool bad;
+  const unsigned lm = root_legal_set(legal, tree, a.A, bad);
   unsigned ctr = 0;
   const unsigned long long seed = a.seed_state[0], tid = a.seed_state[1] + (unsigned long long)tree;
   auto U = [&]() { double u = smz_philox_uniform(seed, tid, ctr++, 1u); return u > 0.0 ? u : 1.0 / 9007199254740992.0; };
   double sum = 0.0;
   for (int i = 0; i < a.A; ++i) {
+    if (!((lm >> i) & 1u)) {
+      a.dirichlet[(size_t)tree * a.A + i] = 0.0;
+      continue;
+    }
     const double al = a.alpha;
     const double d = (al < 1.0 ? al + 1.0 : al) - 1.0 / 3.0, c = 1.0 / sqrt(9.0 * d);
     double gsample = d;
@@ -308,9 +349,10 @@ int grid_for(int n_trees, int threads) { return (int)(((long long)n_trees * G + 
 static const int kThreads = 128;
 
 void smz_launch_root_expand(const SmzArena& a, int lanes, int n_trees, const float* policy, int pstride,
-                            const int* root_to_play, int train, const double* dirichlet, cudaStream_t s) {
+                            const int* root_to_play, int train, const double* dirichlet, const uint32_t* legal,
+                            cudaStream_t s) {
   SMZ_DISPATCH_G(lanes, (k_root_expand<G><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(
-                            a, n_trees, policy, pstride, root_to_play, train, dirichlet)));
+                            a, n_trees, policy, pstride, root_to_play, train, dirichlet, legal)));
 }
 
 void smz_launch_select(const SmzArena& a, int lanes, int n_trees, int sim, int* o_slot, int* o_action, int* o_branch,
@@ -395,6 +437,6 @@ void smz_launch_set_seed(unsigned long long* dst, unsigned long long seed, unsig
   k_set_seed<<<1, 1, 0, s>>>(dst, seed, tree_id_offset);
 }
 
-void smz_launch_dirichlet(const SmzArena& a, int n_trees, cudaStream_t s) {
-  k_dirichlet<<<(n_trees + 127) / 128, 128, 0, s>>>(a, n_trees);
+void smz_launch_dirichlet(const SmzArena& a, int n_trees, const uint32_t* legal, cudaStream_t s) {
+  k_dirichlet<<<(n_trees + 127) / 128, 128, 0, s>>>(a, n_trees, legal);
 }

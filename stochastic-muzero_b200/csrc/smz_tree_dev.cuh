@@ -207,6 +207,18 @@ __device__ unsigned choice_without_replacement(const Group<G>& g, const SmzArena
 }
 
 
+// uniform #uidx of the tree for the lanes that `want` one; the draw only depends on the index, and a window of draws may
+// have been generated ahead (SmzRng::win)
+__device__ __forceinline__ double draw_uniform(const SmzRng& rng, int tree, int uidx, bool want) {
+  const unsigned wofs = (unsigned)(uidx - rng.win_base);
+  const bool hit = rng.win != nullptr && wofs < (unsigned)rng.win_len;
+  double u = hit ? rng.win[wofs] : 0.0;
+  if (__any_sync(FULL, want && !hit)) {
+    if (want && !hit) u = smz_rng_uniform(rng, tree, uidx);
+  }
+  return u;
+}
+
 // ------------------------------------------------------------------------------------------------
 // Per-tree state that flows from the backup of one simulation into the descent of the next.  The fused
 // kernel keeps it in registers; the stand-alone kernels load / store it.
@@ -246,7 +258,7 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
   // across the warp: plain uniform branches instead of votes, loads and draws without divergent regions.
   int level = 0;
   while (__any_sync(FULL, going)) {
-    const bool act = going && g.gl < nch;
+    bool act = going && g.gl < nch;
     const bool chance = (level >> a.kind_shift) & 1;
     const int ci = act ? cbase + g.gl : 0;                     // idle lanes read node 0 and discard it
     int4 st;
@@ -258,16 +270,40 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
       st = a.stat[tb + ci];
       lk = a.link[tb + ci];
     }
-    if (!act) { st = make_int4(0, 0, 0, 0); lk = make_int2(0, 0); }
-    const double pbc = chance ? 0.0 : a.pbc[going ? parent_visit : 0];     // plain load: the table may live in shared memory
-    // the draw only depends on the cursor; a window of draws may have been generated ahead (SmzRng::win)
-    const int uidx = chance ? cursor : cursor + g.gl;
-    const bool want = going && (chance || act);
-    const unsigned wofs = (unsigned)(uidx - rng.win_base);
-    const bool hit = rng.win != nullptr && wofs < (unsigned)rng.win_len;
-    double u = hit ? rng.win[wofs] : 0.0;
-    if (__any_sync(FULL, want && !hit)) {
-      if (want && !hit) u = smz_rng_uniform(rng, tree, uidx);
+    // The root (a decision node in both patterns) scores its legal children only: an illegal action's slot holds key -1.
+    // Child j takes draw `cursor + rank of j among the legal children`, and the root consumes |L| draws.
+    const bool root = level == 0;
+    int width = nch;
+    double pbc, u;
+    if constexpr (MIRROR) {      // the node records are at hand: the draw is indexed by legal rank
+      int rank = g.gl;
+      if (root) {
+        act = act && lk.y >= 0;
+        const unsigned lm = g.ballot(act);
+        rank = __popc(lm & ((1u << g.gl) - 1u));
+        width = __popc(lm);
+      }
+      if (!act) { st = make_int4(0, 0, 0, 0); lk = make_int2(0, 0); }
+      pbc = chance ? 0.0 : a.pbc[going ? parent_visit : 0];     // plain load: the table lives in shared memory
+      u = draw_uniform(rng, tree, chance ? cursor : cursor + rank, going && (chance || act));
+    } else {
+      // the node records are still in flight: the draws are taken by lane index without waiting for them, and child
+      // j gets the draw of lane `rank` by a shuffle.  With a tape only lanes 0..|L|-1 draw, so the tape is read
+      // exactly where the search reads it.
+      pbc = chance ? 0.0 : a.pbc[going ? parent_visit : 0];
+      bool want = going && (chance || act);
+      if (root && rng.mode) {    // every lane takes part in the ballot (no short-circuit around it)
+        const int n_legal = __popc(g.ballot(act && lk.y >= 0));
+        want = want && g.gl < n_legal;
+      }
+      u = draw_uniform(rng, tree, chance ? cursor : cursor + g.gl, want);
+      if (root) {
+        act = act && lk.y >= 0;
+        const unsigned lm = g.ballot(act);
+        width = __popc(lm);
+        u = g.bcast(u, __popc(lm & ((1u << g.gl) - 1u)));
+      }
+      if (!act) { st = make_int4(0, 0, 0, 0); lk = make_int2(0, 0); }
     }
     int pick = 0;
     if (chance) {
@@ -315,7 +351,7 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
         const int ob = __shfl_xor_sync(FULL, best, off, G);
         if (os > score || (os == score && ob > best)) { score = os; best = ob; }
       }
-      if (!chance) { pick = best < 0 ? 0 : best; cursor += going ? nch : 0; }
+      if (!chance) { pick = best < 0 ? 0 : best; cursor += going ? width : 0; }
     }
     const int4 cst = make_int4(g.bcast(st.x, pick), g.bcast(st.y, pick), g.bcast(st.z, pick), 0);
     const int child_cb = g.bcast(lk.x, pick);

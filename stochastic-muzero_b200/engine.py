@@ -52,6 +52,32 @@ def player_tables(number_of_player: int, custom_loop: Optional[str], n_depth: in
     return sign, to_play
 
 
+def legal_rows(legal, n: Optional[int] = None, A: Optional[int] = None) -> torch.Tensor:
+    """A legal-action mask -> bool tensor [n, A] on the device it came from (bool, or 0/1 values; bit a of row i says
+    whether action a is legal at the root of tree i).  The shape is checked always; a mask on the host is also checked
+    for an empty row here, before any GPU work (a mask already on the device is checked by the root kernel: error flag
+    3, see smz_root_legal in include/smz.h)."""
+    t = legal if torch.is_tensor(legal) else torch.as_tensor(np.asarray(legal))
+    if t.dim() != 2 or (n is not None and t.shape[0] != n) or (A is not None and t.shape[1] != A) or t.shape[1] > 32:
+        want = f"[{n if n is not None else 'n'}, {A if A is not None else 'A <= 32'}]"
+        raise ValueError(f"legal-action mask must have shape {want}, got {list(t.shape)}")
+    if not t.is_cuda:
+        if t.dtype != torch.bool and not ((t == 0) | (t == 1)).all():
+            raise ValueError("a legal-action mask holds bools or 0 / 1 values")
+        empty = (~(t != 0).any(1)).nonzero().flatten()
+        if empty.numel():
+            raise ValueError(f"legal-action mask rows {empty[:8].tolist()} have no legal action")
+    return t != 0
+
+
+def pack_legal(mask: torch.Tensor) -> torch.Tensor:
+    """bool [n, A <= 32] -> int32 [n] words, bit a = column a, on the mask's device (the uint32 words of
+    smz_root_legal; bit 31 lands in the sign bit)."""
+    bits = torch.arange(mask.shape[1], device=mask.device, dtype=torch.int64)
+    w = (mask.to(torch.int64) << bits).sum(1)
+    return torch.where(w >= 2 ** 31, w - 2 ** 32, w).to(torch.int32)
+
+
 class RootStats(dict):
     """read_roots() result: the tensors by name; ``block`` = the device block that holds visits | root values | error."""
     block = None
@@ -209,9 +235,15 @@ class SearchEngine:
         assert t.dim() == 2
         self._check(self.lib.smz_set_uniform_tape(self._h, self._ptr(t), t.shape[1]))
 
-    def root(self, obs=None, root_policy=None, root_to_play=None, train=True, dirichlet=None):
+    def root(self, obs=None, root_policy=None, root_to_play=None, train=True, dirichlet=None, legal=None):
+        """Root step of a search of n trees.  ``legal``: bool / 0-1 mask [n, A] (host or device) restricting each
+        root to the legal actions of its position (smz_root_legal in include/smz.h), or None for every action."""
         src = obs if obs is not None else root_policy
         n = int(src.shape[0])
+        words = None
+        if legal is not None:
+            words = pack_legal(self.to_device(legal_rows(legal, n, self.A), torch.bool))
+            self._keep["legal"] = words
         obs_t = self._dev(obs, torch.float32, "obs")
         pol_t = None
         if root_policy is not None:
@@ -219,8 +251,8 @@ class SearchEngine:
         rtp = self._dev(root_to_play, torch.int32, "root_to_play")
         dr = self._dev(dirichlet, torch.float64, "dirichlet")
         self._apply_node_pattern()
-        self._check(self.lib.smz_root(self._h, n, self._ptr(obs_t), self._ptr(pol_t), self._ptr(rtp), int(bool(train)),
-                                      self._ptr(dr), self._stream))
+        self._check(self.lib.smz_root_legal(self._h, n, self._ptr(obs_t), self._ptr(pol_t), self._ptr(rtp),
+                                            self._ptr(words), int(bool(train)), self._ptr(dr), self._stream))
         self.n_trees = n
         self.generation += 1
 
@@ -322,6 +354,9 @@ class SearchEngine:
         if code == 2:       # np.random.choice at monte_carlo_tree_search.py:208 / :294 raises ValueError here
             raise ValueError("probabilities contain NaN or sum to zero: a policy met during expansion was degenerate "
                              "(np.random.choice raises at this point in the reference)")
+        if code == 3:
+            raise ValueError("a legal-action mask was empty or named an action >= A (that tree was searched with every "
+                             "action legal)")
 
     def select_actions(self, temperature: float, uniforms=None):
         """game.py:179-235 for every tree: -> dict(actions int32[n], policy f64[n,A], stored_policy f64[n,A])."""
@@ -395,8 +430,10 @@ class SearchEngine:
                          ar["reward"][n], prior, _is_chance(d, self.paper_alternation), int(self.to_play_table[phase, d]),
                          cb != 0, n))
             if cb:
-                k = self.n_children(d)
-                stack.extend((cb + i, d + 1) for i in reversed(range(k)))
+                kids = range(cb, cb + self.n_children(d))
+                if d == 0:      # the slots of illegal root actions hold key -1 (smz_root_legal): not children
+                    kids = [c for c in kids if ar["key"][c] >= 0]
+                stack.extend((c, d + 1) for c in reversed(kids))
         names = ("depth", "key", "visit", "value_sum", "reward", "prior", "is_chance", "to_play", "expanded", "node")
         dtypes = (np.int32, np.int32, np.int32, np.float32, np.float32, np.float64, np.int8, np.int32, np.int8, np.int32)
         out = {k: np.array([r[i] for r in rows], dtype=dt) for i, (k, dt) in enumerate(zip(names, dtypes))}

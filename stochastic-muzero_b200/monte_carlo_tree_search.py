@@ -23,7 +23,7 @@ import numpy as np
 import torch
 
 from . import batched_model
-from .engine import SearchEngine
+from .engine import SearchEngine, legal_rows
 from .weights import (PackedModel, VisionShape, pack_vision_weights, pack_weights, shape_of, weights_version)
 
 
@@ -141,6 +141,28 @@ def _node_tree(dump, hidden_fetch=None):
         stack.append((d, node))
         nodes.append(node)
     return nodes[0]
+
+
+def _legal_row(legal_actions, A):
+    """``run``'s legal actions (a sequence of action indices, or a bool mask [A]) -> bool mask [1, A] on the host."""
+    if torch.is_tensor(legal_actions):
+        legal_actions = legal_actions.cpu()
+    a = np.asarray(legal_actions)
+    if a.dtype == np.bool_:
+        if a.shape != (A,):
+            raise ValueError(f"a bool legal-action mask has shape [{A}], got {list(a.shape)}")
+        return a.reshape(1, A)
+    idx = a.astype(np.int64).reshape(-1)
+    if idx.size == 0 or (idx < 0).any() or (idx >= A).any():
+        raise ValueError(f"legal actions must be a non-empty sequence of indices in [0, {A}), got {idx.tolist()}")
+    row = np.zeros((1, A), np.bool_)
+    row[0, idx] = True
+    return row
+
+
+def _legal_kw(legal):
+    """root() keyword for an optional mask (no keyword at all without one: the unmasked call stays as it was)."""
+    return {} if legal is None else {"legal": legal}
 
 
 class StaleSearchError(RuntimeError):
@@ -371,13 +393,21 @@ class Monte_carlo_tree_search():
         self._per_model = weakref.WeakKeyDictionary()
 
     # ------------------------------------------------------------------------------------------
-    def run_batch(self, observations, model=None, train=True, root_to_play=None, check=True) -> BatchedRoots:
+    def run_batch(self, observations, model=None, train=True, root_to_play=None, check=True, *,
+                  legal_actions=None) -> BatchedRoots:
         """B independent searches in one call.  ``observations``: float tensor/array [B, obs_dim]
         (host or device).  Returns BatchedRoots (device tensors; ``roots[i]`` gives a Node view).
         ``check`` (default): wait for the search and raise if it met a degenerate policy, like the reference's
-        np.random.choice does; ``check=False`` returns without synchronising (``roots.raise_if_failed()`` later)."""
+        np.random.choice does; ``check=False`` returns without synchronising (``roots.raise_if_failed()`` later).
+        ``legal_actions``: bool / 0-1 mask [B, A] (host or device): each root searches the legal actions of its
+        position only, as the reference's root would with that action space; illegal actions get no child, no visit and
+        prior 0, and ``select_actions`` never returns one.  A host mask with an empty row raises ValueError before any
+        GPU work; a device mask with an empty row or a bit >= A raises ValueError at the check (that tree is searched
+        with every action legal)."""
+        if legal_actions is not None:
+            legal_actions = legal_rows(legal_actions, len(observations))
         if not self._is_fusable(model):
-            roots = self._run_batch_external(observations, model, train, root_to_play)
+            roots = self._run_batch_external(observations, model, train, root_to_play, legal_actions)
             return roots.raise_if_failed() if check else roots
         self.model = model
         vision = getattr(model, "model_structure", None) == "vision_model"
@@ -405,12 +435,12 @@ class Monte_carlo_tree_search():
                 self._weights_seen[key] = ver
         obs = eng.to_device(obs, torch.float32)      # the observations' host-to-device copy is enqueued first
         eng.set_seed(self._next_seed(), self._offset(obs.shape[0]))
-        eng.root(obs=obs, root_to_play=root_to_play, train=train)
+        eng.root(obs=obs, root_to_play=root_to_play, train=train, **_legal_kw(legal_actions))
         eng.simulate(self.num_simulations)
         roots = BatchedRoots(eng, eng.read_roots())
         return roots.raise_if_failed() if check else roots
 
-    def _run_batch_external(self, observations, model, train, root_to_play):
+    def _run_batch_external(self, observations, model, train, root_to_play, legal_actions=None):
         """Any other model family: tree kernels in the engine, network step = five batched device
         functions (batched_model.py) — either supplied directly or built from the six nn.Modules of a
         reference-style Muzero."""
@@ -434,30 +464,36 @@ class Monte_carlo_tree_search():
         C = int(getattr(backend, "C", A))
         eng, _ = self._engine("external", obs.shape[0], A, C)
         eng.set_seed(self._next_seed(), self._offset(obs.shape[0]))
-        store = batched_model.run_search(eng, backend, obs, self.num_simulations, root_to_play, train)
+        store = batched_model.run_search(eng, backend, obs, self.num_simulations, root_to_play, train, legal_actions)
         roots = BatchedRoots(eng, eng.read_roots())
         roots.hidden_store = store
         return roots
 
-    def run(self, observation=None, model=None, train=True):
-        """One search, reference signature (:311).  Returns the root Node."""
+    def run(self, observation=None, model=None, train=True, *, legal_actions=None):
+        """One search, reference signature (:311).  Returns the root Node.  ``legal_actions``: the legal actions of the
+        position, as a sequence of action indices or a bool mask [A] (see ``run_batch``); ``root.children`` then has
+        exactly those keys."""
         self.model = model
         to_play = self.cycle.global_step()
         if self._is_fusable(model):
             obs = observation if torch.is_tensor(observation) else torch.as_tensor(np.asarray(observation))
+            legal = None
+            if legal_actions is not None:
+                legal = _legal_row(legal_actions, model.shape.action_dim if isinstance(model, PackedModel)
+                                   else int(model.action_dimension))
             batch = self.run_batch(obs.reshape(1, *obs.shape[1:]) if obs.dim() > 1 else obs.reshape(1, -1), model, train,
-                                   root_to_play=torch.tensor([to_play], dtype=torch.int32))
+                                   root_to_play=torch.tensor([to_play], dtype=torch.int32), legal_actions=legal)
             eng = batch._engine
             dump = eng.export_tree(0)
             self.root = _node_tree(dump, batch._hidden_fetcher(0))
         else:
-            self.root = self._run_callback(observation, model, train, to_play)
+            self.root = self._run_callback(observation, model, train, to_play, legal_actions)
             return self.root
         self.min_max_stats = MinMaxStats(np.float32(dump["minmax"][0]), np.float32(dump["minmax"][1]))
         self.node = self.root
         return self.root
 
-    def _run_callback(self, observation, model, train, to_play):
+    def _run_callback(self, observation, model, train, to_play, legal_actions=None):
         """Host-model mode: tree kernels on the GPU, the five inference methods called back per
         simulation (:182, :198, :271-286)."""
         h0 = model.representation_function_inference(observation)
@@ -466,7 +502,9 @@ class Monte_carlo_tree_search():
         A = policy.shape[1]
         eng, _ = self._engine("external", 1, A, getattr(model, "chance_dimension", A))
         eng.set_seed(self._next_seed(), self._offset(1))
-        eng.root(root_policy=policy, root_to_play=torch.tensor([to_play], dtype=torch.int32), train=train)
+        legal = None if legal_actions is None else _legal_row(legal_actions, A)
+        eng.root(root_policy=policy, root_to_play=torch.tensor([to_play], dtype=torch.int32), train=train,
+                 **_legal_kw(legal))
         hidden = {0: h0}
         for sim in range(self.num_simulations):
             slot, action, branch = (int(t.item()) for t in eng.select(sim))

@@ -11,7 +11,8 @@ rewards, stored visit policies, root values — Game.store_search_statistics / m
 game.py:179-204, :291-337) is written into preallocated device tensors [T, B, ...].
 
 The environment is any object with `reset(mask) -> obs[B, ...]` and
-`step(action[B]) -> (obs, reward[B], done[B])` on the device.  `VectorCartPole` is the synthetic vector
+`step(action[B]) -> (obs, reward[B], done[B])` on the device; one that also has `legal_mask() -> bool[B, A]` gets
+each search restricted to the legal actions of its position.  `VectorCartPole` is the synthetic vector
 environment used here: CartPole-v1's published equations of motion (Barto, Sutton & Anderson 1983, as used by
 gymnasium's cartpole.py: gravity 9.8, cart 1.0 kg, pole 0.1 kg, half-length 0.5 m, force 10 N, tau 0.02 s,
 Euler integration, termination at |x| > 2.4 or |theta| > 12 degrees, reward 1 per step, 500-step limit),
@@ -85,7 +86,8 @@ class SelfPlay:
                "child_visits": torch.zeros(T, B, A, dtype=torch.float64, device=dev),
                "root_values": torch.zeros(T, B, device=dev)}
         for t in range(T):
-            roots = self.mcts.run_batch(obs, self.model, train=train)               # one move of every game
+            legal = env.legal_mask() if hasattr(env, "legal_mask") else None
+            roots = self.mcts.run_batch(obs, self.model, train=train, legal_actions=legal)   # one move of every game
             pick = roots.select_actions(temperature)                                # game.py:223-235 on the device
             buf["observations"][t], buf["actions"][t] = obs, pick["actions"]
             buf["child_visits"][t], buf["root_values"][t] = pick["stored_policy"], roots.root_values
@@ -96,16 +98,20 @@ class SelfPlay:
 
 
 @torch.no_grad()
-def reanalyse(mcts, model, observations: torch.Tensor, chunk: int = 16384, train: bool = True) -> Dict[str, torch.Tensor]:
+def reanalyse(mcts, model, observations: torch.Tensor, chunk: int = 16384, train: bool = True,
+              legal_actions: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
     """Reanalyse (self_play.py:30-44, game.py:112-116, replay_buffer.py:229-266): re-run the search over stored
     observations of old games with the current weights.  Every stored position is an independent tree, so
     the [T, B, ...] trajectory block is simply flattened into large batches for the engine.
+    ``legal_actions``: optional bool mask [T, B, A] of the stored positions' legal actions.
     Returns fresh targets: child_visits [T, B, A] (stored visit policy) and root_values [T, B]."""
     T, B = observations.shape[:2]
     flat = observations.reshape((T * B,) + tuple(observations.shape[2:]))
+    legal = None if legal_actions is None else legal_actions.reshape(T * B, -1)
     visits, values = [], []
     for lo in range(0, T * B, chunk):
-        roots = mcts.run_batch(flat[lo:lo + chunk], model, train=train)
+        roots = mcts.run_batch(flat[lo:lo + chunk], model, train=train,
+                               legal_actions=None if legal is None else legal[lo:lo + chunk])
         visits.append(roots.select_actions(0.0)["stored_policy"])
         values.append(roots.root_values.clone())
     child_visits = torch.cat(visits)
