@@ -164,6 +164,30 @@ enum {
 };
 int smz_set_node_pattern(smz_engine* e, int32_t pattern);
 
+/* Search policy at decision nodes.  SMZ_SEARCH_PUCT (default) is the reference's pUCT with Dirichlet noise at the root
+ * (smz_root / smz_root_legal).  SMZ_SEARCH_GUMBEL is Gumbel MuZero (Danihelka et al., "Policy improvement by planning
+ * with Gumbel", ICLR 2022), rooted by smz_root_gumbel and read out by smz_read_gumbel:
+ *   - per decision node, over its existing children i (the root: its legal children) with prior p_i (float64 at the
+ *     root, float32 below), visit count N_i and q_i = reward + discount * value() in float32 (pUCT's value term before
+ *     min-max normalisation), and the node's own network value v: v_mix = (v + sum N * (sum_{N_i>0} p_i q_i) /
+ *     (sum_{N_i>0} p_i)) / (sum N + 1) (v when sum N = 0); completed value cq_i = q_i if N_i > 0 else v_mix;
+ *     r_i = (cq_i - min cq) / max(max cq - min cq, 1e-8); sigma_i = (c_visit + max N) * c_scale * r_i.  float64, in
+ *     this order, sums in ascending child order;
+ *   - interior decision nodes: argmax of pi'_i - N_i / (1 + sum N), pi' = p_i exp(sigma_i - max sigma) / sum_j ...;
+ *   - root: one Gumbel g_a per legal action per search; logit_a = log p_a - max_b log p_b; the children whose visit
+ *     count equals the Sequential Halving schedule T[min(m, |L|)][sum N] compete on max(-1e9, g_a + logit_a + sigma_a);
+ *   - ties go to the smaller action, and no decision node draws a uniform; chance nodes and the expansions keep the
+ *     reference's draws; no Dirichlet noise is mixed.
+ * max_considered in [1, 32] (m, default 16), c_visit >= 0 (default 50), c_scale >= 0 (default 0.1), both finite;
+ * anything else, or another policy value, returns SMZ_E_INVALID_ARG.  The setting applies from the next root: in Gumbel
+ * mode smz_root / smz_root_legal return SMZ_E_STATE, in pUCT mode smz_root_gumbel does.  A search already rooted keeps
+ * its policy; switching drops the captured smz_simulate graph. */
+enum {
+  SMZ_SEARCH_PUCT = 0,
+  SMZ_SEARCH_GUMBEL = 1
+};
+int smz_set_search(smz_engine* e, int32_t policy, int32_t max_considered, double c_visit, double c_scale);
+
 /* Tape inputs (rng_mode == SMZ_RNG_TAPE): uniforms_dev is double[n_trees][stride]. */
 int smz_set_uniform_tape(smz_engine* e, const double* uniforms_dev, int32_t stride);
 
@@ -191,6 +215,17 @@ int smz_root(smz_engine* e, int32_t n_trees, const float* obs_dev, const float* 
 int smz_root_legal(smz_engine* e, int32_t n_trees, const float* obs_dev, const float* root_policy_dev,
                    const int32_t* root_to_play_dev, const uint32_t* legal_dev, int32_t train,
                    const double* dirichlet_dev, void* stream);
+
+/* Root step of a Gumbel search (smz_set_search(SMZ_SEARCH_GUMBEL)): smz_root_legal's arguments without Dirichlet noise,
+ * plus root_value_dev float[n_trees], the network value of each root — required with root_policy_dev, NULL with obs_dev
+ * (the internal network's value is used).  train == 0 sets every Gumbel to 0; with train != 0 (also with N == 0)
+ * gumbel_dev is double[n_trees][A] recorded Gumbels (entries at illegal actions are ignored), or NULL to draw them on
+ * the device: -log(-log u), u = uniform #rank of Philox stream 3 keyed by (seed, global tree id), rank = position of
+ * the action among the legal ones, so the draws do not depend on how trees are sharded.  The legal mask behaves as in
+ * smz_root_legal (flag 3 included). */
+int smz_root_gumbel(smz_engine* e, int32_t n_trees, const float* obs_dev, const float* root_policy_dev,
+                    const float* root_value_dev, const int32_t* root_to_play_dev, const uint32_t* legal_dev,
+                    int32_t train, const double* gumbel_dev, void* stream);
 
 /* n_sims full simulations (:325-347) with the internal network (net_mode FP32/BF16). */
 int smz_simulate(smz_engine* e, int32_t n_sims, void* stream);
@@ -241,6 +276,15 @@ int smz_read_roots(smz_engine* e, int32_t* visits_dev, float* root_values_dev, d
  * recorded draws, or NULL for device Philox (stream 2).  Any output may be NULL. */
 int smz_select_actions(smz_engine* e, double temperature, const double* uniforms_dev, int32_t* actions_dev,
                        double* policy_dev, double* stored_policy_dev, void* stream);
+/* Read-out of a Gumbel search: actions_dev int32[n] = argmax over the legal actions with the most visits of
+ * g_a + logit_a + sigma_a (with N = 0 a Gumbel-max sample of the prior); improved_policy_dev double[n][A] = softmax
+ * over the legal actions of logit_a + sigma_a, 0 for illegal actions (the policy target); gumbels_dev double[n][A] =
+ * the search's Gumbels (0 for illegal actions), for replay through smz_root_gumbel.  Any pointer may be NULL.
+ * SMZ_E_STATE unless the current search was rooted by smz_root_gumbel. */
+int smz_read_gumbel(smz_engine* e, int32_t* actions_dev, double* improved_policy_dev, double* gumbels_dev, void* stream);
+/* Network value of every expanded node of a Gumbel search by hidden slot (0 = root, s+1 = node expanded by simulation
+ * s): float[n][N+1].  SMZ_E_STATE unless the current search was rooted by smz_root_gumbel. */
+int smz_read_raw_values(smz_engine* e, float* out_dev, void* stream);
 /* Synchronises `stream`, then copies one tree to host memory. */
 int smz_export_tree(smz_engine* e, int32_t tree, smz_tree_host* out, void* stream);
 /* Hidden state of a slot (0 = root, s+1 = node expanded by simulation s): float[n][hidden_stride]. */

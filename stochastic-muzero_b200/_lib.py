@@ -11,6 +11,7 @@ SMZ_OK, SMZ_E_INVALID_ARG, SMZ_E_CUDA, SMZ_E_CAPACITY, SMZ_E_STATE = 0, -1, -2, 
 NET_EXTERNAL, NET_FP32, NET_BF16, NET_VISION, NET_TC32, NET_F16 = 0, 1, 2, 3, 4, 5
 RNG_PHILOX, RNG_TAPE = 0, 1
 PATTERN_REFERENCE, PATTERN_PAPER = 0, 1
+SEARCH_PUCT, SEARCH_GUMBEL = 0, 1
 
 
 class smz_config(C.Structure):
@@ -60,6 +61,10 @@ SIGNATURES = {
     "smz_set_node_pattern": (C.c_int, [_P, C.c_int32]),
     "smz_root": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
     "smz_root_legal": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, C.c_int32, _P, _P]),
+    "smz_set_search": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_double, C.c_double]),
+    "smz_root_gumbel": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
+    "smz_read_gumbel": (C.c_int, [_P, _P, _P, _P, _P]),
+    "smz_read_raw_values": (C.c_int, [_P, _P, _P]),
     "smz_simulate": (C.c_int, [_P, C.c_int32, _P]),
     "smz_select": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P]),
     "smz_net_step": (C.c_int, [_P, C.c_int32, _P]),

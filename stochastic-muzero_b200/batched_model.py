@@ -91,11 +91,15 @@ def run_search(engine, backend, observations, n_sims, root_to_play=None, train=T
     dev = torch.device("cuda", engine.device)
     h0 = backend.representation(observations)
     B = h0.shape[0]
-    policy, _value = backend.prediction(h0)
+    policy, value = backend.prediction(h0)
     store = torch.zeros((n_sims + 1,) + tuple(h0.shape), dtype=h0.dtype, device=dev)
     store[0] = h0
-    engine.root(root_policy=policy.float(), root_to_play=root_to_play, train=train,
-                **({} if legal is None else {"legal": legal}))
+    kw = {} if legal is None else {"legal": legal}
+    if engine.gumbel:          # the Gumbel search completes Q-values with each node's network value, the root's too
+        engine.root_gumbel(root_policy=policy.float(), root_value=value.float().reshape(-1), root_to_play=root_to_play,
+                           train=train, **kw)
+    else:
+        engine.root(root_policy=policy.float(), root_to_play=root_to_play, train=train, **kw)
     W = engine.dims.policy_stride
     rows = torch.arange(B, device=dev)
     for sim in range(n_sims):

@@ -8,6 +8,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
 #include <vector>
 
 #include "../../include/smz.h"
@@ -75,6 +76,9 @@ struct smz_engine {
   cudaStream_t capture_stream;
   int use_pdl;
   int32_t node_pattern;  // SMZ_PATTERN_*, copied into the arena (a.kind_shift) by the next smz_root
+  // search policy of the next root (smz_set_search), copied into the arena (a.gumbel, a.gumbel_m, a.c_visit, a.c_scale)
+  int32_t search_policy, gumbel_m;
+  double c_visit, c_scale;
 };
 
 const char* smz_last_error(void) { return g_err; }
@@ -168,6 +172,8 @@ int smz_create(const smz_config* cfg, smz_engine** out) {
   a.n_phases = 1;
   a.kind_shift = 1;
   e->node_pattern = SMZ_PATTERN_REFERENCE;
+  e->search_policy = SMZ_SEARCH_PUCT;
+  e->gumbel_m = 16; e->c_visit = 50.0; e->c_scale = 0.1;
   a.rng_mode = c.rng_mode;
   a.discount = (float)c.discount;
   a.one_minus_frac_f32 = (float)(1.0 - c.root_exploration_fraction);
@@ -378,6 +384,63 @@ int smz_set_node_pattern(smz_engine* e, int32_t pattern) {
   return SMZ_OK;
 }
 
+// Sequential Halving's considered visits (Danihelka et al. 2022, as the published implementation tabulates them):
+// row n (0..SMZ_MAX_POLICY) holds the visit count the next simulation's root child must have, for sum N = 0..N-1
+static void considered_visits(int n, int N, int* row) {
+  if (n <= 1) {
+    for (int i = 0; i < N; ++i) row[i] = i;
+    return;
+  }
+  int log2max = 0;
+  while ((1 << log2max) < n) ++log2max;                          // ceil(log2 n)
+  std::vector<int> visits(n, 0);
+  int k = n, len = 0;
+  while (len < N) {
+    const int extra = std::max(1, (int)((double)N / (double)(log2max * k)));
+    for (int r = 0; r < extra; ++r)
+      for (int i = 0; i < k; ++i) {
+        if (len < N) row[len] = visits[i];
+        ++len;
+        ++visits[i];
+      }
+    k = std::max(2, k / 2);
+  }
+}
+
+int smz_set_search(smz_engine* e, int32_t policy, int32_t max_considered, double c_visit, double c_scale) {
+  if (policy != SMZ_SEARCH_PUCT && policy != SMZ_SEARCH_GUMBEL)
+    return fail(SMZ_E_INVALID_ARG, "smz_set_search: policy %d is neither SMZ_SEARCH_PUCT (0) nor SMZ_SEARCH_GUMBEL (1)",
+                policy);
+  if (max_considered < 1 || max_considered > SMZ_MAX_POLICY)
+    return fail(SMZ_E_INVALID_ARG, "smz_set_search: max_considered %d not in [1, %d]", max_considered, SMZ_MAX_POLICY);
+  if (!(c_visit >= 0.0 && c_visit < INFINITY) || !(c_scale >= 0.0 && c_scale < INFINITY))
+    return fail(SMZ_E_INVALID_ARG, "smz_set_search: c_visit and c_scale must be finite and >= 0");
+  if (!e) return fail(SMZ_E_INVALID_ARG, "smz_set_search: null engine");
+  SmzArena& a = e->a;
+  if (policy == SMZ_SEARCH_GUMBEL && !a.raw_value) {      // the Gumbel columns are allocated on first use
+    ON_DEVICE(e);
+    const size_t B = a.B, Nt = a.N > 0 ? a.N : 1;
+    int* table = nullptr;
+    CU(dev_alloc(e, &a.raw_value, B * (a.N + 1)));
+    CU(dev_alloc(e, &a.gumbel_g, B * a.A));
+    CU(dev_alloc(e, &a.root_logit, B * a.A));
+    CU(dev_alloc(e, &table, (SMZ_MAX_POLICY + 1) * Nt));
+    std::vector<int> t((SMZ_MAX_POLICY + 1) * Nt, 0);
+    for (int n = 0; n <= SMZ_MAX_POLICY; ++n) considered_visits(n, a.N, t.data() + n * a.N);
+    CU(cudaMemcpy(table, t.data(), t.size() * sizeof(int), cudaMemcpyHostToDevice));
+    a.cv_table = table;
+  }
+  e->search_policy = policy;
+  e->gumbel_m = max_considered;
+  e->c_visit = c_visit;
+  e->c_scale = c_scale;
+  return SMZ_OK;
+}
+
+static int root_step(smz_engine* e, int32_t n_trees, const float* obs, const float* root_policy,
+                     const float* root_value, const int32_t* root_to_play, const uint32_t* legal, int32_t train,
+                     const double* dirichlet, const double* gumbels, bool gumbel, void* stream);
+
 int smz_root(smz_engine* e, int32_t n_trees, const float* obs, const float* root_policy, const int32_t* root_to_play,
              int32_t train, const double* dirichlet, void* stream) {
   return smz_root_legal(e, n_trees, obs, root_policy, root_to_play, nullptr, train, dirichlet, stream);
@@ -387,6 +450,29 @@ int smz_root_legal(smz_engine* e, int32_t n_trees, const float* obs, const float
                    const int32_t* root_to_play, const uint32_t* legal, int32_t train, const double* dirichlet,
                    void* stream) {
   if (!e) return fail(SMZ_E_INVALID_ARG, "smz_root: null engine");
+  if (e->search_policy != SMZ_SEARCH_PUCT)
+    return fail(SMZ_E_STATE, "smz_root: the engine is set to the Gumbel search (smz_set_search): root it with "
+                "smz_root_gumbel");
+  return root_step(e, n_trees, obs, root_policy, nullptr, root_to_play, legal, train, dirichlet, nullptr, false, stream);
+}
+
+int smz_root_gumbel(smz_engine* e, int32_t n_trees, const float* obs, const float* root_policy, const float* root_value,
+                    const int32_t* root_to_play, const uint32_t* legal, int32_t train, const double* gumbels,
+                    void* stream) {
+  if (!e) return fail(SMZ_E_INVALID_ARG, "smz_root_gumbel: null engine");
+  if (e->search_policy != SMZ_SEARCH_GUMBEL)
+    return fail(SMZ_E_STATE, "smz_root_gumbel: the engine is set to the pUCT search (smz_set_search)");
+  if (root_policy && !root_value)
+    return fail(SMZ_E_INVALID_ARG, "smz_root_gumbel: root_value_dev is required with root_policy_dev");
+  if (obs && root_value)
+    return fail(SMZ_E_INVALID_ARG, "smz_root_gumbel: root_value_dev must be NULL with obs_dev (the network's value is "
+                "used)");
+  return root_step(e, n_trees, obs, root_policy, root_value, root_to_play, legal, train, nullptr, gumbels, true, stream);
+}
+
+static int root_step(smz_engine* e, int32_t n_trees, const float* obs, const float* root_policy,
+                     const float* root_value, const int32_t* root_to_play, const uint32_t* legal, int32_t train,
+                     const double* dirichlet, const double* gumbels, bool gumbel, void* stream) {
   if (n_trees < 1 || n_trees > e->a.B) return fail(SMZ_E_CAPACITY, "smz_root: n_trees %d not in [1, %d]", n_trees, e->a.B);
   if ((obs == nullptr) == (root_policy == nullptr))
     return fail(SMZ_E_INVALID_ARG, "smz_root: give exactly one of obs_dev / root_policy_dev");
@@ -401,6 +487,14 @@ int smz_root_legal(smz_engine* e, int32_t n_trees, const float* obs, const float
     a.kind_shift = kind_shift;
     drop_graph(e);
   }
+  if (a.gumbel != (int)gumbel || (gumbel && (a.gumbel_m != e->gumbel_m || a.c_visit != e->c_visit ||
+                                             a.c_scale != e->c_scale))) {
+    a.gumbel = gumbel;
+    a.gumbel_m = e->gumbel_m;
+    a.c_visit = e->c_visit;
+    a.c_scale = e->c_scale;
+    drop_graph(e);
+  }
   smz_launch_begin_search(a, s);       // row counters, error flag, depth statistic
   if (a.dbg) {      // wall-clock stamps: "first" slots start at all-ones (atomicMin), "last" slots at zero (atomicMax)
     std::vector<unsigned long long> init(4 * ((size_t)a.N + 2));
@@ -409,7 +503,7 @@ int smz_root_legal(smz_engine* e, int32_t n_trees, const float* obs, const float
     CU(cudaStreamSynchronize(s));
   }
   e->launches = 0;
-  if (e->cfg.num_simulations == 0) train = 0;   // mcts.py:215-216
+  if (e->cfg.num_simulations == 0 && !gumbel) train = 0;   // mcts.py:215-216
   const float* policy = root_policy;
   if (obs) {
     if (e->vision) { smz_vision_root(e->vision, a, n_trees, obs, s); count_launches(e, 1); }
@@ -419,7 +513,7 @@ int smz_root_legal(smz_engine* e, int32_t n_trees, const float* obs, const float
     count_launches(e, 1);
     policy = a.out_policy;
   }
-  if (train) {
+  if (train && !gumbel) {
     if (dirichlet) {
       CU(cudaMemcpyAsync(a.dirichlet, dirichlet, (size_t)n_trees * a.A * sizeof(double), cudaMemcpyDeviceToDevice, s));
     } else {
@@ -427,8 +521,13 @@ int smz_root_legal(smz_engine* e, int32_t n_trees, const float* obs, const float
       count_launches(e, 1);
     }
   }
-  smz_launch_root_expand(a, e->cfg.lanes_per_tree, n_trees, policy, a.W, root_to_play, train, a.dirichlet, legal, s);
+  smz_launch_root_expand(a, e->cfg.lanes_per_tree, n_trees, policy, a.W, root_to_play, gumbel ? 0 : train, a.dirichlet,
+                         legal, s);
   count_launches(e, 1);
+  if (gumbel) {      // no Dirichlet noise: the root's Gumbels take its place
+    smz_launch_gumbel_root(a, n_trees, obs ? a.out_value : root_value, train, gumbels, s);
+    count_launches(e, 1);
+  }
   CU(cudaGetLastError());
   e->n_trees = n_trees;
   a.row_top = (n_trees + 511) / 512 * 512 + 512;    // see smz_common.cuh: rows of the two branches never share a tile (group of 4)
@@ -607,6 +706,25 @@ int smz_select_actions(smz_engine* e, double temperature, const double* uniforms
   smz_launch_select_actions(e->a, e->n_trees, temperature, uniforms, actions, policy, stored_policy, (cudaStream_t)stream);
   count_launches(e, 1);
   CU(cudaGetLastError());
+  return SMZ_OK;
+}
+
+int smz_read_gumbel(smz_engine* e, int32_t* actions, double* improved_policy, double* gumbels, void* stream) {
+  if (!e) return fail(SMZ_E_INVALID_ARG, "smz_read_gumbel: null engine");
+  if (e->n_trees < 1 || !e->a.gumbel) return fail(SMZ_E_STATE, "smz_read_gumbel: no search rooted by smz_root_gumbel");
+  ON_DEVICE(e);
+  smz_launch_read_gumbel(e->a, e->n_trees, actions, improved_policy, gumbels, (cudaStream_t)stream);
+  count_launches(e, 1);
+  CU(cudaGetLastError());
+  return SMZ_OK;
+}
+
+int smz_read_raw_values(smz_engine* e, float* out, void* stream) {
+  if (!e || !out) return fail(SMZ_E_INVALID_ARG, "smz_read_raw_values: null argument");
+  if (e->n_trees < 1 || !e->a.gumbel) return fail(SMZ_E_STATE, "smz_read_raw_values: no search rooted by smz_root_gumbel");
+  ON_DEVICE(e);
+  CU(cudaMemcpyAsync(out, e->a.raw_value, (size_t)e->n_trees * (e->a.N + 1) * sizeof(float), cudaMemcpyDeviceToDevice,
+                     (cudaStream_t)stream));
   return SMZ_OK;
 }
 

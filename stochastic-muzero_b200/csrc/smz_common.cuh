@@ -6,6 +6,7 @@
 //   root_prior [B][A] f64   priors of the root children after Dirichlet mixing (f64 in the reference)
 //   minmax [B] float2  MinMaxStats, mcts.py:24-36
 //   hidden [N+1][B][Sp] f32  hidden state of every expanded node: slot 0 = root, slot s+1 = sim s
+//   raw_value [B][N+1] f32   network value of every expanded node by the same slot (Gumbel searches only)
 // Node 0 is the root, 1..A its children, simulation s allocates its children at 1 + A + s*Kmax, so a
 // node's child_base also names the hidden slot of the node (no allocator, no counters).
 #pragma once
@@ -79,6 +80,15 @@ struct SmzArena {
   float one_minus_frac_f32;  // f32(1 - frac), the weak-scalar cast the reference performs
   double frac;
   double alpha;
+  // Gumbel MuZero search (smz_set_search): null / 0 unless a Gumbel search has been rooted on this engine.  The tree
+  // kernels take the mode as a template argument; these columns are only read or written by the Gumbel instantiations.
+  int gumbel;                // 1: the current search uses the Gumbel rule at decision nodes
+  int gumbel_m;              // max_considered_actions
+  double c_visit, c_scale;
+  float* raw_value;          // [B][N+1] the network value of every expanded node, by hidden slot (slot 0 = root)
+  double* gumbel_g;          // [B][A] the root's Gumbels (0 for illegal actions)
+  double* root_logit;        // [B][A] log(prior) - max over legal log(prior) at the root (0 for illegal actions)
+  const int* cv_table;       // [SMZ_MAX_POLICY + 1][max(N, 1)] considered visits of Sequential Halving, T[n][sum of N]
 };
 
 #ifdef __CUDACC__

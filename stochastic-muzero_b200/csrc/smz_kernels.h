@@ -22,6 +22,11 @@ void smz_launch_set_seed(unsigned long long* dst, unsigned long long seed, unsig
 void smz_launch_dirichlet(const SmzArena& a, int n_trees, const uint32_t* legal, cudaStream_t s);
 void smz_launch_select_actions(const SmzArena& a, int n_trees, double temperature, const double* u, int* actions,
                                double* policy, double* stored, cudaStream_t s);
+// Gumbel searches: root values, logits and Gumbels after the root expansion; the action / improved-policy read-out
+void smz_launch_gumbel_root(const SmzArena& a, int n_trees, const float* root_value, int train, const double* given,
+                            cudaStream_t s);
+void smz_launch_read_gumbel(const SmzArena& a, int n_trees, int* actions, double* improved, double* gumbels,
+                            cudaStream_t s);
 
 // ---- network (smz_net_f32.cu / smz_net_bf16.cu) --------------------------------------------------
 // Model shape and the padded fp32 weight image the CUDA-core path reads (built by smz_net_pack).

@@ -85,7 +85,7 @@ __global__ void k_root_expand(SmzArena a, int n_trees, const float* __restrict__
   }
 }
 
-template <int G>
+template <int G, bool GUMBEL>
 __global__ void k_select(SmzArena a, int n_trees, int sim, int* __restrict__ o_slot, int* __restrict__ o_action,
                          int* __restrict__ o_branch) {
   Group<G> g;
@@ -98,10 +98,10 @@ __global__ void k_select(SmzArena a, int n_trees, int sim, int* __restrict__ o_s
   ts.mm = a.minmax[tree];
   const int4 rs = a.stat[(size_t)tree * a.M];
   ts.root = make_int2(rs.x, rs.y);
-  select_phase<G>(g, a, rng, tree, alive, sim, ts, o_slot, o_action, o_branch);
+  select_phase<G, false, GUMBEL>(g, a, rng, tree, alive, sim, ts, o_slot, o_action, o_branch);
 }
 
-template <int G>
+template <int G, bool GUMBEL>
 __global__ void k_expand_backup(SmzArena a, int n_trees, int sim, const float* __restrict__ policy, int pstride,
                                 const float* __restrict__ value, const float* __restrict__ reward) {
   Group<G> g;
@@ -109,13 +109,13 @@ __global__ void k_expand_backup(SmzArena a, int n_trees, int sim, const float* _
   const bool alive = tree < n_trees;
   if (!alive) tree = n_trees - 1;
   const SmzRng rng = smz_make_rng(a);
-  expand_backup_phase(g, a, rng, tree, alive, sim, policy, pstride, value, reward);
+  expand_backup_phase<G, false, GUMBEL>(g, a, rng, tree, alive, sim, policy, pstride, value, reward);
 }
 
 // expansion + backup of simulation `sim` followed by the descent of simulation `sim + 1` for the same
 // tree by the same lanes: one launch per simulation instead of two, the path nodes just updated are
 // re-read from L1/L2.
-template <int G>
+template <int G, bool GUMBEL>
 __global__ void k_backup_select(SmzArena a, int n_trees, int sim) {
   smz_pdl_wait();                 // the network step of `sim` must have landed
   smz_pdl_launch_dependents();    // the next network step may set itself up (barriers, TMEM, weights)
@@ -126,10 +126,11 @@ __global__ void k_backup_select(SmzArena a, int n_trees, int sim) {
   const bool stamp = a.dbg && blockIdx.x == 0 && threadIdx.x == 0;
   if (stamp) a.dbg[0] = clock64();
   const SmzRng rng = smz_make_rng(a);
-  const TreeState ts = expand_backup_phase(g, a, rng, tree, alive, sim, a.out_policy, a.W, a.out_value, a.out_reward);
+  const TreeState ts = expand_backup_phase<G, false, GUMBEL>(g, a, rng, tree, alive, sim, a.out_policy, a.W, a.out_value,
+                                                             a.out_reward);
   __syncwarp();
   if (stamp) a.dbg[1] = clock64();
-  select_phase<G>(g, a, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr);
+  select_phase<G, false, GUMBEL>(g, a, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr);
   if (stamp) { a.dbg[2] = clock64(); a.dbg[3] = a.path_len[tree]; }
 }
 
@@ -148,7 +149,7 @@ __host__ __device__ inline size_t smz_mirror_bytes(int tpb, int M, int A, int n_
   return b + 16;
 }
 
-template <int G>
+template <int G, bool GUMBEL>
 __global__ void k_backup_select_sm(SmzArena a, int n_trees, int sim, int n_tab) {
   extern __shared__ int4 smz_sm_nodes[];
   Group<G> g;
@@ -192,11 +193,11 @@ __global__ void k_backup_select_sm(SmzArena a, int n_trees, int sim, int n_tab) 
   __syncthreads();
   const bool stamp = a.dbg && blockIdx.x == 0 && threadIdx.x == 0;
   if (stamp) a.dbg[0] = clock64();
-  const TreeState ts = expand_backup_phase<G, true>(g, al, rng, tree, alive, sim, a.out_policy, a.W, a.out_value, a.out_reward,
-                                                    sst, slk);
+  const TreeState ts = expand_backup_phase<G, true, GUMBEL>(g, al, rng, tree, alive, sim, a.out_policy, a.W, a.out_value,
+                                                            a.out_reward, sst, slk);
   __syncwarp();
   if (stamp) a.dbg[1] = clock64();
-  select_phase<G, true>(g, al, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr, sst, slk, srp);
+  select_phase<G, true, GUMBEL>(g, al, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr, sst, slk, srp);
   if (stamp) { a.dbg[2] = clock64(); a.dbg[3] = a.path_len[tree]; }
   if (a.dbg) {
     __syncthreads();
@@ -332,6 +333,100 @@ __global__ void k_dirichlet(SmzArena a, int n_trees, const uint32_t* __restrict_
   for (int i = 0; i < a.A; ++i) a.dirichlet[(size_t)tree * a.A + i] /= (sum > 0.0 ? sum : 1.0);
 }
 
+// Root of a Gumbel search, one thread per tree, after k_root_expand: the root's network value into raw_value slot 0, the
+// root logits log(p_a) - max_b log(p_b) over the legal actions (float64 root priors), and one Gumbel per legal action in
+// ascending order (train): given by the caller, or -log(-log u) of the uniform #rank of Philox stream 3; eval: 0.
+__global__ void k_gumbel_root(SmzArena a, int n_trees, const float* __restrict__ root_value, int train,
+                              const double* __restrict__ given) {
+  const int tree = blockIdx.x * blockDim.x + threadIdx.x;
+  if (tree >= n_trees) return;
+  const size_t tb = (size_t)tree * a.M, ro = (size_t)tree * a.A;
+  a.raw_value[(size_t)tree * (a.N + 1)] = root_value[tree];
+  double mx = -__longlong_as_double(0x7ff0000000000000LL);
+  for (int i = 0; i < a.A; ++i)
+    if (a.link[tb + 1 + i].y >= 0) mx = fmax(mx, log(a.root_prior[ro + i]));
+  const unsigned long long seed = a.seed_state[0], tid = a.seed_state[1] + (unsigned long long)tree;
+  unsigned rank = 0;
+  for (int i = 0; i < a.A; ++i) {
+    double gv = 0.0, lg = 0.0;
+    if (a.link[tb + 1 + i].y >= 0) {
+      lg = __dsub_rn(log(a.root_prior[ro + i]), mx);
+      if (train && given) {
+        gv = given[ro + i];
+      } else if (train) {
+        double u = smz_philox_uniform(seed, tid, rank, 3u);
+        u = u > 0.0 ? u : 1.0 / 9007199254740992.0;         // (0, 1): u = 0 would give an infinite Gumbel
+        gv = -log(-log(u));
+      }
+      ++rank;
+    }
+    a.gumbel_g[ro + i] = gv;
+    a.root_logit[ro + i] = lg;
+  }
+}
+
+// Read-out of a Gumbel search, one thread per tree: action = argmax over the legal actions with the most visits of
+// g + logit + sigma (ties: the smaller action); improved policy = softmax over the legal actions of logit + sigma
+// (0 for illegal actions); sigma from the completed Q-values of the root as the descent forms them.
+__global__ void k_read_gumbel(SmzArena a, int n_trees, int* __restrict__ actions, double* __restrict__ improved,
+                              double* __restrict__ gumbels) {
+  const int tree = blockIdx.x * blockDim.x + threadIdx.x;
+  if (tree >= n_trees) return;
+  const size_t tb = (size_t)tree * a.M, ro = (size_t)tree * a.A;
+  const double inf = __longlong_as_double(0x7ff0000000000000LL);
+  int nv[SMZ_MAX_POLICY];
+  double cq[SMZ_MAX_POLICY];
+  bool legal[SMZ_MAX_POLICY];
+  int sn = 0, mn = 0;
+  double spq = 0.0, sp = 0.0;
+  for (int i = 0; i < a.A; ++i) {
+    const int4 st = a.stat[tb + 1 + i];
+    legal[i] = a.link[tb + 1 + i].y >= 0;
+    nv[i] = legal[i] ? st.x : 0;
+    cq[i] = 0.0;
+    if (!legal[i]) continue;
+    sn += st.x;
+    mn = max(mn, st.x);
+    if (st.x > 0) {
+      const float q = __fadd_rn(__int_as_float(st.z), __fmul_rn(a.discount, __fdiv_rn(__int_as_float(st.y), (float)st.x)));
+      const double p = a.root_prior[ro + i];
+      cq[i] = (double)q;
+      spq = __dadd_rn(spq, __dmul_rn(p, (double)q));
+      sp = __dadd_rn(sp, p);
+    }
+  }
+  const double vhat = (double)a.raw_value[(size_t)tree * (a.N + 1)];
+  const double vmix = sn == 0 ? vhat
+                              : __ddiv_rn(__dadd_rn(vhat, __ddiv_rn(__dmul_rn((double)sn, spq), sp)), (double)(sn + 1));
+  double lo = inf, hi = -inf;
+  for (int i = 0; i < a.A; ++i) {
+    if (!legal[i]) continue;
+    if (nv[i] == 0) cq[i] = vmix;
+    lo = fmin(lo, cq[i]);
+    hi = fmax(hi, cq[i]);
+  }
+  const double scale = __dmul_rn(__dadd_rn(a.c_visit, (double)mn), a.c_scale), range = fmax(__dsub_rn(hi, lo), 1e-8);
+  int best = -1;
+  double bs = -inf, zmax = -inf;
+  for (int i = 0; i < a.A; ++i) {
+    if (!legal[i]) continue;
+    const double sigma = __dmul_rn(scale, __ddiv_rn(__dsub_rn(cq[i], lo), range));
+    const double z = __dadd_rn(a.root_logit[ro + i], sigma);
+    cq[i] = z;                                             // from here on: logit + sigma
+    zmax = fmax(zmax, z);
+    const double s = __dadd_rn(__dadd_rn(a.gumbel_g[ro + i], a.root_logit[ro + i]), sigma);
+    if (nv[i] == mn && (best < 0 || s > bs)) { best = i; bs = s; }
+  }
+  if (actions) actions[tree] = best;
+  if (gumbels)
+    for (int i = 0; i < a.A; ++i) gumbels[ro + i] = a.gumbel_g[ro + i];
+  if (!improved) return;
+  double se = 0.0;
+  for (int i = 0; i < a.A; ++i)
+    if (legal[i]) { cq[i] = exp(__dsub_rn(cq[i], zmax)); se = __dadd_rn(se, cq[i]); }
+  for (int i = 0; i < a.A; ++i) improved[ro + i] = legal[i] ? __ddiv_rn(cq[i], se) : 0.0;
+}
+
 template <int G>
 int grid_for(int n_trees, int threads) { return (int)(((long long)n_trees * G + threads - 1) / threads); }
 
@@ -345,6 +440,10 @@ int grid_for(int n_trees, int threads) { return (int)(((long long)n_trees * G + 
     case 16: { constexpr int G = 16; CALL; } break; \
     default: { constexpr int G = 32; CALL; } break; \
   }
+// lane width and search rule (V = a.gumbel) of the per-simulation tree kernels
+#define SMZ_DISPATCH_GV(G_, V_, CALL)                                        \
+  if (V_) { constexpr bool V = true; SMZ_DISPATCH_G(G_, CALL); }             \
+  else { constexpr bool V = false; SMZ_DISPATCH_G(G_, CALL); }
 
 static const int kThreads = 128;
 
@@ -357,14 +456,14 @@ void smz_launch_root_expand(const SmzArena& a, int lanes, int n_trees, const flo
 
 void smz_launch_select(const SmzArena& a, int lanes, int n_trees, int sim, int* o_slot, int* o_action, int* o_branch,
                        cudaStream_t s) {
-  SMZ_DISPATCH_G(lanes, (k_select<G><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(a, n_trees, sim, o_slot,
-                                                                                         o_action, o_branch)));
+  SMZ_DISPATCH_GV(lanes, a.gumbel, (k_select<G, V><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(
+                                       a, n_trees, sim, o_slot, o_action, o_branch)));
 }
 
 void smz_launch_expand_backup(const SmzArena& a, int lanes, int n_trees, int sim, const float* policy, int pstride,
                               const float* value, const float* reward, cudaStream_t s) {
-  SMZ_DISPATCH_G(lanes, (k_expand_backup<G><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(
-                            a, n_trees, sim, policy, pstride, value, reward)));
+  SMZ_DISPATCH_GV(lanes, a.gumbel, (k_expand_backup<G, V><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(
+                                       a, n_trees, sim, policy, pstride, value, reward)));
 }
 
 // shared-memory mirror: node records of (trees per block) trees + tables must fit; SMZ_NO_TREE_SMEM=1 keeps the
@@ -395,17 +494,18 @@ static bool mirror_pays(int blocks) {
 void smz_launch_backup_select(const SmzArena& a, int lanes, int n_trees, int sim, bool pdl, cudaStream_t s) {
   if (smz_tree_mirror_fits(a, lanes) && mirror_pays((n_trees * lanes + kThreads - 1) / kThreads)) {
     const size_t smem = mirror_bytes(a, lanes);
-    SMZ_DISPATCH_G(lanes, (cudaFuncSetAttribute((const void*)k_backup_select_sm<G>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                                (int)smem),
-                           getenv("SMZ_NO_CARVEOUT") ? cudaSuccess :
-                           cudaFuncSetAttribute((const void*)k_backup_select_sm<G>, cudaFuncAttributePreferredSharedMemoryCarveout,
-                                                cudaSharedmemCarveoutMaxShared),
-                           smz_launch(k_backup_select_sm<G>, dim3(grid_for<G>(n_trees, kThreads)), dim3(kThreads), smem, s, pdl,
-                                      a, n_trees, sim, rcp_entries(a))));
+    SMZ_DISPATCH_GV(lanes, a.gumbel,
+                    (cudaFuncSetAttribute((const void*)k_backup_select_sm<G, V>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                          (int)smem),
+                     getenv("SMZ_NO_CARVEOUT") ? cudaSuccess :
+                     cudaFuncSetAttribute((const void*)k_backup_select_sm<G, V>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                                          cudaSharedmemCarveoutMaxShared),
+                     smz_launch(k_backup_select_sm<G, V>, dim3(grid_for<G>(n_trees, kThreads)), dim3(kThreads), smem, s, pdl,
+                                a, n_trees, sim, rcp_entries(a))));
     return;
   }
-  SMZ_DISPATCH_G(lanes, (smz_launch(k_backup_select<G>, dim3(grid_for<G>(n_trees, kThreads)), dim3(kThreads), 0, s, pdl,
-                                    a, n_trees, sim)));
+  SMZ_DISPATCH_GV(lanes, a.gumbel, (smz_launch(k_backup_select<G, V>, dim3(grid_for<G>(n_trees, kThreads)), dim3(kThreads), 0,
+                                               s, pdl, a, n_trees, sim)));
 }
 
 void smz_launch_read_roots(const SmzArena& a, int n_trees, int* visits, float* values, double* priors, float* rewards,
@@ -439,4 +539,14 @@ void smz_launch_set_seed(unsigned long long* dst, unsigned long long seed, unsig
 
 void smz_launch_dirichlet(const SmzArena& a, int n_trees, const uint32_t* legal, cudaStream_t s) {
   k_dirichlet<<<(n_trees + 127) / 128, 128, 0, s>>>(a, n_trees, legal);
+}
+
+void smz_launch_gumbel_root(const SmzArena& a, int n_trees, const float* root_value, int train, const double* given,
+                            cudaStream_t s) {
+  k_gumbel_root<<<(n_trees + 127) / 128, 128, 0, s>>>(a, n_trees, root_value, train, given);
+}
+
+void smz_launch_read_gumbel(const SmzArena& a, int n_trees, int* actions, double* improved, double* gumbels,
+                            cudaStream_t s) {
+  k_read_gumbel<<<(n_trees + 127) / 128, 128, 0, s>>>(a, n_trees, actions, improved, gumbels);
 }

@@ -220,6 +220,91 @@ __device__ __forceinline__ double draw_uniform(const SmzRng& rng, int tree, int 
 }
 
 // ------------------------------------------------------------------------------------------------
+// Gumbel MuZero decision rule (Danihelka et al., ICLR 2022; smz_set_search in include/smz.h), one lane per child.
+// float64 sum over the lanes in ascending order, as a sequential loop adds; lanes that take no part hold +0.0, which
+// leaves the sum unchanged (a sum that starts at +0.0 never becomes -0.0 under round-to-nearest).
+template <int G>
+__device__ __forceinline__ double seq_sum_f64(const Group<G>& g, double x) {
+  double acc = 0.0;
+#pragma unroll
+  for (int i = 0; i < G; ++i) acc = __dadd_rn(acc, g.bcast(x, i));
+  return acc;
+}
+
+// sigma_i = (c_visit + max N) * c_scale * r_i of the completed Q-values, for the lanes `on` (the node's existing
+// children: visit count n, prior p, q = reward + discount * value() in float32); the node's own network value is vhat.
+template <int G>
+__device__ __forceinline__ double gumbel_sigma(const Group<G>& g, const SmzArena& a, bool on, int n, double p, float q,
+                                               double vhat, int& sum_n) {
+  int sn = on ? n : 0, mn = sn;
+#pragma unroll
+  for (int off = G / 2; off > 0; off >>= 1) {
+    sn += __shfl_xor_sync(FULL, sn, off, G);
+    mn = max(mn, __shfl_xor_sync(FULL, mn, off, G));
+  }
+  const bool vis = on && n > 0;
+  const double qd = (double)q;
+  const double spq = seq_sum_f64(g, vis ? __dmul_rn(p, qd) : 0.0);
+  const double sp = seq_sum_f64(g, vis ? p : 0.0);
+  // v_mix = (vhat + sum N * (sum p q) / (sum p)) / (sum N + 1), left to right
+  const double vmix = sn == 0 ? vhat
+                              : __ddiv_rn(__dadd_rn(vhat, __ddiv_rn(__dmul_rn((double)sn, spq), sp)), (double)(sn + 1));
+  const double cq = vis ? qd : vmix;
+  const double inf = __longlong_as_double(0x7ff0000000000000LL);
+  double lo = on ? cq : inf, hi = on ? cq : -inf;
+#pragma unroll
+  for (int off = G / 2; off > 0; off >>= 1) {
+    lo = fmin(lo, __shfl_xor_sync(FULL, lo, off, G));
+    hi = fmax(hi, __shfl_xor_sync(FULL, hi, off, G));
+  }
+  const double r = __ddiv_rn(__dsub_rn(cq, lo), fmax(__dsub_rn(hi, lo), 1e-8));
+  sum_n = sn;
+  return on ? __dmul_rn(__dmul_rn(__dadd_rn(a.c_visit, (double)mn), a.c_scale), r) : 0.0;
+}
+
+// The child a decision node descends to under the Gumbel rule; no uniform is drawn.  Root (lanes = actions, `act` = a
+// legal child): argmax over the children whose visit count is the considered count T[min(m, |L|)][sum N] of
+// max(-1e9, g + logit + sigma).  Elsewhere: argmax of pi'_i - N_i / (1 + sum N), pi' = softmax-weighted priors
+// p_i exp(sigma_i - max sigma) / sum.  Ties go to the smaller action; a root with no child at the considered count
+// (the schedule rules it out) takes its first legal child.
+template <int G>
+__device__ __forceinline__ int gumbel_pick(const Group<G>& g, const SmzArena& a, int tree, bool going, bool act, bool root,
+                                           int4 st, double prior_root, double gum, double lgt, int cbase, int width) {
+  const int slot = (root || !going) ? 0 : (cbase - 1 - a.A) / a.Kmax + 1;     // a group that stopped reads slot 0
+  const double vhat = (double)a.raw_value[(size_t)tree * (a.N + 1) + slot];
+  const double p = root ? prior_root : (double)__int_as_float(st.w);
+  float q = 0.f;
+  if (act && st.x > 0) {
+    const float val = smz_div_r32(__int_as_float(st.y), (float)st.x, a.rcp32[st.x]);
+    q = __fadd_rn(__int_as_float(st.z), __fmul_rn(a.discount, val));
+  }
+  int sum_n;
+  const double sigma = gumbel_sigma(g, a, act, st.x, p, q, vhat, sum_n);
+  const double inf = __longlong_as_double(0x7ff0000000000000LL);
+  double score = -inf;
+  int best = act ? g.gl : 64;
+  if (root) {
+    const int n_cons = min(a.gumbel_m, width);
+    const int considered = a.cv_table[n_cons * a.N + min(sum_n, a.N - 1)];
+    if (act && st.x == considered) score = fmax(-1e9, __dadd_rn(__dadd_rn(gum, lgt), sigma));
+  } else {
+    double ms = act ? sigma : -inf;
+#pragma unroll
+    for (int off = G / 2; off > 0; off >>= 1) ms = fmax(ms, __shfl_xor_sync(FULL, ms, off, G));
+    const double w = act ? __dmul_rn(p, exp(__dsub_rn(sigma, ms))) : 0.0;
+    const double sw = seq_sum_f64(g, w);
+    if (act) score = __dsub_rn(__ddiv_rn(w, sw), __ddiv_rn((double)st.x, (double)(1 + sum_n)));
+  }
+#pragma unroll
+  for (int off = G / 2; off > 0; off >>= 1) {
+    const double os = __shfl_xor_sync(FULL, score, off, G);
+    const int ob = __shfl_xor_sync(FULL, best, off, G);
+    if (os > score || (os == score && ob < best)) { score = os; best = ob; }
+  }
+  return best < G ? best : 0;
+}
+
+// ------------------------------------------------------------------------------------------------
 // Per-tree state that flows from the backup of one simulation into the descent of the next.  The fused
 // kernel keeps it in registers; the stand-alone kernels load / store it.
 struct TreeState {
@@ -232,7 +317,7 @@ struct TreeState {
 // while descending, so the backup needs ONE round trip (the record) instead of two (index -> stat).
 // The tree is appended to the per-branch row list of the simulation, from which the network step tiles its leaves.
 // Called by every thread of the block: the row reservation below synchronises the block.
-template <int G, bool MIRROR = false>
+template <int G, bool MIRROR = false, bool GUMBEL = false>
 __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& a, const SmzRng& rng, int tree, bool alive,
                                              int sim, TreeState ts, int* __restrict__ o_slot, int* __restrict__ o_action,
                                              int* __restrict__ o_branch, const int4* __restrict__ sst = nullptr,
@@ -254,6 +339,14 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
   bool going = alive;
   // the Dirichlet-mixed root priors are f64 and only used at depth 0: one load, before the loop
   const double prior0 = (alive && g.gl < a.A) ? (srp ? srp[g.gl] : a.root_prior[(size_t)tree * a.A + g.gl]) : 0.0;
+  // Gumbel rule: the root's Gumbels and logits, read from the arena (L2) by both kernels
+  double gum0 = 0.0, lgt0 = 0.0;
+  if constexpr (GUMBEL) {
+    if (alive && g.gl < a.A) {
+      gum0 = a.gumbel_g[(size_t)tree * a.A + g.gl];
+      lgt0 = a.root_logit[(size_t)tree * a.A + g.gl];
+    }
+  }
   // Every group that is still descending is at depth == level, so the node kind (and the child count) is uniform
   // across the warp: plain uniform branches instead of votes, loads and draws without divergent regions.
   int level = 0;
@@ -284,15 +377,15 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
         width = __popc(lm);
       }
       if (!act) { st = make_int4(0, 0, 0, 0); lk = make_int2(0, 0); }
-      pbc = chance ? 0.0 : a.pbc[going ? parent_visit : 0];     // plain load: the table lives in shared memory
-      u = draw_uniform(rng, tree, chance ? cursor : cursor + rank, going && (chance || act));
+      pbc = (GUMBEL || chance) ? 0.0 : a.pbc[going ? parent_visit : 0];     // plain load: the table lives in shared memory
+      u = draw_uniform(rng, tree, chance ? cursor : cursor + rank, going && (chance || (!GUMBEL && act)));
     } else {
       // the node records are still in flight: the draws are taken by lane index without waiting for them, and child
       // j gets the draw of lane `rank` by a shuffle.  With a tape only lanes 0..|L|-1 draw, so the tape is read
       // exactly where the search reads it.
-      pbc = chance ? 0.0 : a.pbc[going ? parent_visit : 0];
-      bool want = going && (chance || act);
-      if (root && rng.mode) {    // every lane takes part in the ballot (no short-circuit around it)
+      pbc = (GUMBEL || chance) ? 0.0 : a.pbc[going ? parent_visit : 0];
+      bool want = going && (chance || (!GUMBEL && act));     // a Gumbel decision node draws nothing
+      if (!GUMBEL && root && rng.mode) {    // every lane takes part in the ballot (no short-circuit around it)
         const int n_legal = __popc(g.ballot(act && lk.y >= 0));
         want = want && g.gl < n_legal;
       }
@@ -326,7 +419,9 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
       pk = pk < nch ? pk : nch - 1;
       if (chance) { pick = pk; cursor += going ? 1 : 0; }
     }
-    if (!chance) {
+    if (GUMBEL && !chance) {
+      pick = gumbel_pick(g, a, tree, going, act, root, st, prior0, gum0, lgt0, cbase, width);
+    } else if (!chance) {
       // decision node: argmax of ucb_score, one fresh uniform per child (mcts.py:235-243, T3/T5/T6)
       double score = -__longlong_as_double(0x7ff0000000000000LL);
       int best = -1;
@@ -448,7 +543,7 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
 }
 
 // ------------------------------------------------------------------------------------------------
-template <int G, bool MIRROR = false>
+template <int G, bool MIRROR = false, bool GUMBEL = false>
 __device__ __forceinline__ TreeState expand_backup_phase(const Group<G>& g, const SmzArena& a, const SmzRng& rng, int tree,
                                                          bool alive, int sim, const float* __restrict__ policy,
                                                          int pstride, const float* __restrict__ value,
@@ -490,6 +585,7 @@ __device__ __forceinline__ TreeState expand_backup_phase(const Group<G>& g, cons
     a.link[tb + leaf].x = cb;
     a.ucursor[tree] = cursor;
     if (branch) reinterpret_cast<int*>(a.stat + tb + leaf)[2] = __float_as_int(rew);     // Node.reward of the leaf
+    if constexpr (GUMBEL) a.raw_value[(size_t)tree * (a.N + 1) + sim + 1] = v;        // the leaf's slot is sim + 1
     if constexpr (MIRROR) {
       slk[leaf].x = cb;
       if (branch) sst[leaf].z = __float_as_int(rew);

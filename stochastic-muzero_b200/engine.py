@@ -151,6 +151,15 @@ class SearchEngine:
         self.paper_alternation = None         # pattern of the current search and of the uploaded player tables
         self._next_paper = bool(paper_alternation)
         self._apply_node_pattern()
+        self.gumbel = False                   # search policy of the following root steps (set_search)
+
+    def set_search(self, gumbel: bool, max_considered_actions: int = 16, c_visit: float = 50.0, c_scale: float = 0.1):
+        """Search policy of the searches rooted from now on (smz_set_search in include/smz.h): the reference's pUCT
+        (``gumbel=False``, rooted by ``root``) or Gumbel MuZero (rooted by ``root_gumbel``, read out by ``read_gumbel``).
+        Invalid values raise ValueError."""
+        self._check(self.lib.smz_set_search(self._h, _lib.SEARCH_GUMBEL if gumbel else _lib.SEARCH_PUCT,
+                                            int(max_considered_actions), float(c_visit), float(c_scale)))
+        self.gumbel = bool(gumbel)
 
     def set_node_pattern(self, paper_alternation: bool):
         """Node pattern of the searches started by the following root() calls; a search already rooted keeps its own."""
@@ -253,6 +262,32 @@ class SearchEngine:
         self._apply_node_pattern()
         self._check(self.lib.smz_root_legal(self._h, n, self._ptr(obs_t), self._ptr(pol_t), self._ptr(rtp),
                                             self._ptr(words), int(bool(train)), self._ptr(dr), self._stream))
+        self.n_trees = n
+        self.generation += 1
+
+    def root_gumbel(self, obs=None, root_policy=None, root_value=None, root_to_play=None, train=True, gumbels=None,
+                    legal=None):
+        """Root step of a Gumbel search (smz_root_gumbel): like ``root``, without Dirichlet noise; ``root_value`` [n]
+        (the network value of each root) goes with ``root_policy``; ``gumbels``: float64 [n, A] recorded Gumbels, or None
+        to draw them on the device (train) — with ``train=False`` every Gumbel is 0."""
+        src = obs if obs is not None else root_policy
+        n = int(src.shape[0])
+        words = None
+        if legal is not None:
+            words = pack_legal(self.to_device(legal_rows(legal, n, self.A), torch.bool))
+            self._keep["legal"] = words
+        obs_t = self._dev(obs, torch.float32, "obs")
+        pol_t = None
+        if root_policy is not None:
+            pol_t = self._pad_policy(self._dev(root_policy, torch.float32, "root_policy"), "root_policy")
+        val_t = self._dev(None if root_value is None else torch.as_tensor(root_value).reshape(-1), torch.float32,
+                          "root_value")
+        rtp = self._dev(root_to_play, torch.int32, "root_to_play")
+        g_t = self._dev(gumbels, torch.float64, "gumbels")
+        self._apply_node_pattern()
+        self._check(self.lib.smz_root_gumbel(self._h, n, self._ptr(obs_t), self._ptr(pol_t), self._ptr(val_t),
+                                             self._ptr(rtp), self._ptr(words), int(bool(train)), self._ptr(g_t),
+                                             self._stream))
         self.n_trees = n
         self.generation += 1
 
@@ -366,6 +401,22 @@ class SearchEngine:
                "stored_policy": self._new(n, A, dtype=torch.float64)}
         self._check(self.lib.smz_select_actions(self._h, float(temperature), self._ptr(u), self._ptr(out["actions"]),
                                                 self._ptr(out["policy"]), self._ptr(out["stored_policy"]), self._stream))
+        return out
+
+    def read_gumbel(self):
+        """Read-out of a Gumbel search (smz_read_gumbel): dict(actions int32[n], improved_policy f64[n, A],
+        gumbels f64[n, A])."""
+        n, A = self.n_trees, self.A
+        out = {"actions": self._new(n, dtype=torch.int32), "improved_policy": self._new(n, A, dtype=torch.float64),
+               "gumbels": self._new(n, A, dtype=torch.float64)}
+        self._check(self.lib.smz_read_gumbel(self._h, self._ptr(out["actions"]), self._ptr(out["improved_policy"]),
+                                             self._ptr(out["gumbels"]), self._stream))
+        return out
+
+    def read_raw_values(self):
+        """Network value of every expanded node of a Gumbel search by hidden slot: float32 [n, N + 1]."""
+        out = self._new(self.n_trees, self.N + 1, dtype=torch.float32)
+        self._check(self.lib.smz_read_raw_values(self._h, self._ptr(out), self._stream))
         return out
 
     def read_hidden(self, slot):

@@ -222,6 +222,12 @@ class BatchedRoots:
             self._engine.raise_for_error(self.host()["error"])
         return self
 
+    def gumbel(self):
+        """Read-out of a Gumbel search (``Monte_carlo_tree_search(..., gumbel=True)``): dict(actions int32[B] — the
+        action to play, improved_policy float64[B, A] — the policy target, 0 for illegal actions)."""
+        out = self._live().read_gumbel()
+        return {"actions": out["actions"], "improved_policy": out["improved_policy"]}
+
     def select_actions(self, temperature: float = 0.0, uniforms=None):
         """Batched Game.policy_step / store_search_statistics (game.py:179-235) on the device:
         dict(actions, policy, stored_policy); root values are `self.root_values`."""
@@ -261,7 +267,8 @@ class Monte_carlo_tree_search():
                  maxium_action_sample=2,
                  number_of_player=1,
                  custom_loop=None,
-                 *, net="tc32", device=None, seed=None, max_batch=None, tree_id_offset=None, paper_alternation=False):
+                 *, net="tc32", device=None, seed=None, max_batch=None, tree_id_offset=None, paper_alternation=False,
+                 gumbel=False, max_considered_actions=16, c_visit=50.0, c_scale=0.1):
         """Same nine arguments as the reference (:76-85).  Keyword-only extras: ``net`` — the fused MLP network step:
         "tc32" (default: the reference's fp32 precision on the tensor cores, fp16 hi/lo split operands, 1e-5 against the
         reference's inference), "fp32" (the same precision on CUDA cores), "bf16" / "f16" (throughput modes with
@@ -272,9 +279,17 @@ class Monte_carlo_tree_search():
         numpy identically still draw different noise; default rank * max_batch when torch.distributed is
         initialised, else 0), ``paper_alternation`` (search with the Stochastic MuZero node alternation — decision,
         chance, decision, ... from the root, so afterstate_dynamics sees states and dynamics sees afterstates —
-        instead of the reference's depth pattern F,F,T,T,...; default off: the reference's search)."""
+        instead of the reference's depth pattern F,F,T,T,...; default off: the reference's search), ``gumbel`` (search
+        with Gumbel MuZero — Gumbel-Top-k and Sequential Halving at the root, completed-Q selection below — instead of
+        pUCT with Dirichlet noise, with ``max_considered_actions`` / ``c_visit`` / ``c_scale``; read its action and
+        policy target with ``BatchedRoots.gumbel()``; default off: the reference's search)."""
         self._net, self._device, self._seed, self._max_batch = net, device, seed, max_batch
         self._paper = bool(paper_alternation)
+        self.gumbel = bool(gumbel)
+        self.max_considered_actions, self.c_visit, self.c_scale = int(max_considered_actions), float(c_visit), float(c_scale)
+        if not 1 <= self.max_considered_actions <= 32 or not (0 <= self.c_visit < float("inf")) or \
+                not (0 <= self.c_scale < float("inf")):
+            raise ValueError("max_considered_actions must be in [1, 32], c_visit and c_scale finite and >= 0")
         self._tree_id_offset = tree_id_offset
         self._engines = {}
         self._weights_seen = {}
@@ -328,7 +343,8 @@ class Monte_carlo_tree_search():
         section = config.get("monte_carlo_tree_search", config)
         keys = ("pb_c_base", "pb_c_init", "discount", "root_dirichlet_alpha", "root_exploration_fraction",
                 "num_simulations", "maxium_action_sample", "number_of_player", "custom_loop")
-        return cls(**{k: section[k] for k in keys if k in section}, **extras)
+        opts = {k: section[k] for k in ("gumbel", "max_considered_actions", "c_visit", "c_scale") if k in section}
+        return cls(**{k: section[k] for k in keys if k in section}, **{**opts, **extras})
 
     def _base_seed(self):
         if self._seed is None:
@@ -347,6 +363,8 @@ class Monte_carlo_tree_search():
                                paper_alternation=self._paper)
             self._engines[key] = eng
             self._weights_seen.pop(key, None)
+        if self.gumbel or eng.gumbel:      # host-side setting, applied by the next root step
+            eng.set_search(self.gumbel, self.max_considered_actions, self.c_visit, self.c_scale)
         return eng, key
 
     @staticmethod
@@ -435,7 +453,10 @@ class Monte_carlo_tree_search():
                 self._weights_seen[key] = ver
         obs = eng.to_device(obs, torch.float32)      # the observations' host-to-device copy is enqueued first
         eng.set_seed(self._next_seed(), self._offset(obs.shape[0]))
-        eng.root(obs=obs, root_to_play=root_to_play, train=train, **_legal_kw(legal_actions))
+        if self.gumbel:
+            eng.root_gumbel(obs=obs, root_to_play=root_to_play, train=train, **_legal_kw(legal_actions))
+        else:
+            eng.root(obs=obs, root_to_play=root_to_play, train=train, **_legal_kw(legal_actions))
         eng.simulate(self.num_simulations)
         roots = BatchedRoots(eng, eng.read_roots())
         return roots.raise_if_failed() if check else roots
@@ -497,14 +518,18 @@ class Monte_carlo_tree_search():
         """Host-model mode: tree kernels on the GPU, the five inference methods called back per
         simulation (:182, :198, :271-286)."""
         h0 = model.representation_function_inference(observation)
-        policy, _value = model.prediction_function_inference(h0)
+        policy, value0 = model.prediction_function_inference(h0)
         policy = np.asarray(policy, dtype=np.float32).reshape(1, -1)
         A = policy.shape[1]
         eng, _ = self._engine("external", 1, A, getattr(model, "chance_dimension", A))
         eng.set_seed(self._next_seed(), self._offset(1))
         legal = None if legal_actions is None else _legal_row(legal_actions, A)
-        eng.root(root_policy=policy, root_to_play=torch.tensor([to_play], dtype=torch.int32), train=train,
-                 **_legal_kw(legal))
+        if self.gumbel:
+            eng.root_gumbel(root_policy=policy, root_value=np.array([value0], dtype=np.float32).reshape(1),
+                            root_to_play=torch.tensor([to_play], dtype=torch.int32), train=train, **_legal_kw(legal))
+        else:
+            eng.root(root_policy=policy, root_to_play=torch.tensor([to_play], dtype=torch.int32), train=train,
+                     **_legal_kw(legal))
         hidden = {0: h0}
         for sim in range(self.num_simulations):
             slot, action, branch = (int(t.item()) for t in eng.select(sim))

@@ -88,7 +88,11 @@ class SelfPlay:
         for t in range(T):
             legal = env.legal_mask() if hasattr(env, "legal_mask") else None
             roots = self.mcts.run_batch(obs, self.model, train=train, legal_actions=legal)   # one move of every game
-            pick = roots.select_actions(temperature)                                # game.py:223-235 on the device
+            if getattr(self.mcts, "gumbel", False):      # Gumbel search: its action, its improved policy as the target
+                g = roots.gumbel()
+                pick = {"actions": g["actions"], "stored_policy": g["improved_policy"]}
+            else:
+                pick = roots.select_actions(temperature)                            # game.py:223-235 on the device
             buf["observations"][t], buf["actions"][t] = obs, pick["actions"]
             buf["child_visits"][t], buf["root_values"][t] = pick["stored_policy"], roots.root_values
             obs, reward, done = env.step(pick["actions"])
@@ -104,7 +108,8 @@ def reanalyse(mcts, model, observations: torch.Tensor, chunk: int = 16384, train
     observations of old games with the current weights.  Every stored position is an independent tree, so
     the [T, B, ...] trajectory block is simply flattened into large batches for the engine.
     ``legal_actions``: optional bool mask [T, B, A] of the stored positions' legal actions.
-    Returns fresh targets: child_visits [T, B, A] (stored visit policy) and root_values [T, B]."""
+    Returns fresh targets: child_visits [T, B, A] (stored visit policy; the improved policy of a Gumbel search) and
+    root_values [T, B]."""
     T, B = observations.shape[:2]
     flat = observations.reshape((T * B,) + tuple(observations.shape[2:]))
     legal = None if legal_actions is None else legal_actions.reshape(T * B, -1)
@@ -112,7 +117,10 @@ def reanalyse(mcts, model, observations: torch.Tensor, chunk: int = 16384, train
     for lo in range(0, T * B, chunk):
         roots = mcts.run_batch(flat[lo:lo + chunk], model, train=train,
                                legal_actions=None if legal is None else legal[lo:lo + chunk])
-        visits.append(roots.select_actions(0.0)["stored_policy"])
+        if getattr(mcts, "gumbel", False):         # the Gumbel search's policy target
+            visits.append(roots.gumbel()["improved_policy"])
+        else:
+            visits.append(roots.select_actions(0.0)["stored_policy"])
         values.append(roots.root_values.clone())
     child_visits = torch.cat(visits)
     return {"child_visits": child_visits.reshape(T, B, -1), "root_values": torch.cat(values).reshape(T, B)}
