@@ -188,6 +188,32 @@ enum {
 };
 int smz_set_search(smz_engine* e, int32_t policy, int32_t max_considered, double c_visit, double c_scale);
 
+/* The Sequential Halving schedules of every budget b in [0, num_simulations], as the Gumbel search uses them (host
+ * memory, no engine, no GPU): out int32[num_simulations + 1][33][max(num_simulations, 1)], entry (b, n, i) = the visit
+ * count the root child of simulation i must have when n actions are considered and the budget is b (i < b; the rest 0). */
+int smz_sequential_halving_table(int32_t num_simulations, int32_t* out);
+
+/* Per-tree simulation budgets and exploration flags of the NEXT root step (smz_root, smz_root_legal or smz_root_gumbel),
+ * which must root the same n_trees.  budget_dev: int32[n_trees] in [0, N], or NULL (every tree N); explore_dev:
+ * uint8[n_trees] (0 / non-zero), or NULL (every tree follows the root step's `train`).  Both are copied on `stream`: the
+ * caller's buffers may be reused once the call is enqueued.  A root step not preceded by this call uses N and `train`
+ * for every tree.
+ * Tree b then behaves bit for bit as the reference's search with num_simulations = budget[b]: same arena, same draws,
+ * same min-max bounds, record entries and read-out.  For s >= budget[b] it takes no part in simulation s: no descent,
+ * no draw, no row for the network step, no expansion, no backup, no record entry, no depth statistic.  Per tree:
+ *   - the exploration flag replaces `train` for that tree's root noise: Dirichlet in pUCT mode, Gumbels in Gumbel mode
+ *     (a tree with the flag off is a train = 0 search, with it on a train = 1 search);
+ *   - pUCT: no Dirichlet noise for a tree whose budget is 0 (:215-216 per tree); as with train = 0, no noise is drawn
+ *     or recorded for a tree without noise;
+ *   - Gumbel: the root follows the Sequential Halving schedule of its own budget, T_budget[min(m, |L|)][sum N]
+ *     (smz_sequential_halving_table); a budget-0 tree still draws its Gumbels.
+ * A budget outside [0, N] raises error flag 4 (smz_read_roots) and that tree is searched with N.  Budgets live in an
+ * arena column written by the root step: searches with different budgets replay the same captured smz_simulate graph.
+ * smz_simulate(n) still runs n simulation steps; a caller that knows the largest budget runs only that many (a step in
+ * which no tree takes part costs its launches only: every network kernel leaves at once when it has no rows). */
+int smz_set_root_budgets(smz_engine* e, int32_t n_trees, const int32_t* budget_dev, const uint8_t* explore_dev,
+                         void* stream);
+
 /* Tape inputs (rng_mode == SMZ_RNG_TAPE): uniforms_dev is double[n_trees][stride]. */
 int smz_set_uniform_tape(smz_engine* e, const double* uniforms_dev, int32_t stride);
 
@@ -234,7 +260,9 @@ int smz_simulate(smz_engine* e, int32_t n_sims, void* stream);
 
 /* pUCT / chance descent of simulation `sim` (:262-267).  Optional outputs, each [n_trees] or NULL:
  * leaf_parent_slot (hidden-state slot of search_path[-2]), leaf_action (history[-1]),
- * leaf_branch (0 = afterstate pair :339-342, 1 = dynamics pair :333-337). */
+ * leaf_branch (0 = afterstate pair :339-342, 1 = dynamics pair :333-337).  A tree without simulation `sim` (its budget
+ * is used up, smz_set_root_budgets) gets leaf_parent_slot -1; its other outputs are unspecified, and
+ * smz_expand_backup ignores its inputs. */
 int smz_select(smz_engine* e, int32_t sim, int32_t* leaf_parent_slot_dev, int32_t* leaf_action_dev,
                int32_t* leaf_branch_dev, void* stream);
 /* internal network on the leaves chosen by the last smz_select */
@@ -264,7 +292,8 @@ int smz_net_eval(smz_engine* e, int32_t which, int32_t n_rows, const float* in_d
  * visits int32[n][A], root_values float[n] (= Node.value() of the root), priors double[n][A],
  * rewards float[n][A]; error_dev int32[1] = the search's error flag (0 ok, 1 uniform tape exhausted,
  * 2 NaN / all-zero policy met during an expansion — where np.random.choice raises in the reference,
- * monte_carlo_tree_search.py:208/:294, 3 a legal-action mask of smz_root_legal was empty or had a bit >= A set), delivered with the same read-out so that the host needs no extra
+ * monte_carlo_tree_search.py:208/:294, 3 a legal-action mask of smz_root_legal was empty or had a bit >= A set,
+ * 4 a budget of smz_set_root_budgets was outside [0, N]), delivered with the same read-out so that the host needs no extra
  * synchronisation to learn about it.  Any pointer may be NULL. */
 int smz_read_roots(smz_engine* e, int32_t* visits_dev, float* root_values_dev, double* priors_dev,
                    float* rewards_dev, int32_t* error_dev, void* stream);
@@ -291,12 +320,14 @@ int smz_export_tree(smz_engine* e, int32_t tree, smz_tree_host* out, void* strea
 int smz_read_hidden(smz_engine* e, int32_t slot, float* out_dev, void* stream);
 /* record == 1: network outputs of every simulation so a run can be replayed by the CPU oracle.
  * policy float[n][N][policy_stride], value/reward float[n][N], branch int8[n][N],
- * dirichlet double[n][A], root_policy float[n][policy_stride]. */
+ * dirichlet double[n][A], root_policy float[n][policy_stride].  Entries of simulations s >= budget[b] of a tree are
+ * not written (they hold whatever an earlier search left there). */
 int smz_read_record(smz_engine* e, float* policy_dev, float* value_dev, float* reward_dev,
                     int8_t* branch_dev, double* dirichlet_dev, float* root_policy_dev, void* stream);
 /* Synchronises `stream`.  Mean leaf depth and kernel-launch count of the last smz_root + smz_simulate, and the
- * number of kernels this engine has launched since smz_create (bench bookkeeping: `gpu_launches`).  Returns
- * SMZ_E_CAPACITY / SMZ_E_STATE / SMZ_E_INVALID_ARG when the last search raised its error flag 1 / 2 / 3 (see
+ * number of kernels this engine has launched since smz_create (bench bookkeeping: `gpu_launches`).  The depth is
+ * averaged over the simulations actually run, sum over the trees of min(budget, simulations done).  Returns
+ * SMZ_E_CAPACITY / SMZ_E_STATE / SMZ_E_INVALID_ARG when the last search raised its error flag 1 / 2 / 3 or 4 (see
  * smz_read_roots). */
 int smz_stats(smz_engine* e, double* mean_leaf_depth, int64_t* launches, int64_t* launches_total, void* stream);
 

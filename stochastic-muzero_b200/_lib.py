@@ -62,6 +62,8 @@ SIGNATURES = {
     "smz_root": (C.c_int, [_P, C.c_int32, _P, _P, _P, C.c_int32, _P, _P]),
     "smz_root_legal": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "smz_set_search": (C.c_int, [_P, C.c_int32, C.c_int32, C.c_double, C.c_double]),
+    "smz_sequential_halving_table": (C.c_int, [C.c_int32, _P]),
+    "smz_set_root_budgets": (C.c_int, [_P, C.c_int32, _P, _P, _P]),
     "smz_root_gumbel": (C.c_int, [_P, C.c_int32, _P, _P, _P, _P, _P, C.c_int32, _P, _P]),
     "smz_read_gumbel": (C.c_int, [_P, _P, _P, _P, _P]),
     "smz_read_raw_values": (C.c_int, [_P, _P, _P]),

@@ -84,9 +84,12 @@ def is_batched_backend(model) -> bool:
     return all(callable(getattr(model, n, None)) for n in BATCHED_METHODS)
 
 
-def run_search(engine, backend, observations, n_sims, root_to_play=None, train=True, legal=None):
+def run_search(engine, backend, observations, n_sims, root_to_play=None, train=True, legal=None, budget=None,
+               explore=None):
     """Drive one batched search with an external batched network: the engine's select / expand_backup
-    hooks around torch calls.  ``legal``: optional legal-action mask [B, A] of the roots (SearchEngine.root).
+    hooks around torch calls.  ``legal``: optional legal-action mask [B, A] of the roots (SearchEngine.root);
+    ``budget`` / ``explore``: optional per-tree simulation budgets and exploration flags (SearchEngine.root): the search
+    runs max(budget) simulations, and a tree without simulation s (select's parent slot -1) is not sent to the model.
     Returns the hidden-state store [N+1, B, ...] (slot-major like the arena's)."""
     dev = torch.device("cuda", engine.device)
     h0 = backend.representation(observations)
@@ -95,6 +98,11 @@ def run_search(engine, backend, observations, n_sims, root_to_play=None, train=T
     store = torch.zeros((n_sims + 1,) + tuple(h0.shape), dtype=h0.dtype, device=dev)
     store[0] = h0
     kw = {} if legal is None else {"legal": legal}
+    if budget is not None:
+        kw["budget"] = budget
+        n_sims = min(n_sims, int(budget.max()) if budget.numel() else 0)     # one host read per search
+    if explore is not None:
+        kw["explore"] = explore
     if engine.gumbel:          # the Gumbel search completes Q-values with each node's network value, the root's too
         engine.root_gumbel(root_policy=policy.float(), root_value=value.float().reshape(-1), root_to_play=root_to_play,
                            train=train, **kw)
@@ -104,12 +112,13 @@ def run_search(engine, backend, observations, n_sims, root_to_play=None, train=T
     rows = torch.arange(B, device=dev)
     for sim in range(n_sims):
         slot, action, branch = engine.select(sim)
-        parent = store[slot.long(), rows]
+        live = slot >= 0                           # trees whose budget is used up take no part in this simulation
+        parent = store[slot.long().clamp(min=0), rows]
         is_dyn = branch.bool()
         pol = torch.zeros(B, W, dtype=torch.float32, device=dev)
         val = torch.zeros(B, dtype=torch.float32, device=dev)
         rew = torch.zeros(B, dtype=torch.float32, device=dev)
-        i_a, i_d = (~is_dyn).nonzero(as_tuple=True)[0], is_dyn.nonzero(as_tuple=True)[0]
+        i_a, i_d = (live & ~is_dyn).nonzero(as_tuple=True)[0], (live & is_dyn).nonzero(as_tuple=True)[0]
         if i_a.numel():
             h = backend.afterstate_dynamics(parent[i_a], action[i_a])
             p, v = backend.afterstate_prediction(h)

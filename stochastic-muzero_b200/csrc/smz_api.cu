@@ -79,6 +79,9 @@ struct smz_engine {
   // search policy of the next root (smz_set_search), copied into the arena (a.gumbel, a.gumbel_m, a.c_visit, a.c_scale)
   int32_t search_policy, gumbel_m;
   double c_visit, c_scale;
+  // smz_set_root_budgets: the next root step takes the staged budgets (a.budget) / exploration flags (a.explore_in) of
+  // pend_trees trees; has_budgets: the current search was given budgets (smz_stats' depth average)
+  int pend_budget, pend_explore, pend_trees, has_budgets;
 };
 
 const char* smz_last_error(void) { return g_err; }
@@ -157,6 +160,7 @@ int smz_create(const smz_config* cfg, smz_engine** out) {
   memset(&e->a, 0, sizeof(e->a));
   e->img32_buf = nullptr; e->blob_buf = nullptr; e->bf16 = nullptr; e->tc32 = nullptr; e->vision = nullptr;
   e->n_trees = 0; e->sims_done = 0; e->have_weights = 0; e->launches = 0; e->launches_total = 0;
+  e->pend_budget = e->pend_explore = e->pend_trees = e->has_budgets = 0;
   e->use_pdl = getenv("SMZ_NO_PDL") ? 0 : 1;
   e->graph_exec = nullptr; e->graph_trees = e->graph_sims = e->graph_first = -1; e->capture_stream = nullptr;
 
@@ -192,7 +196,7 @@ int smz_create(const smz_config* cfg, smz_engine** out) {
   cudaError_t r = cudaSuccess;
 #define ALLOC(ptr, n) if (r == cudaSuccess) r = dev_alloc(e, &(ptr), (n))
   ALLOC(a.stat, B * M); ALLOC(a.link, B * M); ALLOC(a.root_prior, B * a.A); ALLOC(a.minmax, B);
-  ALLOC(a.ucursor, B); ALLOC(a.root_to_play, B); ALLOC(a.path, B * a.path_stride); ALLOC(a.path_len, B);
+  ALLOC(a.ucursor, B); ALLOC(a.root_to_play, B); ALLOC(a.budget, B); ALLOC(a.explore_in, B); ALLOC(a.path, B * a.path_stride); ALLOC(a.path_len, B);
   ALLOC(a.leaf_node, B); ALLOC(a.leaf_slot, B); ALLOC(a.leaf_action, B); ALLOC(a.leaf_branch, B);
   ALLOC(a.branch_count, (size_t)(a.N + 1) * 2); ALLOC(a.rows, 2 * RC); ALLOC(a.rows4, 2 * RC); ALLOC(a.error_flag, 1);
   ALLOC(a.depth_sum, 1);
@@ -387,6 +391,7 @@ int smz_set_node_pattern(smz_engine* e, int32_t pattern) {
 // Sequential Halving's considered visits (Danihelka et al. 2022, as the published implementation tabulates them):
 // row n (0..SMZ_MAX_POLICY) holds the visit count the next simulation's root child must have, for sum N = 0..N-1
 static void considered_visits(int n, int N, int* row) {
+  if (N <= 0) return;
   if (n <= 1) {
     for (int i = 0; i < N; ++i) row[i] = i;
     return;
@@ -407,6 +412,21 @@ static void considered_visits(int n, int N, int* row) {
   }
 }
 
+// T_b[n][i] for every budget b in [0, N]: row (b, n) at ((b * (SMZ_MAX_POLICY + 1)) + n) * max(N, 1), entries i < b set,
+// the rest 0
+static void budget_schedules(int N, int* out) {
+  const size_t Nt = N > 0 ? N : 1;
+  std::fill(out, out + (size_t)(N + 1) * (SMZ_MAX_POLICY + 1) * Nt, 0);
+  for (int b = 0; b <= N; ++b)
+    for (int n = 0; n <= SMZ_MAX_POLICY; ++n) considered_visits(n, b, out + ((size_t)b * (SMZ_MAX_POLICY + 1) + n) * Nt);
+}
+
+int smz_sequential_halving_table(int32_t num_simulations, int32_t* out) {
+  if (num_simulations < 0 || !out) return fail(SMZ_E_INVALID_ARG, "smz_sequential_halving_table: bad argument");
+  budget_schedules(num_simulations, out);
+  return SMZ_OK;
+}
+
 int smz_set_search(smz_engine* e, int32_t policy, int32_t max_considered, double c_visit, double c_scale) {
   if (policy != SMZ_SEARCH_PUCT && policy != SMZ_SEARCH_GUMBEL)
     return fail(SMZ_E_INVALID_ARG, "smz_set_search: policy %d is neither SMZ_SEARCH_PUCT (0) nor SMZ_SEARCH_GUMBEL (1)",
@@ -424,11 +444,13 @@ int smz_set_search(smz_engine* e, int32_t policy, int32_t max_considered, double
     CU(dev_alloc(e, &a.raw_value, B * (a.N + 1)));
     CU(dev_alloc(e, &a.gumbel_g, B * a.A));
     CU(dev_alloc(e, &a.root_logit, B * a.A));
-    CU(dev_alloc(e, &table, (SMZ_MAX_POLICY + 1) * Nt));
-    std::vector<int> t((SMZ_MAX_POLICY + 1) * Nt, 0);
-    for (int n = 0; n <= SMZ_MAX_POLICY; ++n) considered_visits(n, a.N, t.data() + n * a.N);
+    const size_t n_tab = (size_t)(a.N + 1) * (SMZ_MAX_POLICY + 1) * Nt;     // one schedule per budget
+    CU(dev_alloc(e, &table, n_tab));
+    std::vector<int> t(n_tab);
+    budget_schedules(a.N, t.data());
     CU(cudaMemcpy(table, t.data(), t.size() * sizeof(int), cudaMemcpyHostToDevice));
     a.cv_table = table;
+    a.cv_table_n = table + (size_t)a.N * (SMZ_MAX_POLICY + 1) * Nt;
   }
   e->search_policy = policy;
   e->gumbel_m = max_considered;
@@ -440,6 +462,21 @@ int smz_set_search(smz_engine* e, int32_t policy, int32_t max_considered, double
 static int root_step(smz_engine* e, int32_t n_trees, const float* obs, const float* root_policy,
                      const float* root_value, const int32_t* root_to_play, const uint32_t* legal, int32_t train,
                      const double* dirichlet, const double* gumbels, bool gumbel, void* stream);
+
+int smz_set_root_budgets(smz_engine* e, int32_t n_trees, const int32_t* budget, const uint8_t* explore, void* stream) {
+  if (!e) return fail(SMZ_E_INVALID_ARG, "smz_set_root_budgets: null engine");
+  if (n_trees < 1 || n_trees > e->a.B)
+    return fail(SMZ_E_CAPACITY, "smz_set_root_budgets: n_trees %d not in [1, %d]", n_trees, e->a.B);
+  ON_DEVICE(e);
+  cudaStream_t s = (cudaStream_t)stream;
+  // stream-ordered copies into the engine: the caller's buffers may be reused once this call has been enqueued
+  if (budget) CU(cudaMemcpyAsync(e->a.budget, budget, (size_t)n_trees * sizeof(int32_t), cudaMemcpyDeviceToDevice, s));
+  if (explore) CU(cudaMemcpyAsync(e->a.explore_in, explore, (size_t)n_trees, cudaMemcpyDeviceToDevice, s));
+  e->pend_budget = budget != nullptr;
+  e->pend_explore = explore != nullptr;
+  e->pend_trees = n_trees;
+  return SMZ_OK;
+}
 
 int smz_root(smz_engine* e, int32_t n_trees, const float* obs, const float* root_policy, const int32_t* root_to_play,
              int32_t train, const double* dirichlet, void* stream) {
@@ -479,9 +516,21 @@ static int root_step(smz_engine* e, int32_t n_trees, const float* obs, const flo
   if (obs && e->cfg.net_mode == SMZ_NET_EXTERNAL) return fail(SMZ_E_STATE, "smz_root: obs given but engine has no network");
   if (obs && !e->have_weights) return fail(SMZ_E_STATE, "smz_root: smz_set_weights has not been called");
   if (e->cfg.rng_mode == SMZ_RNG_TAPE && !e->a.tape_u) return fail(SMZ_E_STATE, "smz_root: no uniform tape set");
+  if ((e->pend_budget || e->pend_explore) && e->pend_trees != n_trees)
+    return fail(SMZ_E_INVALID_ARG, "smz_root: smz_set_root_budgets was given %d trees, the root step %d", e->pend_trees,
+                n_trees);
   cudaStream_t s = (cudaStream_t)stream;
   ON_DEVICE(e);
   SmzArena& a = e->a;
+  // this root step's budgets / exploration flags (staged by smz_set_root_budgets), consumed here
+  const int* budget = e->pend_budget ? a.budget : nullptr;
+  const unsigned char* explore = e->pend_explore ? a.explore_in : nullptr;
+  e->has_budgets = e->pend_budget;
+  e->pend_budget = e->pend_explore = e->pend_trees = 0;
+  if (a.budgeted != e->has_budgets) {   // the tree kernels with or without the budget predicate: a different graph
+    a.budgeted = e->has_budgets;
+    drop_graph(e);
+  }
   const int kind_shift = e->node_pattern == SMZ_PATTERN_PAPER ? 0 : 1;
   if (a.kind_shift != kind_shift) {   // the captured simulation graph holds the arena by value
     a.kind_shift = kind_shift;
@@ -513,19 +562,20 @@ static int root_step(smz_engine* e, int32_t n_trees, const float* obs, const flo
     count_launches(e, 1);
     policy = a.out_policy;
   }
-  if (train && !gumbel) {
+  // Dirichlet noise for the trees that explore (their flag, else `train`) and have a simulation (mcts.py:215-216)
+  if ((train || explore) && !gumbel && e->cfg.num_simulations > 0) {
     if (dirichlet) {
       CU(cudaMemcpyAsync(a.dirichlet, dirichlet, (size_t)n_trees * a.A * sizeof(double), cudaMemcpyDeviceToDevice, s));
     } else {
-      smz_launch_dirichlet(a, n_trees, legal, s);
+      smz_launch_dirichlet(a, n_trees, legal, train, budget, explore, s);
       count_launches(e, 1);
     }
   }
   smz_launch_root_expand(a, e->cfg.lanes_per_tree, n_trees, policy, a.W, root_to_play, gumbel ? 0 : train, a.dirichlet,
-                         legal, s);
+                         legal, budget, explore, s);
   count_launches(e, 1);
   if (gumbel) {      // no Dirichlet noise: the root's Gumbels take its place
-    smz_launch_gumbel_root(a, n_trees, obs ? a.out_value : root_value, train, gumbels, s);
+    smz_launch_gumbel_root(a, n_trees, obs ? a.out_value : root_value, train, gumbels, explore, s);
     count_launches(e, 1);
   }
   CU(cudaGetLastError());
@@ -800,7 +850,13 @@ int smz_stats(smz_engine* e, double* mean_leaf_depth, int64_t* launches, int64_t
   CU(cudaMemcpy(&ds, e->a.depth_sum, sizeof(ds), cudaMemcpyDeviceToHost));
   CU(cudaMemcpy(&err, e->a.error_flag, sizeof(err), cudaMemcpyDeviceToHost));
   if (mean_leaf_depth) {
-    const double n = (double)e->n_trees * (double)e->sims_done;
+    double n = (double)e->n_trees * (double)e->sims_done;
+    if (e->has_budgets && e->n_trees > 0) {      // simulations actually run: sum over the trees of min(budget, sims_done)
+      std::vector<int32_t> bud(e->n_trees);
+      CU(cudaMemcpy(bud.data(), e->a.budget, bud.size() * sizeof(int32_t), cudaMemcpyDeviceToHost));
+      n = 0.0;
+      for (int32_t b : bud) n += (double)std::min(b, e->sims_done);
+    }
     *mean_leaf_depth = n > 0 ? (double)ds / n : 0.0;
   }
   if (launches) *launches = e->launches;
@@ -810,5 +866,8 @@ int smz_stats(smz_engine* e, double* mean_leaf_depth, int64_t* launches, int64_t
   if (err == 3)
     return fail(SMZ_E_INVALID_ARG, "a legal-action mask was empty or named an action >= action_dim; that tree was "
                 "searched with every action legal");
+  if (err == 4)
+    return fail(SMZ_E_INVALID_ARG, "a simulation budget was outside [0, num_simulations]; that tree was searched with "
+                "num_simulations");
   return SMZ_OK;
 }

@@ -5,6 +5,7 @@
 //   link [B][M] int2   {child_base i32 (0 = not expanded), key i32}
 //   root_prior [B][A] f64   priors of the root children after Dirichlet mixing (f64 in the reference)
 //   minmax [B] float2  MinMaxStats, mcts.py:24-36
+//   budget [B] int     simulations of each tree, in [0, N] (N unless the root step was given budgets)
 //   hidden [N+1][B][Sp] f32  hidden state of every expanded node: slot 0 = root, slot s+1 = sim s
 //   raw_value [B][N+1] f32   network value of every expanded node by the same slot (Gumbel searches only)
 // Node 0 is the root, 1..A its children, simulation s allocates its children at 1 + A + s*Kmax, so a
@@ -33,6 +34,10 @@ struct SmzArena {
   float2* minmax;
   int* ucursor;
   int* root_to_play;
+  int budgeted;     // 1: the current search was given budgets; selects the BUDGET instantiations of the tree kernels
+  int* budget;      // [B] simulations of each tree (smz_set_root_budgets; N without): tree b takes part in simulation s
+                    // iff s < budget[b].  Written by the root step only, so the captured simulation graph stays valid.
+  unsigned char* explore_in;  // [B] staging of the next root step's exploration flags (smz_set_root_budgets)
   // per-simulation scratch
   int4* path;       // [B][path_stride] per level {node, visit_count, value_sum, reward} captured by the descent
   int* path_len;    // [B]
@@ -88,7 +93,9 @@ struct SmzArena {
   float* raw_value;          // [B][N+1] the network value of every expanded node, by hidden slot (slot 0 = root)
   double* gumbel_g;          // [B][A] the root's Gumbels (0 for illegal actions)
   double* root_logit;        // [B][A] log(prior) - max over legal log(prior) at the root (0 for illegal actions)
-  const int* cv_table;       // [SMZ_MAX_POLICY + 1][max(N, 1)] considered visits of Sequential Halving, T[n][sum of N]
+  const int* cv_table;       // [N + 1][SMZ_MAX_POLICY + 1][max(N, 1)] considered visits of Sequential Halving,
+                             // T_budget[n][sum of N]: each tree follows the schedule of its own budget
+  const int* cv_table_n;     // cv_table's slice of budget N: the schedule of every tree of a search without budgets
 };
 
 #ifdef __CUDACC__

@@ -8,7 +8,7 @@
 // ---- tree kernels (smz_tree.cu, compiled with -fmad=false) ---------------------------------------
 void smz_launch_root_expand(const SmzArena& a, int lanes, int n_trees, const float* policy, int pstride,
                             const int* root_to_play, int train, const double* dirichlet, const uint32_t* legal,
-                            cudaStream_t s);
+                            const int* budget, const unsigned char* explore, cudaStream_t s);
 void smz_launch_select(const SmzArena& a, int lanes, int n_trees, int sim, int* o_slot, int* o_action, int* o_branch,
                        cudaStream_t s);
 void smz_launch_expand_backup(const SmzArena& a, int lanes, int n_trees, int sim, const float* policy, int pstride,
@@ -19,12 +19,13 @@ void smz_launch_read_roots(const SmzArena& a, int n_trees, int* visits, float* v
                            int* error_out, cudaStream_t s);
 void smz_launch_begin_search(const SmzArena& a, cudaStream_t s);
 void smz_launch_set_seed(unsigned long long* dst, unsigned long long seed, unsigned long long tree_id_offset, cudaStream_t s);
-void smz_launch_dirichlet(const SmzArena& a, int n_trees, const uint32_t* legal, cudaStream_t s);
+void smz_launch_dirichlet(const SmzArena& a, int n_trees, const uint32_t* legal, int train, const int* budget,
+                          const unsigned char* explore, cudaStream_t s);
 void smz_launch_select_actions(const SmzArena& a, int n_trees, double temperature, const double* u, int* actions,
                                double* policy, double* stored, cudaStream_t s);
 // Gumbel searches: root values, logits and Gumbels after the root expansion; the action / improved-policy read-out
 void smz_launch_gumbel_root(const SmzArena& a, int n_trees, const float* root_value, int train, const double* given,
-                            cudaStream_t s);
+                            const unsigned char* explore, cudaStream_t s);
 void smz_launch_read_gumbel(const SmzArena& a, int n_trees, int* actions, double* improved, double* gumbels,
                             cudaStream_t s);
 

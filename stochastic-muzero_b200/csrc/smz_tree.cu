@@ -30,10 +30,23 @@ __device__ __forceinline__ unsigned root_legal_set(const uint32_t* __restrict__ 
   return bad ? all : m;
 }
 
+// Simulation budget of a tree at the root step: given (smz_set_root_budgets) or N.  A budget outside [0, N] is `bad`: the
+// tree is then searched with N (k_root_expand raises flag 4).
+__device__ __forceinline__ int root_budget(const int* __restrict__ budget, int tree, int N, bool& bad) {
+  const int b = budget ? budget[tree] : N;
+  bad = b < 0 || b > N;
+  return bad ? N : b;
+}
+// Root noise of a tree (Dirichlet in pUCT mode, Gumbels in Gumbel mode): its exploration flag, or the call's `train`.
+__device__ __forceinline__ bool root_explores(const unsigned char* __restrict__ explore, int tree, int train) {
+  return explore ? explore[tree] != 0 : train != 0;
+}
+
 template <int G>
 __global__ void k_root_expand(SmzArena a, int n_trees, const float* __restrict__ policy, int pstride,
                               const int* __restrict__ root_to_play, int train,
-                              const double* __restrict__ dirichlet, const uint32_t* __restrict__ legal) {
+                              const double* __restrict__ dirichlet, const uint32_t* __restrict__ legal,
+                              const int* budget, const unsigned char* __restrict__ explore) {   // budget may be a.budget
   Group<G> g;
   int tree = (blockIdx.x * blockDim.x + threadIdx.x) / G;
   const bool alive = tree < n_trees;
@@ -41,6 +54,10 @@ __global__ void k_root_expand(SmzArena a, int n_trees, const float* __restrict__
   const size_t tb = (size_t)tree * a.M;
   bool bad;
   const unsigned lm = root_legal_set(legal, tree, a.A, bad);
+  bool bad_budget;
+  const int bud = root_budget(budget, tree, a.N, bad_budget);
+  // Dirichlet noise (pUCT only: `train` is 0 in Gumbel mode) iff the tree explores and has a simulation (mcts.py:215-216)
+  const bool noise = (explore ? explore[tree] != 0 && !a.gumbel : train != 0) && bud > 0;
   // the root's action space is the legal set L: lane i works on its i-th action, so the policy is compacted before
   // it is normalised and drawn from (with every action legal, lane i is action i)
   const int n = __popc(lm);
@@ -54,7 +71,7 @@ __global__ void k_root_expand(SmzArena a, int n_trees, const float* __restrict__
   if (!alive) return;
   if (g.gl < n) {
     double prior = (double)p;
-    if (train) {
+    if (noise) {
       const double nz = dirichlet[(size_t)tree * a.A + act];
       prior = __dadd_rn((double)__fmul_rn(p, a.one_minus_frac_f32), __dmul_rn(nz, a.frac));
     }
@@ -68,10 +85,12 @@ __global__ void k_root_expand(SmzArena a, int n_trees, const float* __restrict__
     a.root_prior[(size_t)tree * a.A + g.gl] = 0.0;
     a.stat[tb + 1 + g.gl] = make_int4(0, 0, 0, 0);
     a.link[tb + 1 + g.gl] = make_int2(0, -1);
-    if (train) a.dirichlet[(size_t)tree * a.A + g.gl] = 0.0;
+    if (noise) a.dirichlet[(size_t)tree * a.A + g.gl] = 0.0;
   }
   if (g.gl == 0) {
     if (bad) *a.error_flag = 3;
+    if (bad_budget) *a.error_flag = 4;
+    a.budget[tree] = bud;
     a.stat[tb] = make_int4(0, 0, 0, 0);
     a.link[tb] = make_int2(1, -1);
     a.minmax[tree] = make_float2(__int_as_float(0x7f800000), __int_as_float(0xff800000));
@@ -85,29 +104,36 @@ __global__ void k_root_expand(SmzArena a, int n_trees, const float* __restrict__
   }
 }
 
-template <int G, bool GUMBEL>
+// BUDGET (compile time, like GUMBEL): the search was given per-tree budgets (smz_set_root_budgets), so a tree takes part
+// in simulation `sim` iff sim < a.budget[tree].  Without budgets every tree has N simulations: the default instantiations
+// do not read the column and keep their registers.
+template <int G, bool GUMBEL, bool BUDGET>
 __global__ void k_select(SmzArena a, int n_trees, int sim, int* __restrict__ o_slot, int* __restrict__ o_action,
                          int* __restrict__ o_branch) {
   Group<G> g;
   int tree = (blockIdx.x * blockDim.x + threadIdx.x) / G;
-  const bool alive = tree < n_trees;
-  if (!alive) tree = n_trees - 1;
+  const bool exists = tree < n_trees;
+  if (!exists) tree = n_trees - 1;
+  const int bud = BUDGET ? a.budget[tree] : a.N;
+  const bool alive = exists && (!BUDGET || sim < bud);
   const SmzRng rng = smz_make_rng(a);
   TreeState ts;
   ts.cursor = a.ucursor[tree];
   ts.mm = a.minmax[tree];
   const int4 rs = a.stat[(size_t)tree * a.M];
   ts.root = make_int2(rs.x, rs.y);
-  select_phase<G, false, GUMBEL>(g, a, rng, tree, alive, sim, ts, o_slot, o_action, o_branch);
+  select_phase<G, false, GUMBEL>(g, a, rng, tree, alive, BUDGET ? bud : -1, sim, ts, o_slot, o_action, o_branch);
+  if (BUDGET && exists && !alive && g.gl == 0 && o_slot) o_slot[tree] = -1;     // no simulation `sim` for this tree
 }
 
-template <int G, bool GUMBEL>
+template <int G, bool GUMBEL, bool BUDGET>
 __global__ void k_expand_backup(SmzArena a, int n_trees, int sim, const float* __restrict__ policy, int pstride,
                                 const float* __restrict__ value, const float* __restrict__ reward) {
   Group<G> g;
   int tree = (blockIdx.x * blockDim.x + threadIdx.x) / G;
-  const bool alive = tree < n_trees;
-  if (!alive) tree = n_trees - 1;
+  const bool exists = tree < n_trees;
+  if (!exists) tree = n_trees - 1;
+  const bool alive = exists && (!BUDGET || sim < a.budget[tree]);
   const SmzRng rng = smz_make_rng(a);
   expand_backup_phase<G, false, GUMBEL>(g, a, rng, tree, alive, sim, policy, pstride, value, reward);
 }
@@ -115,14 +141,17 @@ __global__ void k_expand_backup(SmzArena a, int n_trees, int sim, const float* _
 // expansion + backup of simulation `sim` followed by the descent of simulation `sim + 1` for the same
 // tree by the same lanes: one launch per simulation instead of two, the path nodes just updated are
 // re-read from L1/L2.
-template <int G, bool GUMBEL>
+template <int G, bool GUMBEL, bool BUDGET>
 __global__ void k_backup_select(SmzArena a, int n_trees, int sim) {
-  smz_pdl_wait();                 // the network step of `sim` must have landed
-  smz_pdl_launch_dependents();    // the next network step may set itself up (barriers, TMEM, weights)
   Group<G> g;
   int tree = (blockIdx.x * blockDim.x + threadIdx.x) / G;
-  const bool alive = tree < n_trees;
-  if (!alive) tree = n_trees - 1;
+  const bool exists = tree < n_trees;
+  if (!exists) tree = n_trees - 1;
+  const int bud = BUDGET ? a.budget[tree] : a.N;     // written by the root step: requested before the wait
+  smz_pdl_wait();                 // the network step of `sim` must have landed
+  smz_pdl_launch_dependents();    // the next network step may set itself up (barriers, TMEM, weights)
+  // a tree whose budget is used up takes no part in either phase (its TreeState is then never read)
+  const bool alive = exists && (!BUDGET || sim < bud), alive_next = exists && (!BUDGET || sim + 1 < bud);
   const bool stamp = a.dbg && blockIdx.x == 0 && threadIdx.x == 0;
   if (stamp) a.dbg[0] = clock64();
   const SmzRng rng = smz_make_rng(a);
@@ -130,7 +159,7 @@ __global__ void k_backup_select(SmzArena a, int n_trees, int sim) {
                                                              a.out_reward);
   __syncwarp();
   if (stamp) a.dbg[1] = clock64();
-  select_phase<G, false, GUMBEL>(g, a, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr);
+  select_phase<G, false, GUMBEL>(g, a, rng, tree, alive_next, BUDGET ? bud : -1, sim + 1, ts, nullptr, nullptr, nullptr);
   if (stamp) { a.dbg[2] = clock64(); a.dbg[3] = a.path_len[tree]; }
 }
 
@@ -149,13 +178,15 @@ __host__ __device__ inline size_t smz_mirror_bytes(int tpb, int M, int A, int n_
   return b + 16;
 }
 
-template <int G, bool GUMBEL>
+template <int G, bool GUMBEL, bool BUDGET>
 __global__ void k_backup_select_sm(SmzArena a, int n_trees, int sim, int n_tab) {
   extern __shared__ int4 smz_sm_nodes[];
   Group<G> g;
   int tree = (blockIdx.x * blockDim.x + threadIdx.x) / G;
-  const bool alive = tree < n_trees;
-  if (!alive) tree = n_trees - 1;
+  const bool exists = tree < n_trees;
+  if (!exists) tree = n_trees - 1;
+  const int bud = BUDGET ? a.budget[tree] : a.N;
+  const bool alive = exists && (!BUDGET || sim < bud), alive_next = exists && (!BUDGET || sim + 1 < bud);
   const int tpb = blockDim.x / G, lt = threadIdx.x / G;           // trees per block, local tree
   // ---- carve-up: [stat][link][root priors][uniform window][pbc][rcp64][rcp32]
   int4* sst = smz_sm_nodes + (size_t)lt * a.M;
@@ -173,7 +204,8 @@ __global__ void k_backup_select_sm(SmzArena a, int n_trees, int sim, int n_tab) 
   const int cursor0 = a.ucursor[tree];
   {
     const size_t tb = (size_t)tree * a.M;
-    const int used = 1 + a.A + sim * a.Kmax;                      // nodes allocated before this expansion
+    // nodes allocated before this expansion (a tree whose budget is used up never reads its mirror)
+    const int used = (BUDGET && !alive) ? 0 : 1 + a.A + sim * a.Kmax;
     for (int i = g.gl; i < used; i += G) {
       sst[i] = a.stat[tb + i];
       slk[i] = a.link[tb + i];
@@ -197,7 +229,7 @@ __global__ void k_backup_select_sm(SmzArena a, int n_trees, int sim, int n_tab) 
                                                             a.out_reward, sst, slk);
   __syncwarp();
   if (stamp) a.dbg[1] = clock64();
-  select_phase<G, true, GUMBEL>(g, al, rng, tree, alive, sim + 1, ts, nullptr, nullptr, nullptr, sst, slk, srp);
+  select_phase<G, true, GUMBEL>(g, al, rng, tree, alive_next, BUDGET ? bud : -1, sim + 1, ts, nullptr, nullptr, nullptr, sst, slk, srp);
   if (stamp) { a.dbg[2] = clock64(); a.dbg[3] = a.path_len[tree]; }
   if (a.dbg) {
     __syncthreads();
@@ -301,11 +333,13 @@ __global__ void k_select_actions(SmzArena a, int n_trees, double temperature, co
 // Dirichlet(alpha) per tree on the device: Gamma(alpha) by Marsaglia-Tsang (alpha+1 boost), Philox
 // stream 1.  Production mode only; parity runs pass recorded noise (np.random.dirichlet, mcts.py:220).
 // Draws are taken for the legal actions of the root only, in ascending order; an illegal action's noise is 0.
-__global__ void k_dirichlet(SmzArena a, int n_trees, const uint32_t* __restrict__ legal) {
+__global__ void k_dirichlet(SmzArena a, int n_trees, const uint32_t* __restrict__ legal, int train,
+                            const int* __restrict__ budget, const unsigned char* __restrict__ explore) {
   const int tree = blockIdx.x * blockDim.x + threadIdx.x;
   if (tree >= n_trees) return;
   bool bad;
-  const unsigned lm = root_legal_set(legal, tree, a.A, bad);
+  unsigned lm = root_legal_set(legal, tree, a.A, bad);
+  if (!root_explores(explore, tree, train) || root_budget(budget, tree, a.N, bad) == 0) return;   // no noise: as train = 0
   unsigned ctr = 0;
   const unsigned long long seed = a.seed_state[0], tid = a.seed_state[1] + (unsigned long long)tree;
   auto U = [&]() { double u = smz_philox_uniform(seed, tid, ctr++, 1u); return u > 0.0 ? u : 1.0 / 9007199254740992.0; };
@@ -336,10 +370,11 @@ __global__ void k_dirichlet(SmzArena a, int n_trees, const uint32_t* __restrict_
 // Root of a Gumbel search, one thread per tree, after k_root_expand: the root's network value into raw_value slot 0, the
 // root logits log(p_a) - max_b log(p_b) over the legal actions (float64 root priors), and one Gumbel per legal action in
 // ascending order (train): given by the caller, or -log(-log u) of the uniform #rank of Philox stream 3; eval: 0.
-__global__ void k_gumbel_root(SmzArena a, int n_trees, const float* __restrict__ root_value, int train,
-                              const double* __restrict__ given) {
+__global__ void k_gumbel_root(SmzArena a, int n_trees, const float* __restrict__ root_value, int train_call,
+                              const double* __restrict__ given, const unsigned char* __restrict__ explore) {
   const int tree = blockIdx.x * blockDim.x + threadIdx.x;
   if (tree >= n_trees) return;
+  const bool train = root_explores(explore, tree, train_call);     // a budget-0 tree draws its Gumbels too
   const size_t tb = (size_t)tree * a.M, ro = (size_t)tree * a.A;
   a.raw_value[(size_t)tree * (a.N + 1)] = root_value[tree];
   double mx = -__longlong_as_double(0x7ff0000000000000LL);
@@ -444,25 +479,29 @@ int grid_for(int n_trees, int threads) { return (int)(((long long)n_trees * G + 
 #define SMZ_DISPATCH_GV(G_, V_, CALL)                                        \
   if (V_) { constexpr bool V = true; SMZ_DISPATCH_G(G_, CALL); }             \
   else { constexpr bool V = false; SMZ_DISPATCH_G(G_, CALL); }
+// ... and per-tree budgets (U = a.budgeted)
+#define SMZ_DISPATCH_GVU(G_, V_, U_, CALL)                                   \
+  if (U_) { constexpr bool U = true; SMZ_DISPATCH_GV(G_, V_, CALL); }        \
+  else { constexpr bool U = false; SMZ_DISPATCH_GV(G_, V_, CALL); }
 
 static const int kThreads = 128;
 
 void smz_launch_root_expand(const SmzArena& a, int lanes, int n_trees, const float* policy, int pstride,
                             const int* root_to_play, int train, const double* dirichlet, const uint32_t* legal,
-                            cudaStream_t s) {
+                            const int* budget, const unsigned char* explore, cudaStream_t s) {
   SMZ_DISPATCH_G(lanes, (k_root_expand<G><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(
-                            a, n_trees, policy, pstride, root_to_play, train, dirichlet, legal)));
+                            a, n_trees, policy, pstride, root_to_play, train, dirichlet, legal, budget, explore)));
 }
 
 void smz_launch_select(const SmzArena& a, int lanes, int n_trees, int sim, int* o_slot, int* o_action, int* o_branch,
                        cudaStream_t s) {
-  SMZ_DISPATCH_GV(lanes, a.gumbel, (k_select<G, V><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(
+  SMZ_DISPATCH_GVU(lanes, a.gumbel, a.budgeted, (k_select<G, V, U><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(
                                        a, n_trees, sim, o_slot, o_action, o_branch)));
 }
 
 void smz_launch_expand_backup(const SmzArena& a, int lanes, int n_trees, int sim, const float* policy, int pstride,
                               const float* value, const float* reward, cudaStream_t s) {
-  SMZ_DISPATCH_GV(lanes, a.gumbel, (k_expand_backup<G, V><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(
+  SMZ_DISPATCH_GVU(lanes, a.gumbel, a.budgeted, (k_expand_backup<G, V, U><<<grid_for<G>(n_trees, kThreads), kThreads, 0, s>>>(
                                        a, n_trees, sim, policy, pstride, value, reward)));
 }
 
@@ -494,17 +533,17 @@ static bool mirror_pays(int blocks) {
 void smz_launch_backup_select(const SmzArena& a, int lanes, int n_trees, int sim, bool pdl, cudaStream_t s) {
   if (smz_tree_mirror_fits(a, lanes) && mirror_pays((n_trees * lanes + kThreads - 1) / kThreads)) {
     const size_t smem = mirror_bytes(a, lanes);
-    SMZ_DISPATCH_GV(lanes, a.gumbel,
-                    (cudaFuncSetAttribute((const void*)k_backup_select_sm<G, V>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    SMZ_DISPATCH_GVU(lanes, a.gumbel, a.budgeted,
+                    (cudaFuncSetAttribute((const void*)k_backup_select_sm<G, V, U>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                           (int)smem),
                      getenv("SMZ_NO_CARVEOUT") ? cudaSuccess :
-                     cudaFuncSetAttribute((const void*)k_backup_select_sm<G, V>, cudaFuncAttributePreferredSharedMemoryCarveout,
+                     cudaFuncSetAttribute((const void*)k_backup_select_sm<G, V, U>, cudaFuncAttributePreferredSharedMemoryCarveout,
                                           cudaSharedmemCarveoutMaxShared),
-                     smz_launch(k_backup_select_sm<G, V>, dim3(grid_for<G>(n_trees, kThreads)), dim3(kThreads), smem, s, pdl,
+                     smz_launch(k_backup_select_sm<G, V, U>, dim3(grid_for<G>(n_trees, kThreads)), dim3(kThreads), smem, s, pdl,
                                 a, n_trees, sim, rcp_entries(a))));
     return;
   }
-  SMZ_DISPATCH_GV(lanes, a.gumbel, (smz_launch(k_backup_select<G, V>, dim3(grid_for<G>(n_trees, kThreads)), dim3(kThreads), 0,
+  SMZ_DISPATCH_GVU(lanes, a.gumbel, a.budgeted, (smz_launch(k_backup_select<G, V, U>, dim3(grid_for<G>(n_trees, kThreads)), dim3(kThreads), 0,
                                                s, pdl, a, n_trees, sim)));
 }
 
@@ -537,13 +576,14 @@ void smz_launch_set_seed(unsigned long long* dst, unsigned long long seed, unsig
   k_set_seed<<<1, 1, 0, s>>>(dst, seed, tree_id_offset);
 }
 
-void smz_launch_dirichlet(const SmzArena& a, int n_trees, const uint32_t* legal, cudaStream_t s) {
-  k_dirichlet<<<(n_trees + 127) / 128, 128, 0, s>>>(a, n_trees, legal);
+void smz_launch_dirichlet(const SmzArena& a, int n_trees, const uint32_t* legal, int train, const int* budget,
+                          const unsigned char* explore, cudaStream_t s) {
+  k_dirichlet<<<(n_trees + 127) / 128, 128, 0, s>>>(a, n_trees, legal, train, budget, explore);
 }
 
 void smz_launch_gumbel_root(const SmzArena& a, int n_trees, const float* root_value, int train, const double* given,
-                            cudaStream_t s) {
-  k_gumbel_root<<<(n_trees + 127) / 128, 128, 0, s>>>(a, n_trees, root_value, train, given);
+                            const unsigned char* explore, cudaStream_t s) {
+  k_gumbel_root<<<(n_trees + 127) / 128, 128, 0, s>>>(a, n_trees, root_value, train, given, explore);
 }
 
 void smz_launch_read_gumbel(const SmzArena& a, int n_trees, int* actions, double* improved, double* gumbels,

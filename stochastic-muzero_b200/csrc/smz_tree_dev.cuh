@@ -266,10 +266,11 @@ __device__ __forceinline__ double gumbel_sigma(const Group<G>& g, const SmzArena
 // legal child): argmax over the children whose visit count is the considered count T[min(m, |L|)][sum N] of
 // max(-1e9, g + logit + sigma).  Elsewhere: argmax of pi'_i - N_i / (1 + sum N), pi' = softmax-weighted priors
 // p_i exp(sigma_i - max sigma) / sum.  Ties go to the smaller action; a root with no child at the considered count
-// (the schedule rules it out) takes its first legal child.
+// (the schedule rules it out) takes its first legal child.  T is the schedule of the tree's budget `bud` (-1: a search
+// without budgets, T_N).
 template <int G>
 __device__ __forceinline__ int gumbel_pick(const Group<G>& g, const SmzArena& a, int tree, bool going, bool act, bool root,
-                                           int4 st, double prior_root, double gum, double lgt, int cbase, int width) {
+                                           int4 st, double prior_root, double gum, double lgt, int cbase, int width, int bud) {
   const int slot = (root || !going) ? 0 : (cbase - 1 - a.A) / a.Kmax + 1;     // a group that stopped reads slot 0
   const double vhat = (double)a.raw_value[(size_t)tree * (a.N + 1) + slot];
   const double p = root ? prior_root : (double)__int_as_float(st.w);
@@ -285,7 +286,8 @@ __device__ __forceinline__ int gumbel_pick(const Group<G>& g, const SmzArena& a,
   int best = act ? g.gl : 64;
   if (root) {
     const int n_cons = min(a.gumbel_m, width);
-    const int considered = a.cv_table[n_cons * a.N + min(sum_n, a.N - 1)];
+    const int* T = bud < 0 ? a.cv_table_n : a.cv_table + (size_t)bud * (SMZ_MAX_POLICY + 1) * a.N;
+    const int considered = T[n_cons * a.N + min(sum_n, a.N - 1)];
     if (act && st.x == considered) score = fmax(-1e9, __dadd_rn(__dadd_rn(gum, lgt), sigma));
   } else {
     double ms = act ? sigma : -inf;
@@ -317,9 +319,11 @@ struct TreeState {
 // while descending, so the backup needs ONE round trip (the record) instead of two (index -> stat).
 // The tree is appended to the per-branch row list of the simulation, from which the network step tiles its leaves.
 // Called by every thread of the block: the row reservation below synchronises the block.
+// `alive`: the tree takes part in simulation `sim` (it exists and sim < its budget); `bud` = its budget, or -1 in a search
+// without budgets (the Gumbel root's schedule).
 template <int G, bool MIRROR = false, bool GUMBEL = false>
 __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& a, const SmzRng& rng, int tree, bool alive,
-                                             int sim, TreeState ts, int* __restrict__ o_slot, int* __restrict__ o_action,
+                                             int bud, int sim, TreeState ts, int* __restrict__ o_slot, int* __restrict__ o_action,
                                              int* __restrict__ o_branch, const int4* __restrict__ sst = nullptr,
                                              const int2* __restrict__ slk = nullptr, const double* __restrict__ srp = nullptr) {
   const size_t tb = (size_t)tree * a.M;
@@ -420,7 +424,7 @@ __device__ __forceinline__ void select_phase(const Group<G>& g, const SmzArena& 
       if (chance) { pick = pk; cursor += going ? 1 : 0; }
     }
     if (GUMBEL && !chance) {
-      pick = gumbel_pick(g, a, tree, going, act, root, st, prior0, gum0, lgt0, cbase, width);
+      pick = gumbel_pick(g, a, tree, going, act, root, st, prior0, gum0, lgt0, cbase, width, bud);
     } else if (!chance) {
       // decision node: argmax of ucb_score, one fresh uniform per child (mcts.py:235-243, T3/T5/T6)
       double score = -__longlong_as_double(0x7ff0000000000000LL);

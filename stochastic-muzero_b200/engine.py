@@ -78,6 +78,41 @@ def pack_legal(mask: torch.Tensor) -> torch.Tensor:
     return torch.where(w >= 2 ** 31, w - 2 ** 32, w).to(torch.int32)
 
 
+def budget_rows(budget, n: int, N: int) -> torch.Tensor:
+    """Per-tree simulation budgets -> int32 tensor [n] on the device they came from.  An int is every tree's budget.
+    Integer dtypes only, shape [n]; budgets on the host are also checked against [0, N] here, before any GPU work (budgets
+    already on the device are checked by the root kernel: error flag 4, see smz_set_root_budgets in include/smz.h)."""
+    if isinstance(budget, (bool, np.bool_)) or (not torch.is_tensor(budget) and not isinstance(budget, (int, np.integer))
+                                                and np.asarray(budget).dtype == np.bool_):
+        raise ValueError("simulation budgets are integers, not bools")
+    if isinstance(budget, (int, np.integer)):
+        budget = np.full(n, int(budget), np.int64)
+    t = budget if torch.is_tensor(budget) else torch.as_tensor(np.asarray(budget))
+    if t.dtype.is_floating_point or t.dtype.is_complex or t.dtype == torch.bool:
+        raise ValueError(f"simulation budgets are integers, got {t.dtype}")
+    if t.dim() != 1 or t.shape[0] != n:
+        raise ValueError(f"simulation budgets must have shape [{n}], got {list(t.shape)}")
+    if not t.is_cuda:
+        bad = ((t < 0) | (t > N)).nonzero().flatten()
+        if bad.numel():
+            raise ValueError(f"simulation budgets of trees {bad[:8].tolist()} are outside [0, {N}]: "
+                             f"{t[bad[:8]].tolist()}")
+    return t.to(torch.int32)
+
+
+def explore_rows(explore, n: int) -> torch.Tensor:
+    """Per-tree exploration flags -> uint8 tensor [n] (0 / 1) on the device they came from: bools, or 0 / 1 values on
+    the host."""
+    t = explore if torch.is_tensor(explore) else torch.as_tensor(np.asarray(explore))
+    if t.dim() != 1 or t.shape[0] != n:
+        raise ValueError(f"exploration flags must have shape [{n}], got {list(t.shape)}")
+    if t.dtype.is_floating_point or t.dtype.is_complex:
+        raise ValueError(f"exploration flags are bools or 0 / 1 integers, got {t.dtype}")
+    if not t.is_cuda and t.dtype != torch.bool and not ((t == 0) | (t == 1)).all():
+        raise ValueError("exploration flags are bools or 0 / 1 values")
+    return (t != 0).to(torch.uint8)
+
+
 class RootStats(dict):
     """read_roots() result: the tensors by name; ``block`` = the device block that holds visits | root values | error."""
     block = None
@@ -152,6 +187,7 @@ class SearchEngine:
         self._next_paper = bool(paper_alternation)
         self._apply_node_pattern()
         self.gumbel = False                   # search policy of the following root steps (set_search)
+        self.budgets = None                   # int32 [n] budgets of the current search (host or device), None without
 
     def set_search(self, gumbel: bool, max_considered_actions: int = 16, c_visit: float = 50.0, c_scale: float = 0.1):
         """Search policy of the searches rooted from now on (smz_set_search in include/smz.h): the reference's pUCT
@@ -244,15 +280,34 @@ class SearchEngine:
         assert t.dim() == 2
         self._check(self.lib.smz_set_uniform_tape(self._h, self._ptr(t), t.shape[1]))
 
-    def root(self, obs=None, root_policy=None, root_to_play=None, train=True, dirichlet=None, legal=None):
+    def _set_budgets(self, n, budget, explore):
+        """Validate and stage per-tree budgets / exploration flags for the root step that follows (smz_set_root_budgets
+        in include/smz.h); None for both leaves the root step as it was.  Returns the int32 budgets (or None)."""
+        bud = None if budget is None else budget_rows(budget, n, self.N)
+        exp = None if explore is None else explore_rows(explore, n)
+        self.budgets = bud
+        if bud is None and exp is None:
+            return None
+        bud_d = None if bud is None else self.to_device(bud, torch.int32)
+        exp_d = None if exp is None else self.to_device(exp, torch.uint8)
+        self._check(self.lib.smz_set_root_budgets(self._h, n, self._ptr(bud_d), self._ptr(exp_d), self._stream))
+        self._keep["budget"], self._keep["explore"] = bud_d, exp_d
+        return bud
+
+    def root(self, obs=None, root_policy=None, root_to_play=None, train=True, dirichlet=None, legal=None, budget=None,
+             explore=None):
         """Root step of a search of n trees.  ``legal``: bool / 0-1 mask [n, A] (host or device) restricting each
-        root to the legal actions of its position (smz_root_legal in include/smz.h), or None for every action."""
+        root to the legal actions of its position (smz_root_legal in include/smz.h), or None for every action.
+        ``budget``: int, or int [n] (host or device), the simulations of each tree in [0, N] (smz_set_root_budgets), or
+        None for N; ``explore``: bool / 0-1 [n] per-tree root noise replacing ``train``, or None.  Host inputs are
+        checked before any GPU work."""
         src = obs if obs is not None else root_policy
         n = int(src.shape[0])
         words = None
         if legal is not None:
             words = pack_legal(self.to_device(legal_rows(legal, n, self.A), torch.bool))
             self._keep["legal"] = words
+        self._set_budgets(n, budget, explore)
         obs_t = self._dev(obs, torch.float32, "obs")
         pol_t = None
         if root_policy is not None:
@@ -266,16 +321,18 @@ class SearchEngine:
         self.generation += 1
 
     def root_gumbel(self, obs=None, root_policy=None, root_value=None, root_to_play=None, train=True, gumbels=None,
-                    legal=None):
+                    legal=None, budget=None, explore=None):
         """Root step of a Gumbel search (smz_root_gumbel): like ``root``, without Dirichlet noise; ``root_value`` [n]
         (the network value of each root) goes with ``root_policy``; ``gumbels``: float64 [n, A] recorded Gumbels, or None
-        to draw them on the device (train) — with ``train=False`` every Gumbel is 0."""
+        to draw them on the device (train) — with ``train=False`` every Gumbel is 0.  ``budget`` / ``explore`` as in
+        ``root`` (a tree's flag decides whether it draws Gumbels)."""
         src = obs if obs is not None else root_policy
         n = int(src.shape[0])
         words = None
         if legal is not None:
             words = pack_legal(self.to_device(legal_rows(legal, n, self.A), torch.bool))
             self._keep["legal"] = words
+        self._set_budgets(n, budget, explore)
         obs_t = self._dev(obs, torch.float32, "obs")
         pol_t = None
         if root_policy is not None:
@@ -392,6 +449,9 @@ class SearchEngine:
         if code == 3:
             raise ValueError("a legal-action mask was empty or named an action >= A (that tree was searched with every "
                              "action legal)")
+        if code == 4:
+            raise ValueError("a simulation budget was outside [0, num_simulations] (that tree was searched with "
+                             "num_simulations)")
 
     def select_actions(self, temperature: float, uniforms=None):
         """game.py:179-235 for every tree: -> dict(actions int32[n], policy f64[n,A], stored_policy f64[n,A])."""

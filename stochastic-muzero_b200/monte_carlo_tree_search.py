@@ -23,7 +23,7 @@ import numpy as np
 import torch
 
 from . import batched_model
-from .engine import SearchEngine, legal_rows
+from .engine import SearchEngine, budget_rows, explore_rows, legal_rows
 from .weights import (PackedModel, VisionShape, pack_vision_weights, pack_weights, shape_of, weights_version)
 
 
@@ -165,6 +165,25 @@ def _legal_kw(legal):
     return {} if legal is None else {"legal": legal}
 
 
+def _budget_plan(num_simulations, n, N):
+    """``num_simulations`` of run_batch / run -> (budgets for the root step or None, simulation steps to run).  None: every
+    tree N; an int or a host sequence: checked here, and the search runs max(budget) steps; a device tensor: N steps, no
+    host synchronisation (its range is checked by the root kernel)."""
+    if num_simulations is None:
+        return None, N
+    bud = budget_rows(num_simulations, n, N)
+    return bud, N if bud.is_cuda else (int(bud.max()) if bud.numel() else 0)
+
+
+def _root_kw(legal, budget, explore):
+    kw = _legal_kw(legal)
+    if budget is not None:
+        kw["budget"] = budget
+    if explore is not None:
+        kw["explore"] = explore
+    return kw
+
+
 class StaleSearchError(RuntimeError):
     """A view of a finished search was used after the engine's arena had been reused by a newer search."""
 
@@ -186,6 +205,7 @@ class BatchedRoots:
         self.rewards = stats["rewards"]           # float32 [B, A]
         self.root_values = stats["root_values"]   # float32 [B]
         self.error = stats.get("error")           # int32 [1] device: the search's error flag (engine.raise_for_error)
+        self.budgets = engine.budgets             # int32 [B] simulations of each tree (host or device), None = N each
         self._block = getattr(stats, "block", None)   # visit counts | root values | error flag in one device block
         self._host = None
 
@@ -412,7 +432,7 @@ class Monte_carlo_tree_search():
 
     # ------------------------------------------------------------------------------------------
     def run_batch(self, observations, model=None, train=True, root_to_play=None, check=True, *,
-                  legal_actions=None) -> BatchedRoots:
+                  legal_actions=None, num_simulations=None, explore=None) -> BatchedRoots:
         """B independent searches in one call.  ``observations``: float tensor/array [B, obs_dim]
         (host or device).  Returns BatchedRoots (device tensors; ``roots[i]`` gives a Node view).
         ``check`` (default): wait for the search and raise if it met a degenerate policy, like the reference's
@@ -421,11 +441,20 @@ class Monte_carlo_tree_search():
         position only, as the reference's root would with that action space; illegal actions get no child, no visit and
         prior 0, and ``select_actions`` never returns one.  A host mask with an empty row raises ValueError before any
         GPU work; a device mask with an empty row or a bit >= A raises ValueError at the check (that tree is searched
-        with every action legal)."""
+        with every action legal).
+        ``num_simulations``: the simulations of each tree — an int <= N, or an int sequence / tensor [B] (host or device)
+        — or None for N (the constructor's ``num_simulations``).  A tree with budget n is the search with num_simulations
+        = n.  Host budgets run max(budget) simulation steps; a device tensor runs N steps and needs no host
+        synchronisation.  ``explore``: bool / 0-1 [B] per-tree root noise (Dirichlet, or Gumbels with ``gumbel``)
+        replacing ``train`` for that tree, or None.  Out-of-range host budgets raise ValueError before any GPU work, device
+        ones at the check (that tree is searched with N)."""
         if legal_actions is not None:
             legal_actions = legal_rows(legal_actions, len(observations))
+        budget, n_sims = _budget_plan(num_simulations, len(observations), self.num_simulations)
+        if explore is not None:
+            explore = explore_rows(explore, len(observations))
         if not self._is_fusable(model):
-            roots = self._run_batch_external(observations, model, train, root_to_play, legal_actions)
+            roots = self._run_batch_external(observations, model, train, root_to_play, legal_actions, budget, explore)
             return roots.raise_if_failed() if check else roots
         self.model = model
         vision = getattr(model, "model_structure", None) == "vision_model"
@@ -453,15 +482,17 @@ class Monte_carlo_tree_search():
                 self._weights_seen[key] = ver
         obs = eng.to_device(obs, torch.float32)      # the observations' host-to-device copy is enqueued first
         eng.set_seed(self._next_seed(), self._offset(obs.shape[0]))
+        kw = _root_kw(legal_actions, budget, explore)
         if self.gumbel:
-            eng.root_gumbel(obs=obs, root_to_play=root_to_play, train=train, **_legal_kw(legal_actions))
+            eng.root_gumbel(obs=obs, root_to_play=root_to_play, train=train, **kw)
         else:
-            eng.root(obs=obs, root_to_play=root_to_play, train=train, **_legal_kw(legal_actions))
-        eng.simulate(self.num_simulations)
+            eng.root(obs=obs, root_to_play=root_to_play, train=train, **kw)
+        eng.simulate(n_sims)
         roots = BatchedRoots(eng, eng.read_roots())
         return roots.raise_if_failed() if check else roots
 
-    def _run_batch_external(self, observations, model, train, root_to_play, legal_actions=None):
+    def _run_batch_external(self, observations, model, train, root_to_play, legal_actions=None, budget=None,
+                            explore=None):
         """Any other model family: tree kernels in the engine, network step = five batched device
         functions (batched_model.py) — either supplied directly or built from the six nn.Modules of a
         reference-style Muzero."""
@@ -485,15 +516,20 @@ class Monte_carlo_tree_search():
         C = int(getattr(backend, "C", A))
         eng, _ = self._engine("external", obs.shape[0], A, C)
         eng.set_seed(self._next_seed(), self._offset(obs.shape[0]))
-        store = batched_model.run_search(eng, backend, obs, self.num_simulations, root_to_play, train, legal_actions)
+        store = batched_model.run_search(eng, backend, obs, self.num_simulations, root_to_play, train, legal_actions,
+                                         budget, explore)
         roots = BatchedRoots(eng, eng.read_roots())
         roots.hidden_store = store
         return roots
 
-    def run(self, observation=None, model=None, train=True, *, legal_actions=None):
+    def run(self, observation=None, model=None, train=True, *, legal_actions=None, num_simulations=None):
         """One search, reference signature (:311).  Returns the root Node.  ``legal_actions``: the legal actions of the
         position, as a sequence of action indices or a bool mask [A] (see ``run_batch``); ``root.children`` then has
-        exactly those keys."""
+        exactly those keys.  ``num_simulations``: an int <= N, this search's budget (None: N)."""
+        if num_simulations is not None:
+            if not isinstance(num_simulations, (int, np.integer)) or isinstance(num_simulations, (bool, np.bool_)):
+                raise ValueError(f"run's num_simulations is an int, got {num_simulations!r}")
+            budget_rows(int(num_simulations), 1, self.num_simulations)
         self.model = model
         to_play = self.cycle.global_step()
         if self._is_fusable(model):
@@ -503,18 +539,19 @@ class Monte_carlo_tree_search():
                 legal = _legal_row(legal_actions, model.shape.action_dim if isinstance(model, PackedModel)
                                    else int(model.action_dimension))
             batch = self.run_batch(obs.reshape(1, *obs.shape[1:]) if obs.dim() > 1 else obs.reshape(1, -1), model, train,
-                                   root_to_play=torch.tensor([to_play], dtype=torch.int32), legal_actions=legal)
+                                   root_to_play=torch.tensor([to_play], dtype=torch.int32), legal_actions=legal,
+                                   num_simulations=num_simulations)
             eng = batch._engine
             dump = eng.export_tree(0)
             self.root = _node_tree(dump, batch._hidden_fetcher(0))
         else:
-            self.root = self._run_callback(observation, model, train, to_play, legal_actions)
+            self.root = self._run_callback(observation, model, train, to_play, legal_actions, num_simulations)
             return self.root
         self.min_max_stats = MinMaxStats(np.float32(dump["minmax"][0]), np.float32(dump["minmax"][1]))
         self.node = self.root
         return self.root
 
-    def _run_callback(self, observation, model, train, to_play, legal_actions=None):
+    def _run_callback(self, observation, model, train, to_play, legal_actions=None, num_simulations=None):
         """Host-model mode: tree kernels on the GPU, the five inference methods called back per
         simulation (:182, :198, :271-286)."""
         h0 = model.representation_function_inference(observation)
@@ -524,14 +561,15 @@ class Monte_carlo_tree_search():
         eng, _ = self._engine("external", 1, A, getattr(model, "chance_dimension", A))
         eng.set_seed(self._next_seed(), self._offset(1))
         legal = None if legal_actions is None else _legal_row(legal_actions, A)
+        budget, n_sims = _budget_plan(num_simulations, 1, self.num_simulations)
+        kw = _root_kw(legal, budget, None)
         if self.gumbel:
             eng.root_gumbel(root_policy=policy, root_value=np.array([value0], dtype=np.float32).reshape(1),
-                            root_to_play=torch.tensor([to_play], dtype=torch.int32), train=train, **_legal_kw(legal))
+                            root_to_play=torch.tensor([to_play], dtype=torch.int32), train=train, **kw)
         else:
-            eng.root(root_policy=policy, root_to_play=torch.tensor([to_play], dtype=torch.int32), train=train,
-                     **_legal_kw(legal))
+            eng.root(root_policy=policy, root_to_play=torch.tensor([to_play], dtype=torch.int32), train=train, **kw)
         hidden = {0: h0}
-        for sim in range(self.num_simulations):
+        for sim in range(n_sims):                 # the model is called for the tree's own simulations only
             slot, action, branch = (int(t.item()) for t in eng.select(sim))
             if branch:
                 reward, h = model.dynamics_function_inference(hidden[slot], np.int64(action))

@@ -69,10 +69,25 @@ class VectorCartPole:
 
 
 class SelfPlay:
-    """Lock-step self-play of B games for T moves; trajectories stay on the device."""
+    """Lock-step self-play of B games for T moves; trajectories stay on the device.
 
-    def __init__(self, mcts, model, env, horizon: int):
+    ``playout_cap=(p_full, n_fast)``: playout-cap randomisation (Wu 2019, "Accelerating Self-Play Learning in Go"; used
+    by KataGo).  Every move of every game draws, from a generator seeded with ``seed``, a full search (the search's N
+    simulations, root noise as ``train`` says) with probability p_full, else a fast search of n_fast simulations.  With
+    pUCT the fast search has no Dirichlet noise; with Gumbel it keeps its Gumbels, which are how Gumbel picks the move.
+    The buffer's ``full_search`` [T, B] marks the full searches, whose policy targets a trainer keeps.  None: every move
+    is a full search and the buffer is as without the option."""
+
+    def __init__(self, mcts, model, env, horizon: int, playout_cap=None, seed: int = 0):
         self.mcts, self.model, self.env, self.T = mcts, model, env, horizon
+        if playout_cap is not None:
+            p_full, n_fast = playout_cap
+            if not 0.0 <= float(p_full) <= 1.0:
+                raise ValueError(f"playout_cap's p_full must be in [0, 1], got {p_full}")
+            if isinstance(n_fast, bool) or not isinstance(n_fast, (int,)) or not 0 <= n_fast <= mcts.num_simulations:
+                raise ValueError(f"playout_cap's n_fast must be an int in [0, {mcts.num_simulations}], got {n_fast!r}")
+            playout_cap = (float(p_full), int(n_fast))
+        self.playout_cap, self.seed = playout_cap, int(seed)
 
     @torch.no_grad()
     def run(self, temperature: float = 1.0, train: bool = True) -> Dict[str, torch.Tensor]:
@@ -85,10 +100,22 @@ class SelfPlay:
                "rewards": torch.zeros(T, B, device=dev), "dones": torch.zeros(T, B, dtype=torch.bool, device=dev),
                "child_visits": torch.zeros(T, B, A, dtype=torch.float64, device=dev),
                "root_values": torch.zeros(T, B, device=dev)}
+        gumbel = getattr(self.mcts, "gumbel", False)
+        if self.playout_cap is not None:
+            buf["full_search"] = torch.zeros(T, B, dtype=torch.bool, device=dev)
+            gen = torch.Generator(device=dev).manual_seed(self.seed)
+            N, (p_full, n_fast) = self.mcts.num_simulations, self.playout_cap
         for t in range(T):
             legal = env.legal_mask() if hasattr(env, "legal_mask") else None
-            roots = self.mcts.run_batch(obs, self.model, train=train, legal_actions=legal)   # one move of every game
-            if getattr(self.mcts, "gumbel", False):      # Gumbel search: its action, its improved policy as the target
+            cap = {}
+            if self.playout_cap is not None:       # budgets and flags stay on the device: no host round-trip per move
+                full = torch.rand(B, device=dev, generator=gen) < p_full
+                buf["full_search"][t] = full
+                cap["num_simulations"] = torch.where(full, N, n_fast).to(torch.int32)
+                if not gumbel:
+                    cap["explore"] = full & bool(train)
+            roots = self.mcts.run_batch(obs, self.model, train=train, legal_actions=legal, **cap)   # one move of every game
+            if gumbel:                                   # Gumbel search: its action, its improved policy as the target
                 g = roots.gumbel()
                 pick = {"actions": g["actions"], "stored_policy": g["improved_policy"]}
             else:
@@ -103,20 +130,31 @@ class SelfPlay:
 
 @torch.no_grad()
 def reanalyse(mcts, model, observations: torch.Tensor, chunk: int = 16384, train: bool = True,
-              legal_actions: Optional[torch.Tensor] = None) -> Dict[str, torch.Tensor]:
+              legal_actions: Optional[torch.Tensor] = None, num_simulations=None) -> Dict[str, torch.Tensor]:
     """Reanalyse (self_play.py:30-44, game.py:112-116, replay_buffer.py:229-266): re-run the search over stored
     observations of old games with the current weights.  Every stored position is an independent tree, so
     the [T, B, ...] trajectory block is simply flattened into large batches for the engine.
     ``legal_actions``: optional bool mask [T, B, A] of the stored positions' legal actions.
+    ``num_simulations``: an int, or an int [T, B] tensor / array giving each stored position its own budget (older or less
+    valuable data may get fewer simulations), or None for the search's N.
     Returns fresh targets: child_visits [T, B, A] (stored visit policy; the improved policy of a Gumbel search) and
     root_values [T, B]."""
     T, B = observations.shape[:2]
     flat = observations.reshape((T * B,) + tuple(observations.shape[2:]))
     legal = None if legal_actions is None else legal_actions.reshape(T * B, -1)
+    budget = num_simulations
+    if budget is not None and not isinstance(budget, int):
+        budget = budget if torch.is_tensor(budget) else torch.as_tensor(budget)
+        if tuple(budget.shape) != (T, B):
+            raise ValueError(f"reanalyse's num_simulations must be an int or have shape [{T}, {B}], got "
+                             f"{list(budget.shape)}")
+        budget = budget.reshape(T * B)
     visits, values = [], []
     for lo in range(0, T * B, chunk):
         roots = mcts.run_batch(flat[lo:lo + chunk], model, train=train,
-                               legal_actions=None if legal is None else legal[lo:lo + chunk])
+                               legal_actions=None if legal is None else legal[lo:lo + chunk],
+                               num_simulations=budget if budget is None or isinstance(budget, int)
+                               else budget[lo:lo + chunk])
         if getattr(mcts, "gumbel", False):         # the Gumbel search's policy target
             visits.append(roots.gumbel()["improved_policy"])
         else:
